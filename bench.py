@@ -5,6 +5,7 @@
     python bench.py --workload c3 ...                           # the north-star size as the headline workload
     python bench.py --impl reference --steps 2 --warmup 1       # the reference on the host cores (same --workload)
     torchrun --nproc-per-node N ... bench.py --gpus N ...       # N ranks (see "multi-GPU" below)
+    python bench.py ... --dump-outputs DIR                      # also save what the last timed step computed
 
 A "step" is one evaluation of LML and its full theta-gradient (build -> Cholesky -> solves -> inverse -> gradient
 contraction).  Headline workload: BASELINE.json `configs[1]` (c2: d=10, n=500, N=5500, preconditioned) unless
@@ -19,6 +20,10 @@ D2H of the result every step).  The same line carries, measured in the same run 
   c5       BASELINE configs[4]: N=51000 build + Cholesky in the base / rescale_origin / precon modes.
 Multi-GPU: the headline stays the c2 evaluation, one independent candidate per rank and step plus one all_gather of the
 result rows ("weak"); the sharded candidate scan rides along as `c4_scan` with its own strong-scaling numbers.
+--steps sets the number of timed steps, each on its own theta (step_theta); with the same arguments the inputs (seeded
+data and thetas) are the same from run to run.  --dump-outputs DIR writes the result rows of the last timed step, as the
+caller of gegp_lml_eval receives them ([ranks, 10 + d] float64 in the OUT_* slots of include/gegp.h: LML, sigma^2, beta,
+ln det, info, ..., then the theta-gradient), to DIR/lml_eval_out.npy, so that two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -72,6 +77,13 @@ def make_problem(n, d, seed=0):
 def step_theta(theta, step, rank):
     """A different candidate every step and rank (no result can be cached)."""
     return theta * (1.0 + 0.003 * step + 0.0007 * rank)
+
+
+def dump_outputs(out_dir, **arrays):
+    """--dump-outputs: each device tensor as out_dir/<name>.npy in float64."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy().astype(np.float64))
 
 
 # ----------------------------------------------------------------------------------------------- clocks
@@ -289,6 +301,8 @@ def run_b200(args):
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     clocks = sampler.stop() if rank == 0 else None
     last = last.clone()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, lml_eval_out=last)
     info_ok = bool((last[:, L.OUT_INFO] == 0).all().item())
     value = world * K / (ms_total * 1e-3)
 
@@ -668,7 +682,13 @@ def main():
     ap.add_argument("--no-c5", action="store_true", help="skip the N=51000 build + Cholesky block (BASELINE configs[4])")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-phases", action="store_true", help="profiling aid: skip the roofline / phase measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the result rows of the last one to DIR/lml_eval_out.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the CUDA path computed; it needs --impl b200")
     if args.impl == "reference":
         run_reference(args)
     else:
