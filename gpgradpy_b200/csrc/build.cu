@@ -471,22 +471,36 @@ int launch_build_cov(const Ctx& ctx, const Geom& gm, const double* theta, int64_
   return 0;
 }
 
+// Both cross-covariance kernels put test points on gridDim.y, which is limited to 65535.  A small training set lets
+// the prediction chunk hold far more test points than that (n = 20, d = 2: ~700k gradient points per GiB), so the
+// launch is issued in slices of at most MAX_GRID_Y grid rows, each with Xs and out advanced to its first point.  Every
+// test point is computed by the same thread arithmetic whichever slice it lands in.
+constexpr int MAX_GRID_Y = 65535;
+
 int launch_cross_cov(const Ctx& ctx, const Geom& gm, const double* theta, const double* pinv, const double* Xs, int nx,
                      double* out, int64_t ld) {
   const size_t smem = (size_t)(8 * gm.d + gm.d) * sizeof(double);
-  dim3 grid((gm.n + 255) / 256, (nx + 7) / 8, 1);
-  cross_cov_kernel<<<grid, 256, smem, ctx.stream>>>(gm, theta, pinv, Xs, nx, out, ld);
-  GEGP_CHECK_LAUNCH();
+  constexpr int SLICE = 8 * MAX_GRID_Y;   // 8 test points per CTA row
+  for (int x0 = 0; x0 < nx; x0 += SLICE) {
+    const int cx = (nx - x0 < SLICE) ? nx - x0 : SLICE;
+    dim3 grid((gm.n + 255) / 256, (cx + 7) / 8, 1);
+    cross_cov_kernel<<<grid, 256, smem, ctx.stream>>>(gm, theta, pinv, Xs + (int64_t)x0 * gm.d, cx,
+                                                      out + (int64_t)x0 * ld, ld);
+    GEGP_CHECK_LAUNCH();
+  }
   return 0;
 }
 
 int launch_cross_cov_dx(const Ctx& ctx, const Geom& gm, const double* theta, const double* pinv, const double* Xs, int nx,
                         double* out, int64_t ld) {
-  if (nx <= 0) return 0;
   const size_t smem = (size_t)(2 * gm.d) * sizeof(double);
-  dim3 grid((gm.n + 255) / 256, nx, 1);
-  cross_cov_dx_kernel<<<grid, 256, smem, ctx.stream>>>(gm, theta, pinv, Xs, nx, out, ld);
-  GEGP_CHECK_LAUNCH();
+  for (int x0 = 0; x0 < nx; x0 += MAX_GRID_Y) {   // one test point (d + 1 output rows) per CTA row
+    const int cx = (nx - x0 < MAX_GRID_Y) ? nx - x0 : MAX_GRID_Y;
+    dim3 grid((gm.n + 255) / 256, cx, 1);
+    cross_cov_dx_kernel<<<grid, 256, smem, ctx.stream>>>(gm, theta, pinv, Xs + (int64_t)x0 * gm.d, cx,
+                                                         out + (int64_t)x0 * (gm.d + 1) * ld, ld);
+    GEGP_CHECK_LAUNCH();
+  }
   return 0;
 }
 

@@ -779,22 +779,27 @@ def kern_hess_x(X, xs, theta, kernel=None):
     return H
 
 
-def eval_model_hess(X, fval, grad, theta, varK, beta, xs, mode="precon", eta=None, kernel=None):
+def eval_model_hess(X, fval, grad, theta, varK, beta, xs, mode="precon", eta=None, kernel=None, noise_vec=None,
+                    mask=None):
     """eval_model(calc_grad=True, calc_hess=True) at ONE point: (mu, sig, dmudx, dsigdx, d2mudx2, d2sigdx2)
-    (eval/GpEvalModel.py:175-180, 356-382)."""
+    (eval/GpEvalModel.py:175-180, 356-382).  noise_vec and mask as in eval_model_grad (grad then holds the rows of
+    the masked points only).  With a mask the rows of k* are a subset of the all-gradient rows, in the order
+    value p, then gradient (j, slot) = all-gradient row n + j n + p; the masked Hessian selects those rows."""
     n, d = X.shape
     if eta is None:
         eta = nugget(n, d, mode, kernel=kernel)[1]
     xs = np.atleast_2d(xs)
-    mu, sig, dmu, dsig = eval_model_grad(X, fval, grad, theta, varK, beta, xs, mode, eta, kernel=kernel)
-    ka = all_K_w_chofac(X, theta, mode, eta, None, 1.0, None, kernel=kernel)
+    mu, sig, dmu, dsig = eval_model_grad(X, fval, grad, theta, varK, beta, xs, mode, eta, noise_vec, mask, kernel=kernel)
+    ka = all_K_w_chofac(X, theta, mode, eta, noise_vec, 1.0, mask, kernel=kernel)
+    sel = _sel(n, mask)
     y = make_data_vec(fval, grad)
-    H = aug_vand(n, n, d)
+    H = aug_vand(n, sel.size, d)
     a = linalg.cho_solve(ka.chofac, y - H @ np.atleast_1d(beta))
-    Kg = kern_grad(X, xs, theta, None, None, kernel=kernel)
+    Kg = kern_grad(X, xs, theta, mask, None, kernel=kernel)
     Kyx, dKxy = Kg[:, :1], Kg[:, 1:].T
     KinvK = linalg.cho_solve(ka.chofac, Kyx)[:, 0]
-    d2K = kern_hess_x(X, xs[0], theta, kernel=kernel)
+    rows = np.concatenate([np.arange(n)] + [n + j * n + sel for j in range(d)])
+    d2K = kern_hess_x(X, xs[0], theta, kernel=kernel)[:, :, rows]
     d2mu = d2K @ a
     term1 = d2K @ KinvK
     term2 = dKxy @ linalg.cho_solve(ka.chofac, dKxy.T)
