@@ -27,7 +27,7 @@ OPT_INV_EARLY = 5
 EXPORTS = (
     "gegp_abi_version", "gegp_set_option", "gegp_workspace_bytes", "gegp_ld", "gegp_build_cov", "gegp_cross_cov", "gegp_potrf",
     "gegp_trsm_rows", "gegp_dinv_doubles", "gegp_potri", "gegp_dgemm", "gegp_lml_eval", "gegp_predict_setup", "gegp_predict", "gegp_profile_begin", "gegp_profile_end",
-    "gegp_predict_grad", "gegp_predict_hess", "gegp_lml_layout", "gegp_symv", "gegp_row_abs_sum", "gegp_row_sq_sum", "gegp_weighted_grad", "gegp_lanczos_step", "gegp_lincomb", "gegp_quad_grad_work_bytes", "gegp_quad_grad", "gegp_dmma_peak", "gegp_lml_direct_terms",
+    "gegp_predict_grad", "gegp_predict_hess", "gegp_predict_hess_batch", "gegp_lml_layout", "gegp_symv", "gegp_row_abs_sum", "gegp_row_sq_sum", "gegp_weighted_grad", "gegp_lanczos_step", "gegp_lincomb", "gegp_quad_grad_work_bytes", "gegp_quad_grad", "gegp_dmma_peak", "gegp_lml_direct_terms",
 )
 
 
@@ -84,6 +84,9 @@ def load():
     lib.gegp_predict_hess.restype = i
     lib.gegp_predict_hess.argtypes = [i, i, i, dp, ip, dp, i, dbl, dp, i64, dp, dp, dp, i, dbl, dbl, dp, dp, dp, dp, dp, dp, dp, ip,
                                       vp, sz, vp]
+    lib.gegp_predict_hess_batch.restype = i
+    lib.gegp_predict_hess_batch.argtypes = [i, i, i, dp, ip, dp, i, dbl, dp, i64, dp, dp, dp, i, dbl, dbl, dp, i, dp, dp, dp, dp,
+                                            dp, dp, ip, vp, sz, vp]
     lib.gegp_lml_layout.restype = i
     lib.gegp_lml_layout.argtypes = [i, i, i, i, i, C.POINTER(i64)]
     lib.gegp_symv.restype = i

@@ -417,6 +417,37 @@ def predict_hess(st: PredictState, xs, varK: float):
     return mu, sig, sig2, dmu, dsg, h3, nneg
 
 
+def predict_hess_batch_bytes(N: int, d: int, nx: int) -> int:
+    """Workspace of gegp_predict_hess_batch for chunks of nx points (include/gegp.h)."""
+    return L.load().gegp_dinv_doubles(N) * 8 + nx * ((d + 1) * ld_of(N) + 128) * 8
+
+
+def predict_hess_batch(st: PredictState, Xs, varK: float, *, chunk_bytes: int = 1 << 30):
+    """gegp_predict_hess_batch at nx points -> (mu, sig, sig2, dmudx [nx, d], dsigdx [nx, d], hess3 [nx, 3, d, d],
+    n_negative) device tensors; chunks of as many points as chunk_bytes of workspace hold (at least one)."""
+    lib = L.load()
+    Xs = to_dev(Xs)
+    nx, d = Xs.shape[0], st.d
+    assert Xs.ndim == 2 and Xs.shape[1] == d and st.alpha is not None
+    dev = device()
+    mu, sig, sig2 = (torch.empty(nx, dtype=F64, device=dev) for _ in range(3))
+    dmu, dsg = (torch.empty((nx, d), dtype=F64, device=dev) for _ in range(2))
+    h3 = torch.empty((nx, 3, d, d), dtype=F64, device=dev)
+    nneg = torch.zeros(1, dtype=torch.int32, device=dev)
+    if nx == 0:
+        return mu, sig, sig2, dmu, dsg, h3, nneg
+    per_x = predict_hess_batch_bytes(st.N, d, 1) - predict_hess_batch_bytes(st.N, d, 0)
+    cx = max(1, min(nx, (chunk_bytes - predict_hess_batch_bytes(st.N, d, 0)) // per_x))
+    nbytes = predict_hess_batch_bytes(st.N, d, cx)
+    ws = workspace(nbytes)
+    rc = lib.gegp_predict_hess_batch(st.n, st.n_g, st.d, _p(st.X), _p(st.slot), _p(st.theta), st.kid, st.khp, _p(st.A),
+                                     st.A.stride(0), _p(st.dinv), _p(st.p), _p(st.alpha), int(st.mode), st.beta, float(varK),
+                                     _p(Xs), nx, _p(mu), _p(sig), _p(sig2), _p(dmu), _p(dsg), _p(h3), _p(nneg), _p(ws), nbytes,
+                                     _stream())
+    _check(rc, "gegp_predict_hess_batch")
+    return mu, sig, sig2, dmu, dsg, h3, nneg
+
+
 # ----------------------------------------------------------------------------------------------------------------
 # 2-norm condition number and its hyper-parameter gradient (kernel/Kernel.py:240,280; optz/GpHparaCon.py:161-235)
 # ----------------------------------------------------------------------------------------------------------------

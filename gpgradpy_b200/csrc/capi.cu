@@ -679,6 +679,66 @@ int gegp_predict_hess(int n, int n_g, int d, const double* X, const int32_t* gra
   return launch_predict_hess(ctx, gm, theta, xs, alpha, bvec, Z, ldz, hess3);
 }
 
+int gegp_predict_hess_batch(int n, int n_g, int d, const double* X, const int32_t* grad_slot, const double* theta, int kernel,
+                            double kernel_hp, const double* A, int64_t lda, const double* dinv, const double* p,
+                            const double* alpha, int mode, double beta, double varK, const double* Xs, int nx, double* mu,
+                            double* sig, double* sig2_out, double* dmudx, double* dsigdx, double* hess3, int* n_negative_dev,
+                            void* work, size_t work_bytes, void* stream) {
+  if (bad_geom(n, n_g, d)) return -1;
+  if (d > 63) return -3;                       // the contraction kernel keeps d (d + 1) / 2 <= 2048 pairs per CTA
+  if (bad_kernel(kernel, kernel_hp)) return -50;
+  if (!X) return -4;
+  if (n_g != n && !grad_slot) return -5;
+  if (!theta) return -6;
+  if (!A) return -7;
+  const int N = n + n_g * d;
+  if (lda < N || (lda & 1)) return -8;
+  if (!dinv) return -9;
+  if (!p) return -10;
+  if (!alpha) return -11;
+  if (!Xs) return -15;
+  if (nx < 0) return -16;
+  if (!mu) return -17;
+  if (!sig) return -18;
+  if (!dmudx) return -20;
+  if (!dsigdx) return -21;
+  if (!hess3) return -22;
+  if (!work || (reinterpret_cast<uintptr_t>(work) & 15)) return -24;
+  (void)mode;
+  const int64_t ldz = gegp_ld(N);
+  const size_t fixed = (size_t)dinv_doubles(N) * sizeof(double);
+  const size_t per_x = ((size_t)(d + 1) * ldz + LEAF) * sizeof(double);
+  const int chunk = work_bytes > fixed ? (int)std::min<size_t>((size_t)nx, (work_bytes - fixed) / per_x) : 0;
+  if (nx > 0 && chunk < 1) return -25;
+  if (nx == 0) return 0;
+  Ctx ctx{(cudaStream_t)stream, 1};
+  const Geom gm = make_geom(n, n_g, d, X, grad_slot, kernel, kernel_hp);
+  const double* pinv = p + N;
+  const double* w = A + (int64_t)N * lda;
+  double* Lt = reinterpret_cast<double*>(work);                 // transposed diagonal blocks of the factor
+  double* Z = Lt + dinv_doubles(N);                              // (d + 1) solved rows per point
+  double* T = Z + (int64_t)chunk * (d + 1) * ldz;                // leaf scratch of the back substitution, chunk x LEAF
+  const int64_t ldb = (int64_t)(d + 1) * ldz;                    // row 0 of every point: z0, then b~ = L^-T z0 in place
+  int rc = stage_leaf_lt(ctx, A, lda, Lt, N);
+  if (rc) return rc;
+  for (int x0 = 0; x0 < nx; x0 += chunk) {
+    const int cx = std::min(chunk, nx - x0);
+    rc = launch_cross_cov_dx(ctx, gm, theta, pinv, Xs + (int64_t)x0 * d, cx, Z, ldz);
+    if (rc) return rc;
+    rc = trsm_right_rec(ctx, A, lda, 0, dinv, 0, 0, Z, ldz, 0, cx * (d + 1), N);
+    if (rc) return rc;
+    rc = launch_predict_grad_rows(ctx, N, d, Z, ldz, cx, w, beta, varK, mu + x0, sig + x0, sig2_out ? sig2_out + x0 : nullptr,
+                                  dmudx + (int64_t)x0 * d, dsigdx + (int64_t)x0 * d, n_negative_dev);
+    if (rc) return rc;
+    rc = trsm_right_lower_rec(ctx, A, lda, dinv, Lt, 0, Z, ldb, cx, N, T);
+    if (rc) return rc;
+    rc = launch_predict_hess_batch(ctx, gm, theta, Xs + (int64_t)x0 * d, cx, alpha, Z, ldb, pinv, Z, ldz,
+                                   hess3 + (int64_t)x0 * 3 * d * d);
+    if (rc) return rc;
+  }
+  return 0;
+}
+
 }  // extern "C"
 
 namespace {

@@ -102,6 +102,10 @@ int launch_predict_grad_rows(const Ctx& ctx, int N, int d, const double* Z, int6
                              int* n_negative);
 int launch_predict_hess(const Ctx& ctx, const Geom& gm, const double* theta, const double* xs, const double* a,
                         const double* b, const double* Z, int64_t ldz, double* out);
+// nx test points at once: bt[x * ldb + c] holds L^-T z0 of point x (b = pinv .* bt), Z the (d + 1) solved rows per point
+// (ld ldz); out[nx, 3, d, d].  d <= 63.
+int launch_predict_hess_batch(const Ctx& ctx, const Geom& gm, const double* theta, const double* Xs, int nx, const double* a,
+                              const double* bt, int64_t ldb, const double* pinv, const double* Z, int64_t ldz, double* out);
 int launch_append_rhs(const Ctx& ctx, int N, int n, const double* y, const double* pinv, int64_t strideP, double* rows,
                       int64_t ld, int64_t strideRows);
 

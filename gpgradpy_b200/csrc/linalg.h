@@ -93,6 +93,13 @@ int chol_trap_inverse(const Ctx& ctx, double* A, int64_t lda, int64_t strideA, i
 // B (r x k) <- B * L^-T for an already factored k x k lower L (col0: global index of L's first column).
 int trsm_right_rec(const Ctx& ctx, const double* L, int64_t ldl, int64_t strideL, const double* Dinv, int64_t strideD,
                    int col0, double* B, int64_t ldb, int64_t strideB, int r, int k);
+// Lt[dinv_doubles(N)] <- the transposed diagonal blocks L_bb^T of a factor (row-major, ld LEAF, zeros elsewhere).
+int stage_leaf_lt(const Ctx& ctx, const double* L, int64_t ldl, double* Lt, int N);
+// B (r x k) <- B * L^-1 (rows against the lower factor, not transposed) for an already factored k x k lower L: the mirror
+// of trsm_right_rec (right block first, then the GEMM update of the left block).  Leaves multiply with the full Dinv blocks
+// and take one refinement step against the staged Lt blocks; T is r x LEAF scratch.
+int trsm_right_lower_rec(const Ctx& ctx, const double* L, int64_t ldl, const double* Dinv, const double* Lt, int col0,
+                         double* B, int64_t ldb, int r, int k, double* T);
 // Kinv (full symmetric N x N) = L^-T L^-1. U (N x N) receives L^-T in its upper triangle (its strictly lower part
 // outside the diagonal blocks is never written nor read).  Kinv doubles as scratch: while U is built its lower triangle
 // holds the transpose L^-1, so that every product of the inverse is an A * B^T with K-contiguous operands (TMA kernel).

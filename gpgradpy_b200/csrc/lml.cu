@@ -545,6 +545,203 @@ int launch_predict_hess(const Ctx& ctx, const Geom& gm, const double* theta, con
   return 0;
 }
 
+// Surrogate Hessians for a batch of test points: one CTA per point (blockIdx.x), the same three outputs per point as
+// predict_hess_kernel.  Summing that kernel's gradient entries over j gives, per training point p with value coefficient
+// c_p, gradient coefficients G_p[j] (zero where slot[p] < 0), s_p = sum_j th_j r_j G_p[j] and r = x_p - x*:
+//   H[i,k] = th_i th_k M[i,k] + delta_ik th_i W,   W = sum_p (2 f1 c_p + 4 f2 s_p),
+//   M[i,k] = sum_p (r_i q_k + r_k q_i),           q_j = 2 (f2 c_p + 2 f3 s_p) r_j + 4 f2 G_p[j],
+// so each radial profile is computed once per (test point, training point) pair: O(n d^2) per point instead of O(n d^3).
+// Applied with c, G from a = K^-1 (y - H beta) (-> d2mu/dx2) and from b = P^-1 L^-T z0 = K^-1 k* (-> term1).
+// term2[i,k] = z_i . z_k reads the point's d solved derivative rows once, in column tiles through shared memory.
+// Thread t owns the upper-triangle pairs e = t, t + 256, ... (d(d+1)/2 >= 256) or, for small d, pair t % P of the
+// point / column subset t / P; the subsets are summed in a fixed order.  Every entry is computed once for i <= k and
+// mirrored, so each Hessian is exactly symmetric.
+constexpr int HB_T = 256;     // threads per CTA
+constexpr int HB_TP = 64;     // training points per tile
+constexpr int HB_CT = 64;     // columns per term2 tile
+constexpr int HB_MAXI = 8;    // upper-triangle pairs per thread: d(d + 1) / 2 <= 8 * 256, d <= 63
+constexpr int HB_MAXD = 63;
+
+__host__ __device__ inline size_t hess_batch_smem_doubles(int d) {
+  const size_t tile = (size_t)HB_TP * (3 * d + 1), gram = (size_t)d * (HB_CT + 1);
+  return 2 * (size_t)d + 3 * HB_T + (tile > gram ? tile : gram);
+}
+
+__global__ void __launch_bounds__(HB_T)
+predict_hess_batch_kernel(Geom gm, const double* __restrict__ theta, const double* __restrict__ Xs,
+                          const double* __restrict__ a, const double* __restrict__ bt, int64_t ldb,
+                          const double* __restrict__ pinv, const double* __restrict__ Z, int64_t ldz,
+                          double* __restrict__ out) {
+  extern __shared__ double sm[];
+  __shared__ double sh[32];
+  const int d = gm.d, n = gm.n, ng = gm.ng, N = gm.N;
+  const int x = blockIdx.x, t = threadIdx.x;
+  bt += (int64_t)x * ldb;          // this point's solved row b~ = L^-T z0 (b = pinv .* b~)
+  double* xs = sm;                 // [d]
+  double* th = xs + d;             // [d]
+  double* red = th + d;            // [3][HB_T] subset partial sums
+  double* tile = red + 3 * HB_T;   // [HB_TP][3d + 1] (r | q_a | q_b) or [d][HB_CT + 1] (derivative rows)
+  const int P = d * (d + 1) / 2;
+  const int G = P >= HB_T ? 1 : HB_T / P;    // subsets of the point / column range
+  const int g = G > 1 ? t / P : 0;
+  const bool active = G == 1 || t < G * P;
+  const int e0 = G > 1 ? t % P : t;
+  const int nit = G > 1 ? 1 : HB_MAXI;
+  for (int j = t; j < d; j += HB_T) { xs[j] = Xs[(int64_t)x * d + j]; th[j] = theta[j]; }
+  int ii[HB_MAXI], kk[HB_MAXI];
+#pragma unroll
+  for (int m = 0; m < HB_MAXI; m++) {
+    int e = e0 + m * HB_T, i = 0;
+    if (m >= nit || e >= P) { ii[m] = kk[m] = -1; continue; }
+    while (e >= d - i) { e -= d - i; i++; }
+    ii[m] = i;
+    kk[m] = i + e;
+  }
+  double acc0[HB_MAXI], acc1[HB_MAXI], acc2[HB_MAXI];
+#pragma unroll
+  for (int m = 0; m < HB_MAXI; m++) acc0[m] = acc1[m] = acc2[m] = 0.0;
+
+  // ---- term2: Gram matrix of the d derivative rows z_1 .. z_d
+  const double* z0 = Z + (int64_t)x * (d + 1) * ldz;
+  constexpr int GLD = HB_CT + 1;
+  for (int c0 = 0; c0 < N; c0 += HB_CT) {
+    __syncthreads();
+    for (int e = t; e < d * HB_CT; e += HB_T) {
+      const int j = e / HB_CT, c = e % HB_CT;
+      tile[j * GLD + c] = (c0 + c < N) ? z0[(int64_t)(1 + j) * ldz + c0 + c] : 0.0;
+    }
+    __syncthreads();
+    if (active) {
+#pragma unroll
+      for (int m = 0; m < HB_MAXI; m++) {
+        if (ii[m] < 0) continue;
+        const double* zi = tile + ii[m] * GLD;
+        const double* zk = tile + kk[m] * GLD;
+        double s = acc2[m];
+        for (int c = g; c < HB_CT; c += G) s += zi[c] * zk[c];
+        acc2[m] = s;
+      }
+    }
+  }
+
+  // ---- d2mu/dx2 and term1: the closed-form contraction over the training points
+  const int TLD = 3 * d + 1;
+  double wa = 0.0, wb = 0.0;
+  for (int p0 = 0; p0 < n; p0 += HB_TP) {
+    __syncthreads();
+    if (t < HB_TP) {
+      double* rr = tile + t * TLD;
+      double* qa = rr + d;
+      double* qb = qa + d;
+      const int p = p0 + t;
+      if (p < n) {
+        const int sp = gm.slot ? gm.slot[p] : p;
+        const double* xp = gm.X + (int64_t)p * d;
+        double s = 0.0, sa = 0.0, sb = 0.0;
+        for (int j = 0; j < d; j++) {
+          const double r = xp[j] - xs[j], u = th[j] * r;
+          s += u * r;
+          double ga = 0.0, gb = 0.0;
+          if (sp >= 0) {
+            const int col = n + j * ng + sp;
+            ga = a[col];
+            gb = bt[col] * pinv[col];
+          }
+          sa += u * ga;
+          sb += u * gb;
+          rr[j] = r;
+          qa[j] = ga;
+          qb[j] = gb;
+        }
+        const RadialProfile ph = radial_profile(gm.ktype, gm.khp, s);
+        const double ca = a[p], cb = bt[p] * pinv[p];
+        const double ua = 2.0 * (ph.f2 * ca + 2.0 * ph.f3 * sa), ub = 2.0 * (ph.f2 * cb + 2.0 * ph.f3 * sb);
+        const double v = 4.0 * ph.f2;
+        for (int j = 0; j < d; j++) {
+          qa[j] = ua * rr[j] + v * qa[j];
+          qb[j] = ub * rr[j] + v * qb[j];
+        }
+        wa += 2.0 * ph.f1 * ca + 4.0 * ph.f2 * sa;
+        wb += 2.0 * ph.f1 * cb + 4.0 * ph.f2 * sb;
+      } else {
+        for (int j = 0; j < 3 * d; j++) rr[j] = 0.0;
+      }
+    }
+    __syncthreads();
+    if (active) {
+#pragma unroll
+      for (int m = 0; m < HB_MAXI; m++) {
+        if (ii[m] < 0) continue;
+        const int i = ii[m], k = kk[m];
+        double s0 = acc0[m], s1 = acc1[m];
+        for (int q = g; q < HB_TP; q += G) {
+          const double* rr = tile + q * TLD;
+          const double ri = rr[i], rk = rr[k];
+          s0 += ri * rr[d + k] + rk * rr[d + i];
+          s1 += ri * rr[2 * d + k] + rk * rr[2 * d + i];
+        }
+        acc0[m] = s0;
+        acc1[m] = s1;
+      }
+    }
+  }
+  wa = block_sum(wa, sh);
+  wb = block_sum(wb, sh);
+
+  // ---- sum the subsets in a fixed order, scale, mirror
+  if (G > 1) {
+    __syncthreads();
+    if (active) {
+      red[t] = acc0[0];
+      red[HB_T + t] = acc1[0];
+      red[2 * HB_T + t] = acc2[0];
+    }
+    __syncthreads();
+    if (t < P) {
+      double s0 = 0.0, s1 = 0.0, s2 = 0.0;
+      for (int q = 0; q < G; q++) {
+        s0 += red[q * P + t];
+        s1 += red[HB_T + q * P + t];
+        s2 += red[2 * HB_T + q * P + t];
+      }
+      acc0[0] = s0;
+      acc1[0] = s1;
+      acc2[0] = s2;
+    }
+  }
+  if (G == 1 || t < P) {
+    double* o = out + (int64_t)x * 3 * d * d;
+#pragma unroll
+    for (int m = 0; m < HB_MAXI; m++) {
+      if (ii[m] < 0) continue;
+      const int i = ii[m], k = kk[m];
+      const double tt = th[i] * th[k];
+      const double h0 = tt * acc0[m] + (i == k ? th[i] * wa : 0.0);
+      const double h1 = tt * acc1[m] + (i == k ? th[i] * wb : 0.0);
+      const double h2 = acc2[m];
+      o[i * d + k] = h0;
+      o[d * d + i * d + k] = h1;
+      o[2 * d * d + i * d + k] = h2;
+      if (i != k) {
+        o[k * d + i] = h0;
+        o[d * d + k * d + i] = h1;
+        o[2 * d * d + k * d + i] = h2;
+      }
+    }
+  }
+}
+
+int launch_predict_hess_batch(const Ctx& ctx, const Geom& gm, const double* theta, const double* Xs, int nx, const double* a,
+                              const double* bt, int64_t ldb, const double* pinv, const double* Z, int64_t ldz, double* out) {
+  if (nx <= 0) return 0;
+  if (gm.d > HB_MAXD) return -908;
+  const size_t smem = hess_batch_smem_doubles(gm.d) * sizeof(double);
+  if (smem > 48 * 1024) GEGP_SET_SMEM(predict_hess_batch_kernel, GEGP_MAX_DYN_SMEM);
+  predict_hess_batch_kernel<<<nx, HB_T, smem, ctx.stream>>>(gm, theta, Xs, a, bt, ldb, pinv, Z, ldz, out);
+  GEGP_CHECK_LAUNCH();
+  return 0;
+}
+
 int launch_predict_rows(const Ctx& ctx, int N, const double* Z, int64_t ldz, int nx, const double* w, double beta,
                         double varK, double* mu, double* sig, double* sig2, int* n_negative) {
   if (nx <= 0) return 0;

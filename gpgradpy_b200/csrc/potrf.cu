@@ -48,6 +48,57 @@ int trsm_right_rec(const Ctx& ctx, const double* L, int64_t ldl, int64_t strideL
                         k - k1);
 }
 
+// Lt block b (LEAF x LEAF, row-major, ld LEAF) <- L_bb^T with explicit zeros below the diagonal and outside a ragged last
+// block: the K-contiguous form of L_bb for the residual product of the leaf refinement below (the strict upper part of
+// the factor's diagonal blocks is never written by the factorisation, so it cannot be read as zeros).
+__global__ void __launch_bounds__(256)
+stage_leaf_lt_kernel(const double* __restrict__ L, int64_t ldl, double* __restrict__ Lt, int N) {
+  const int b0 = blockIdx.x * LEAF;
+  const int k = min(LEAF, N - b0);
+  double* dst = Lt + (int64_t)blockIdx.x * LEAF * LEAF;
+  for (int e = threadIdx.x; e < LEAF * LEAF; e += blockDim.x) {
+    const int i = e / LEAF, j = e % LEAF;   // dst[i][j] = L[b0 + j][b0 + i] for j >= i
+    dst[e] = (j >= i && j < k) ? L[(int64_t)(b0 + j) * ldl + b0 + i] : 0.0;
+  }
+}
+
+int stage_leaf_lt(const Ctx& ctx, const double* L, int64_t ldl, double* Lt, int N) {
+  if (N <= 0) return 0;
+  stage_leaf_lt_kernel<<<(N + LEAF - 1) / LEAF, 256, 0, ctx.stream>>>(L, ldl, Lt, N);
+  GEGP_CHECK_LAUNCH();
+  return 0;
+}
+
+// B (r x k) <- B * L^-1 for one leaf (k <= LEAF), with the explicit inverse L^-1 = Dinv^T and one refinement step:
+//   X1 = B Dinv^T ;  R = B - X1 L ;  X = X1 + R Dinv^T
+// T (r x LEAF, ld LEAF) is scratch; B holds R between the second and the third product and X at the end.
+static int leaf_trsm_lower_right(const Ctx& ctx, const double* Dinv, const double* Lt, double* B, int64_t ldb, int r, int k,
+                                 double* T) {
+  int rc = gemm_f64(ctx, gemm_args(B, ldb, Dinv, LEAF, T, LEAF, r, k, k, 1.0, 0.0, true));          // X1
+  if (rc) return rc;
+  rc = gemm_f64(ctx, gemm_args(T, LEAF, Lt, LEAF, B, ldb, r, k, k, -1.0, 1.0, true));               // R
+  if (rc) return rc;
+  rc = gemm_f64(ctx, gemm_args(B, ldb, Dinv, LEAF, T, LEAF, r, k, k, 1.0, 1.0, true));              // X1 + R Dinv^T
+  if (rc) return rc;
+  const cudaError_t e = cudaMemcpy2DAsync(B, (size_t)ldb * sizeof(double), T, LEAF * sizeof(double), (size_t)k * sizeof(double),
+                                          (size_t)r, cudaMemcpyDeviceToDevice, ctx.stream);
+  return e == cudaSuccess ? 0 : -1000 - (int)e;
+}
+
+int trsm_right_lower_rec(const Ctx& ctx, const double* L, int64_t ldl, const double* Dinv, const double* Lt, int col0,
+                         double* B, int64_t ldb, int r, int k, double* T) {
+  if (r <= 0 || k <= 0) return 0;
+  if (k <= LEAF)
+    return leaf_trsm_lower_right(ctx, dinv_block(Dinv, col0), dinv_block(Lt, col0), B, ldb, r, k, T);
+  // X = [X1 X2], L = [[L11 0],[L21 L22]]:  X2 = B2 L22^-1 ; B1 -= X2 L21 ; X1 = B1 L11^-1
+  const int k1 = split_point(k);
+  int rc = trsm_right_lower_rec(ctx, L + (int64_t)k1 * ldl + k1, ldl, Dinv, Lt, col0 + k1, B + k1, ldb, r, k - k1, T);
+  if (rc) return rc;
+  rc = gemm_f64(ctx, gemm_args(B + k1, ldb, L + (int64_t)k1 * ldl, ldl, B, ldb, r, k1, k - k1, -1.0, 1.0, false));
+  if (rc) return rc;
+  return trsm_right_lower_rec(ctx, L, ldl, Dinv, Lt, col0, B, ldb, r, k1, T);
+}
+
 // U = L^-T by levels: diagonal LEAF blocks first, then for block size bs = LEAF, 2*LEAF, ... every pair
 // (a = [s, s+bs), b = [s+bs, s+2bs)):  U_ab = -(U_aa * L_ba^T) * U_bb.  The product in parentheses is staged in the
 // upper triangle of T (the Kinv buffer, same coordinates as U_ab).  The LOWER triangle of T meanwhile collects

@@ -1295,10 +1295,7 @@ class GaussianProcess:
             mu, sig, sig2, dmudx, dsigdx, h3, nneg = bk.predict_hess(self._pred, x[0], varK)
             dmudx, dsigdx, h3 = dmudx.cpu().numpy()[None, :], dsigdx.cpu().numpy()[None, :], h3.cpu().numpy()
             d2mudx2 = h3[0][None, :, :]
-            d2sig2 = -2.0 * varK * (h3[1] + h3[2])                       # eval/GpEvalModel.py:366-371
-            s = float(sig.item())
-            s = np.nan if s == 0 else s                                  # :374-375
-            d2sigdx2 = ((d2sig2 - 2.0 * np.outer(dsigdx[0], dsigdx[0])) / (2.0 * s))[None, :, :]
+            d2sigdx2 = _d2sigdx2(h3[None], sig.cpu().numpy(), dsigdx, varK)
         elif calc_grad:
             mu, sig, sig2, dmudx, dsigdx, nneg = bk.predict_grad(self._pred, x, float(self.hp_vals.varK))
             dmudx, dsigdx = dmudx.cpu().numpy(), dsigdx.cpu().numpy()
@@ -1318,6 +1315,32 @@ class GaussianProcess:
                 d2mudx2, d2sigdx2 = d2mudx2[0, :, :], d2sigdx2[0, :, :]
         return mu, sig, dmudx, dsigdx, d2mudx2, d2sigdx2
 
+
+    def eval_model_hess_batch(self, x2model_in):
+        """(mu, sig, dmudx, dsigdx, d2mudx2 [nx, dim, dim], d2sigdx2 [nx, dim, dim]) at every row of x2model_in in one
+        chunked pass: what stacking eval_model(x[i:i+1], calc_grad=True, calc_hess=True) over i gives, for an optimiser
+        that takes Newton or trust-region steps on the surrogate from many starts at once.  Same guards as eval_model;
+        d2sigdx2 is NaN at a point where sig = 0 (eval/GpEvalModel.py:374-375)."""
+        assert self.KernEta_chofac is not None, "To evaluate the surr the Cholesky decomposition is required"
+        x = np.asarray(x2model_in, dtype=float)
+        if x.ndim == 1:
+            x = x[None, :]
+        elif x.ndim != 2:
+            raise Exception(f"x2model_in should be a 2d array but it has shape {x.shape}")
+        if not (self.hp_vals == self._hp_vals_model_setup):
+            raise Exception("Cannot change hp_vals between calling setup_eval_model() and eval_model()")
+        if self.b_use_data_scl:
+            x = self.DataScl.x_init_2_scl(x)
+        varK = float(self.hp_vals.varK)
+        mu, sig, sig2, dmudx, dsigdx, h3, nneg = bk.predict_hess_batch(self._pred, x, varK)
+        mu, sig, dmudx, dsigdx, h3 = (t.cpu().numpy() for t in (mu, sig, dmudx, dsigdx, h3))
+        d2mudx2 = h3[:, 0]
+        d2sigdx2 = _d2sigdx2(h3, sig, dsigdx, varK)
+        assert int(nneg.item()) == 0, ("The variance of the surr should be non-negative but min(sig2_wo_sigK) = "
+                                       f"{float(sig2.min().item())}")
+        if self.b_use_data_scl:
+            mu, sig, dmudx, dsigdx, d2mudx2, d2sigdx2 = self.data_scl_2_init(mu, sig, dmudx, dsigdx, d2mudx2, d2sigdx2)
+        return mu, sig, dmudx, dsigdx, d2mudx2, d2sigdx2
 
     def eval_model_var(self, x2model_in, calc_grad=False, calc_hess=False, squeeze_nx=False):
         """(sig2, dsig2dx, None) -- eval/GpEvalModel.py:200-317: posterior variance varK (1 - k*^T K^-1 k*) and its
@@ -1351,6 +1374,15 @@ class GaussianProcess:
             if calc_grad:
                 dsig2dx = dsig2dx[0, :]
         return sig2, dsig2dx, None
+
+
+def _d2sigdx2(h3, sig, dsigdx, varK):
+    """d2sig/dx2 [nx, d, d] from the Hessian slabs h3 [nx, 3, d, d] (d2mu, term1, term2), sig [nx] and dsigdx [nx, d]
+    (eval/GpEvalModel.py:366-375): d2sig2 = -2 varK (term1 + term2), d2sig = (d2sig2 - 2 dsig dsig^T) / (2 sig), NaN where
+    sig = 0."""
+    d2sig2 = -2.0 * varK * (h3[:, 1] + h3[:, 2])
+    s = np.where(sig == 0, np.nan, sig)
+    return (d2sig2 - 2.0 * (dsigdx[:, :, None] * dsigdx[:, None, :])) / (2.0 * s[:, None, None])
 
 
 class _DeviceRtensor:

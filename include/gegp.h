@@ -191,6 +191,21 @@ int gegp_predict_hess(int n, int n_g, int d, const double* X, const int32_t* gra
                       double* dmudx, double* dsigdx, double* hess3, int* n_negative_dev, void* work, size_t work_bytes,
                       void* stream);
 
+/* Surrogate Hessians at nx test points Xs[nx, d] in one chunked pass (a second-order optimiser of an acquisition function
+ * run from many starts at once).  Arguments as gegp_predict_hess with xs replaced by (Xs, nx); outputs mu[nx], sig[nx],
+ * sig2_out[nx] (optional), dmudx[nx, d], dsigdx[nx, d] and hess3[nx, 3, d, d], each point's slab with the meaning of the
+ * one-point call (d2mu/dx2, term1, term2); n_negative_dev counts the negative sig2 entries.  Per chunk of points: one
+ * cross-covariance launch, one forward solve of the (d + 1) rows of every point, one back substitution of all the points'
+ * K^-1 k* at once and one contraction launch.  mu, sig, sig2, dmudx and dsigdx are those of gegp_predict_grad for the same
+ * chunk; hess3 agrees with the one-point call to rounding (its sums run in another order) and every d x d slab is exactly
+ * symmetric.  d <= 63 (else -3).  work >= gegp_dinv_doubles(N) * 8 bytes, plus ((d + 1) * gegp_ld(N) + 128) * 8 bytes per
+ * point of a chunk; the chunk is as many points as fit (at least one, else -25).  nx = 0 writes nothing. */
+int gegp_predict_hess_batch(int n, int n_g, int d, const double* X, const int32_t* grad_slot, const double* theta, int kernel,
+                            double kernel_hp, const double* A, int64_t lda, const double* dinv, const double* p,
+                            const double* alpha, int mode, double beta, double varK, const double* Xs, int nx, double* mu,
+                            double* sig, double* sig2_out, double* dmudx, double* dsigdx, double* hess3, int* n_negative_dev,
+                            void* work, size_t work_bytes, void* stream);
+
 /* Where gegp_lml_eval keeps its per-candidate arrays inside `work` (candidate 0; candidate c adds
  * c * per_candidate_doubles), so that a caller can go on working with the factor and the explicit inverse of the
  * evaluation it has just run (condition number, below).  out[8] = { header_bytes, ld, per_candidate_doubles,
