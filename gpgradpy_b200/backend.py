@@ -359,21 +359,29 @@ def predict_setup(X, y, theta, beta, *, n_g=None, slot=None, noise=None, mode=L.
     return PredictState(A, dinv, p, info, alpha, n, n_g, d, N, X, slot, theta, mode, float(beta), (kid, khp))
 
 
+def _outputs(*shapes):
+    """Uninitialised float64 device tensors of the given shapes, then the zeroed n_negative counter."""
+    dev = device()
+    return [torch.empty(s, dtype=F64, device=dev) for s in shapes] + [torch.zeros(1, dtype=torch.int32, device=dev)]
+
+
+def _chunk_workspace(nx: int, per_x: int, chunk_bytes: int, fixed: int = 0):
+    """(workspace, its size in bytes) for chunks of as many of the nx points as chunk_bytes hold, at least one."""
+    cx = max(1, min(nx, (chunk_bytes - fixed) // per_x))
+    nbytes = fixed + cx * per_x
+    return workspace(nbytes), nbytes
+
+
 def predict(st: PredictState, Xs, varK: float, *, chunk_bytes: int = 1 << 30):
     """gegp_predict -> (mu, sig, sig2, n_negative) device tensors."""
     lib = L.load()
     Xs = to_dev(Xs)
     nx = Xs.shape[0]
-    mu = torch.empty(nx, dtype=F64, device=device())
-    sig = torch.empty(nx, dtype=F64, device=device())
-    sig2 = torch.empty(nx, dtype=F64, device=device())
-    nneg = torch.zeros(1, dtype=torch.int32, device=device())
-    row_bytes = ld_of(st.N) * 8
-    cx = max(1, min(nx, chunk_bytes // row_bytes))
-    ws = workspace(cx * row_bytes)
+    mu, sig, sig2, nneg = _outputs(nx, nx, nx)
+    ws, nbytes = _chunk_workspace(nx, ld_of(st.N) * 8, chunk_bytes)
     rc = lib.gegp_predict(st.n, st.n_g, st.d, _p(st.X), _p(st.slot), _p(st.theta), st.kid, st.khp, _p(st.A), st.A.stride(0), _p(st.dinv),
                           _p(st.p), int(st.mode), st.beta, float(varK), _p(Xs), nx, _p(mu), _p(sig), _p(sig2), _p(nneg), _p(ws),
-                          cx * row_bytes, _stream())
+                          nbytes, _stream())
     _check(rc, "gegp_predict")
     return mu, sig, sig2, nneg
 
@@ -383,16 +391,11 @@ def predict_grad(st: PredictState, Xs, varK: float, *, chunk_bytes: int = 1 << 3
     lib = L.load()
     Xs = to_dev(Xs)
     nx, d = Xs.shape[0], st.d
-    dev = device()
-    mu, sig, sig2 = (torch.empty(nx, dtype=F64, device=dev) for _ in range(3))
-    dmu, dsg = (torch.empty((nx, d), dtype=F64, device=dev) for _ in range(2))
-    nneg = torch.zeros(1, dtype=torch.int32, device=dev)
-    per_x = (d + 1) * ld_of(st.N) * 8
-    cx = max(1, min(nx, chunk_bytes // per_x))
-    ws = workspace(cx * per_x)
+    mu, sig, sig2, dmu, dsg, nneg = _outputs(nx, nx, nx, (nx, d), (nx, d))
+    ws, nbytes = _chunk_workspace(nx, (d + 1) * ld_of(st.N) * 8, chunk_bytes)
     rc = lib.gegp_predict_grad(st.n, st.n_g, st.d, _p(st.X), _p(st.slot), _p(st.theta), st.kid, st.khp, _p(st.A), st.A.stride(0),
                                _p(st.dinv), _p(st.p), int(st.mode), st.beta, float(varK), _p(Xs), nx, _p(mu), _p(sig),
-                               _p(sig2), _p(dmu), _p(dsg), _p(nneg), _p(ws), cx * per_x, _stream())
+                               _p(sig2), _p(dmu), _p(dsg), _p(nneg), _p(ws), nbytes, _stream())
     _check(rc, "gegp_predict_grad")
     return mu, sig, sig2, dmu, dsg, nneg
 
@@ -403,11 +406,7 @@ def predict_hess(st: PredictState, xs, varK: float):
     xs = to_dev(xs).reshape(-1)
     d = st.d
     assert xs.numel() == d and st.alpha is not None
-    dev = device()
-    mu, sig, sig2 = (torch.empty(1, dtype=F64, device=dev) for _ in range(3))
-    dmu, dsg = (torch.empty(d, dtype=F64, device=dev) for _ in range(2))
-    h3 = torch.empty((3, d, d), dtype=F64, device=dev)
-    nneg = torch.zeros(1, dtype=torch.int32, device=dev)
+    mu, sig, sig2, dmu, dsg, h3, nneg = _outputs(1, 1, 1, d, d, (3, d, d))
     nbytes = (d + 2) * ld_of(st.N) * 8
     ws = workspace(nbytes)
     rc = lib.gegp_predict_hess(st.n, st.n_g, st.d, _p(st.X), _p(st.slot), _p(st.theta), st.kid, st.khp, _p(st.A), st.A.stride(0),
@@ -429,17 +428,12 @@ def predict_hess_batch(st: PredictState, Xs, varK: float, *, chunk_bytes: int = 
     Xs = to_dev(Xs)
     nx, d = Xs.shape[0], st.d
     assert Xs.ndim == 2 and Xs.shape[1] == d and st.alpha is not None
-    dev = device()
-    mu, sig, sig2 = (torch.empty(nx, dtype=F64, device=dev) for _ in range(3))
-    dmu, dsg = (torch.empty((nx, d), dtype=F64, device=dev) for _ in range(2))
-    h3 = torch.empty((nx, 3, d, d), dtype=F64, device=dev)
-    nneg = torch.zeros(1, dtype=torch.int32, device=dev)
+    out = _outputs(nx, nx, nx, (nx, d), (nx, d), (nx, 3, d, d))
     if nx == 0:
-        return mu, sig, sig2, dmu, dsg, h3, nneg
-    per_x = predict_hess_batch_bytes(st.N, d, 1) - predict_hess_batch_bytes(st.N, d, 0)
-    cx = max(1, min(nx, (chunk_bytes - predict_hess_batch_bytes(st.N, d, 0)) // per_x))
-    nbytes = predict_hess_batch_bytes(st.N, d, cx)
-    ws = workspace(nbytes)
+        return tuple(out)
+    mu, sig, sig2, dmu, dsg, h3, nneg = out
+    fixed = predict_hess_batch_bytes(st.N, d, 0)
+    ws, nbytes = _chunk_workspace(nx, predict_hess_batch_bytes(st.N, d, 1) - fixed, chunk_bytes, fixed)
     rc = lib.gegp_predict_hess_batch(st.n, st.n_g, st.d, _p(st.X), _p(st.slot), _p(st.theta), st.kid, st.khp, _p(st.A),
                                      st.A.stride(0), _p(st.dinv), _p(st.p), _p(st.alpha), int(st.mode), st.beta, float(varK),
                                      _p(Xs), nx, _p(mu), _p(sig), _p(sig2), _p(dmu), _p(dsg), _p(h3), _p(nneg), _p(ws), nbytes,

@@ -119,6 +119,52 @@ Geom make_geom(int n, int n_g, int d, const double* X, const int32_t* grad_slot,
   return Geom{n, n_g, d, n + n_g * d, X, (n_g == n) ? nullptr : grad_slot, kernel, kernel_hp, kernel_hp_batch};
 }
 
+// The factored training set that gegp_predict_setup leaves behind, as the posterior entry points read it.
+struct Posterior {
+  Geom gm;
+  const double* theta;
+  const double* A;      // factor L (lower), ld lda
+  int64_t lda;
+  const double* dinv;   // inverted diagonal blocks of L
+  const double* pinv;   // P^-1
+  const double* w;      // row N of A: L^-1 P^-1 (y - H beta)
+};
+
+// The arguments every posterior entry point starts with, checked in order: -1 geometry, -50 kernel, -4 X, -5 grad_slot,
+// -6 theta, -7 A, -8 lda, -9 dinv, -10 p.
+int posterior_args(int n, int n_g, int d, const double* X, const int32_t* grad_slot, const double* theta, int kernel,
+                   double kernel_hp, const double* A, int64_t lda, const double* dinv, const double* p, Posterior* ps) {
+  if (bad_geom(n, n_g, d)) return -1;
+  if (bad_kernel(kernel, kernel_hp)) return -50;
+  if (!X) return -4;
+  if (n_g != n && !grad_slot) return -5;
+  if (!theta) return -6;
+  if (!A) return -7;
+  const int N = n + n_g * d;
+  if (lda < N || (lda & 1)) return -8;
+  if (!dinv) return -9;
+  if (!p) return -10;
+  *ps = Posterior{make_geom(n, n_g, d, X, grad_slot, kernel, kernel_hp), theta, A, lda, dinv, p + N, A + (int64_t)N * lda};
+  return 0;
+}
+
+// Test points x0 .. x0 + cx - 1 of Xs: their cross covariances k* (and dk*/dx when dmu is given: d + 1 rows per point)
+// into Z, the forward solve Z := L^-1 P^-1 Z in place, then mu, sig, sig2 (and dmu, dsig) of those points.
+int posterior_chunk(const Ctx& ctx, const Posterior& ps, double beta, double varK, const double* Xs, int x0, int cx,
+                    double* Z, int64_t ldz, double* mu, double* sig, double* sig2, double* dmu, double* dsig,
+                    int* n_negative) {
+  const int d = ps.gm.d, N = ps.gm.N, dr = dmu ? d : 0;
+  const double* xs = Xs + (int64_t)x0 * d;
+  int rc = dmu ? launch_cross_cov_dx(ctx, ps.gm, ps.theta, ps.pinv, xs, cx, Z, ldz)
+               : launch_cross_cov(ctx, ps.gm, ps.theta, ps.pinv, xs, cx, Z, ldz);
+  if (rc) return rc;
+  rc = trsm_right_rec(ctx, ps.A, ps.lda, 0, ps.dinv, 0, 0, Z, ldz, 0, cx * (dr + 1), N);
+  if (rc) return rc;
+  return launch_predict_grad_rows(ctx, N, dr, Z, ldz, cx, ps.w, beta, varK, mu + x0, sig + x0, sig2 ? sig2 + x0 : nullptr,
+                                  dmu ? dmu + (int64_t)x0 * d : nullptr, dsig ? dsig + (int64_t)x0 * d : nullptr,
+                                  n_negative);
+}
+
 }  // namespace
 
 extern "C" {
@@ -552,37 +598,22 @@ int gegp_predict(int n, int n_g, int d, const double* X, const int32_t* grad_slo
                  int64_t lda, const double* dinv, const double* p, int mode, double beta, double varK, const double* Xs,
                  int nx, double* mu,
                  double* sig, double* sig2_out, int* n_negative_dev, void* work, size_t work_bytes, void* stream) {
-  if (bad_geom(n, n_g, d)) return -1;
-  if (bad_kernel(kernel, kernel_hp)) return -50;
-  if (!X) return -4;
-  if (n_g != n && !grad_slot) return -5;
-  if (!theta) return -6;
-  if (!A) return -7;
-  const int N = n + n_g * d;
-  if (lda < N || (lda & 1)) return -8;
-  if (!dinv) return -9;
-  if (!p) return -10;
+  Posterior ps;
+  int rc = posterior_args(n, n_g, d, X, grad_slot, theta, kernel, kernel_hp, A, lda, dinv, p, &ps);
+  if (rc) return rc;
   if (!Xs || nx < 0) return -14;
   if (!mu) return -16;
   if (!sig) return -17;
   if (!work || (reinterpret_cast<uintptr_t>(work) & 15)) return -20;
   (void)mode;
-  const int64_t ldz = gegp_ld(N);
+  const int64_t ldz = gegp_ld(ps.gm.N);
   const int chunk = (int)std::min<size_t>((size_t)nx, work_bytes / (ldz * sizeof(double)));
   if (nx > 0 && chunk < 1) return -21;
   Ctx ctx{(cudaStream_t)stream, 1};
-  const Geom gm = make_geom(n, n_g, d, X, grad_slot, kernel, kernel_hp);
-  const double* pinv = p + N;
-  const double* w = A + (int64_t)N * lda;
   double* Z = reinterpret_cast<double*>(work);
   for (int x0 = 0; x0 < nx; x0 += chunk) {
-    const int cx = std::min(chunk, nx - x0);
-    int rc = launch_cross_cov(ctx, gm, theta, pinv, Xs + (int64_t)x0 * d, cx, Z, ldz);
-    if (rc) return rc;
-    rc = trsm_right_rec(ctx, A, lda, 0, dinv, 0, 0, Z, ldz, 0, cx, N);
-    if (rc) return rc;
-    rc = launch_predict_rows(ctx, N, Z, ldz, cx, w, beta, varK, mu + x0, sig + x0, sig2_out ? sig2_out + x0 : nullptr,
-                             n_negative_dev);
+    rc = posterior_chunk(ctx, ps, beta, varK, Xs, x0, std::min(chunk, nx - x0), Z, ldz, mu, sig, sig2_out, nullptr,
+                         nullptr, n_negative_dev);
     if (rc) return rc;
   }
   return 0;
@@ -592,16 +623,9 @@ int gegp_predict_grad(int n, int n_g, int d, const double* X, const int32_t* gra
                       const double* A, int64_t lda, const double* dinv, const double* p, int mode, double beta,
                       double varK, const double* Xs, int nx, double* mu, double* sig, double* sig2_out, double* dmudx,
                       double* dsigdx, int* n_negative_dev, void* work, size_t work_bytes, void* stream) {
-  if (bad_geom(n, n_g, d)) return -1;
-  if (bad_kernel(kernel, kernel_hp)) return -50;
-  if (!X) return -4;
-  if (n_g != n && !grad_slot) return -5;
-  if (!theta) return -6;
-  if (!A) return -7;
-  const int N = n + n_g * d;
-  if (lda < N || (lda & 1)) return -8;
-  if (!dinv) return -9;
-  if (!p) return -10;
+  Posterior ps;
+  int rc = posterior_args(n, n_g, d, X, grad_slot, theta, kernel, kernel_hp, A, lda, dinv, p, &ps);
+  if (rc) return rc;
   if (!Xs || nx < 0) return -14;
   if (!mu) return -16;
   if (!sig) return -17;
@@ -609,24 +633,15 @@ int gegp_predict_grad(int n, int n_g, int d, const double* X, const int32_t* gra
   if (!dsigdx) return -20;
   if (!work || (reinterpret_cast<uintptr_t>(work) & 15)) return -22;
   (void)mode;
-  const int64_t ldz = gegp_ld(N);
+  const int64_t ldz = gegp_ld(ps.gm.N);
   const size_t per_x = (size_t)(d + 1) * ldz * sizeof(double);
   const int chunk = (int)std::min<size_t>((size_t)nx, work_bytes / per_x);
   if (nx > 0 && chunk < 1) return -23;
   Ctx ctx{(cudaStream_t)stream, 1};
-  const Geom gm = make_geom(n, n_g, d, X, grad_slot, kernel, kernel_hp);
-  const double* pinv = p + N;
-  const double* w = A + (int64_t)N * lda;
   double* Z = reinterpret_cast<double*>(work);
   for (int x0 = 0; x0 < nx; x0 += chunk) {
-    const int cx = std::min(chunk, nx - x0);
-    int rc = launch_cross_cov_dx(ctx, gm, theta, pinv, Xs + (int64_t)x0 * d, cx, Z, ldz);
-    if (rc) return rc;
-    rc = trsm_right_rec(ctx, A, lda, 0, dinv, 0, 0, Z, ldz, 0, cx * (d + 1), N);
-    if (rc) return rc;
-    rc = launch_predict_grad_rows(ctx, N, d, Z, ldz, cx, w, beta, varK, mu + x0, sig + x0,
-                                  sig2_out ? sig2_out + x0 : nullptr, dmudx + (int64_t)x0 * d, dsigdx + (int64_t)x0 * d,
-                                  n_negative_dev);
+    rc = posterior_chunk(ctx, ps, beta, varK, Xs, x0, std::min(chunk, nx - x0), Z, ldz, mu, sig, sig2_out, dmudx, dsigdx,
+                         n_negative_dev);
     if (rc) return rc;
   }
   return 0;
@@ -637,16 +652,9 @@ int gegp_predict_hess(int n, int n_g, int d, const double* X, const int32_t* gra
                       double beta, double varK, const double* xs, double* mu, double* sig, double* sig2_out,
                       double* dmudx, double* dsigdx, double* hess3, int* n_negative_dev, void* work, size_t work_bytes,
                       void* stream) {
-  if (bad_geom(n, n_g, d)) return -1;
-  if (bad_kernel(kernel, kernel_hp)) return -50;
-  if (!X) return -4;
-  if (n_g != n && !grad_slot) return -5;
-  if (!theta) return -6;
-  if (!A) return -7;
-  const int N = n + n_g * d;
-  if (lda < N || (lda & 1)) return -8;
-  if (!dinv) return -9;
-  if (!p) return -10;
+  Posterior ps;
+  int rc = posterior_args(n, n_g, d, X, grad_slot, theta, kernel, kernel_hp, A, lda, dinv, p, &ps);
+  if (rc) return rc;
   if (!alpha) return -11;
   if (!xs) return -15;
   if (!mu) return -16;
@@ -656,27 +664,20 @@ int gegp_predict_hess(int n, int n_g, int d, const double* X, const int32_t* gra
   if (!hess3) return -21;
   if (!work || (reinterpret_cast<uintptr_t>(work) & 15)) return -23;
   (void)mode;
+  const int N = ps.gm.N;
   const int64_t ldz = gegp_ld(N);
   if (work_bytes < (size_t)(d + 2) * ldz * sizeof(double)) return -24;
   Ctx ctx{(cudaStream_t)stream, 1};
-  const Geom gm = make_geom(n, n_g, d, X, grad_slot, kernel, kernel_hp);
-  const double* pinv = p + N;
-  const double* w = A + (int64_t)N * lda;
   double* Z = reinterpret_cast<double*>(work);
-  double* bvec = Z + (int64_t)(d + 1) * ldz;          // K^-1 k* (un-preconditioned)
-  int rc = launch_cross_cov_dx(ctx, gm, theta, pinv, xs, 1, Z, ldz);
+  double* bt = Z + (int64_t)(d + 1) * ldz;             // L^-T z0 (K^-1 k* = P^-1 bt)
+  rc = posterior_chunk(ctx, ps, beta, varK, xs, 0, 1, Z, ldz, mu, sig, sig2_out, dmudx, dsigdx, n_negative_dev);
   if (rc) return rc;
-  rc = trsm_right_rec(ctx, A, lda, 0, dinv, 0, 0, Z, ldz, 0, d + 1, N);
-  if (rc) return rc;
-  rc = launch_predict_grad_rows(ctx, N, d, Z, ldz, 1, w, beta, varK, mu, sig, sig2_out, dmudx, dsigdx, n_negative_dev);
-  if (rc) return rc;
-  cudaError_t e = cudaMemcpyAsync(bvec, Z, (size_t)N * sizeof(double), cudaMemcpyDeviceToDevice, ctx.stream);
+  cudaError_t e = cudaMemcpyAsync(bt, Z, (size_t)N * sizeof(double), cudaMemcpyDeviceToDevice, ctx.stream);
   if (e != cudaSuccess) return -1000 - (int)e;
-  rc = trsv_lower_trans(ctx, A, lda, 0, dinv, 0, bvec, ldz, 0, N, 1);   // L^-T z0
+  // one row: a single trsv launch per leaf, where trsm_right_lower_rec would issue several
+  rc = trsv_lower_trans(ctx, A, lda, 0, dinv, 0, bt, ldz, 0, N, 1);
   if (rc) return rc;
-  rc = launch_scale_vec(ctx, N, bvec, 0, pinv, 0, bvec, 0);              // P^-1 .
-  if (rc) return rc;
-  return launch_predict_hess(ctx, gm, theta, xs, alpha, bvec, Z, ldz, hess3);
+  return launch_predict_hess_batch(ctx, ps.gm, theta, xs, 1, alpha, bt, ldz, ps.pinv, Z, ldz, hess3);
 }
 
 int gegp_predict_hess_batch(int n, int n_g, int d, const double* X, const int32_t* grad_slot, const double* theta, int kernel,
@@ -684,17 +685,10 @@ int gegp_predict_hess_batch(int n, int n_g, int d, const double* X, const int32_
                             const double* alpha, int mode, double beta, double varK, const double* Xs, int nx, double* mu,
                             double* sig, double* sig2_out, double* dmudx, double* dsigdx, double* hess3, int* n_negative_dev,
                             void* work, size_t work_bytes, void* stream) {
-  if (bad_geom(n, n_g, d)) return -1;
-  if (d > 63) return -3;                       // the contraction kernel keeps d (d + 1) / 2 <= 2048 pairs per CTA
-  if (bad_kernel(kernel, kernel_hp)) return -50;
-  if (!X) return -4;
-  if (n_g != n && !grad_slot) return -5;
-  if (!theta) return -6;
-  if (!A) return -7;
-  const int N = n + n_g * d;
-  if (lda < N || (lda & 1)) return -8;
-  if (!dinv) return -9;
-  if (!p) return -10;
+  if (!bad_geom(n, n_g, d) && hess_batch_tile_height(d) == 0) return -3;   // the contraction's tiles exceed shared memory
+  Posterior ps;
+  int rc = posterior_args(n, n_g, d, X, grad_slot, theta, kernel, kernel_hp, A, lda, dinv, p, &ps);
+  if (rc) return rc;
   if (!alpha) return -11;
   if (!Xs) return -15;
   if (nx < 0) return -16;
@@ -705,6 +699,7 @@ int gegp_predict_hess_batch(int n, int n_g, int d, const double* X, const int32_
   if (!hess3) return -22;
   if (!work || (reinterpret_cast<uintptr_t>(work) & 15)) return -24;
   (void)mode;
+  const int N = ps.gm.N;
   const int64_t ldz = gegp_ld(N);
   const size_t fixed = (size_t)dinv_doubles(N) * sizeof(double);
   const size_t per_x = ((size_t)(d + 1) * ldz + LEAF) * sizeof(double);
@@ -712,27 +707,19 @@ int gegp_predict_hess_batch(int n, int n_g, int d, const double* X, const int32_
   if (nx > 0 && chunk < 1) return -25;
   if (nx == 0) return 0;
   Ctx ctx{(cudaStream_t)stream, 1};
-  const Geom gm = make_geom(n, n_g, d, X, grad_slot, kernel, kernel_hp);
-  const double* pinv = p + N;
-  const double* w = A + (int64_t)N * lda;
   double* Lt = reinterpret_cast<double*>(work);                 // transposed diagonal blocks of the factor
   double* Z = Lt + dinv_doubles(N);                              // (d + 1) solved rows per point
   double* T = Z + (int64_t)chunk * (d + 1) * ldz;                // leaf scratch of the back substitution, chunk x LEAF
   const int64_t ldb = (int64_t)(d + 1) * ldz;                    // row 0 of every point: z0, then b~ = L^-T z0 in place
-  int rc = stage_leaf_lt(ctx, A, lda, Lt, N);
+  rc = stage_leaf_lt(ctx, A, lda, Lt, N);
   if (rc) return rc;
   for (int x0 = 0; x0 < nx; x0 += chunk) {
     const int cx = std::min(chunk, nx - x0);
-    rc = launch_cross_cov_dx(ctx, gm, theta, pinv, Xs + (int64_t)x0 * d, cx, Z, ldz);
-    if (rc) return rc;
-    rc = trsm_right_rec(ctx, A, lda, 0, dinv, 0, 0, Z, ldz, 0, cx * (d + 1), N);
-    if (rc) return rc;
-    rc = launch_predict_grad_rows(ctx, N, d, Z, ldz, cx, w, beta, varK, mu + x0, sig + x0, sig2_out ? sig2_out + x0 : nullptr,
-                                  dmudx + (int64_t)x0 * d, dsigdx + (int64_t)x0 * d, n_negative_dev);
+    rc = posterior_chunk(ctx, ps, beta, varK, Xs, x0, cx, Z, ldz, mu, sig, sig2_out, dmudx, dsigdx, n_negative_dev);
     if (rc) return rc;
     rc = trsm_right_lower_rec(ctx, A, lda, dinv, Lt, 0, Z, ldb, cx, N, T);
     if (rc) return rc;
-    rc = launch_predict_hess_batch(ctx, gm, theta, Xs + (int64_t)x0 * d, cx, alpha, Z, ldb, pinv, Z, ldz,
+    rc = launch_predict_hess_batch(ctx, ps.gm, theta, Xs + (int64_t)x0 * d, cx, alpha, Z, ldb, ps.pinv, Z, ldz,
                                    hess3 + (int64_t)x0 * 3 * d * d);
     if (rc) return rc;
   }

@@ -97,13 +97,14 @@ int launch_cross_cov(const Ctx& ctx, const Geom& gm, const double* theta, const 
                      double* out, int64_t ld);
 int launch_cross_cov_dx(const Ctx& ctx, const Geom& gm, const double* theta, const double* pinv, const double* Xs, int nx,
                         double* out, int64_t ld);
+// mu, sig, sig2 of nx points from their (d + 1) solved rows each (ld ldz), and dmu, dsig [nx, d] when d > 0
 int launch_predict_grad_rows(const Ctx& ctx, int N, int d, const double* Z, int64_t ldz, int nx, const double* w,
                              double beta, double varK, double* mu, double* sig, double* sig2, double* dmu, double* dsig,
                              int* n_negative);
-int launch_predict_hess(const Ctx& ctx, const Geom& gm, const double* theta, const double* xs, const double* a,
-                        const double* b, const double* Z, int64_t ldz, double* out);
+// Training points per shared-memory tile of the Hessian contraction at dimension d; 0 where its tiles cannot fit.
+int hess_batch_tile_height(int d);
 // nx test points at once: bt[x * ldb + c] holds L^-T z0 of point x (b = pinv .* bt), Z the (d + 1) solved rows per point
-// (ld ldz); out[nx, 3, d, d].  d <= 63.
+// (ld ldz); out[nx, 3, d, d].  -908 where hess_batch_tile_height(d) = 0.
 int launch_predict_hess_batch(const Ctx& ctx, const Geom& gm, const double* theta, const double* Xs, int nx, const double* a,
                               const double* bt, int64_t ldb, const double* pinv, const double* Z, int64_t ldz, double* out);
 int launch_append_rhs(const Ctx& ctx, int N, int n, const double* y, const double* pinv, int64_t strideP, double* rows,
@@ -117,8 +118,6 @@ int launch_lml_grad(const Ctx& ctx, const Geom& gm, const double* theta, int64_t
                     int64_t ldk, int64_t strideK, const double* alpha_t, int64_t strideAlpha, const double* pinv,
                     int64_t strideP, int mode, double eta, int noisy, const double* varK, double pnlt_grad, double* partial,
                     int64_t stridePartial, double* out, int64_t strideOut, int quad = 0);
-int launch_predict_rows(const Ctx& ctx, int N, const double* Z, int64_t ldz, int nx, const double* w, double beta,
-                        double varK, double* mu, double* sig, double* sig2, int* n_negative);
 
 size_t lml_grad_partial_doubles(int n, int d);
 

@@ -395,36 +395,10 @@ int launch_lml_grad(const Ctx& ctx, const Geom& gm, const double* theta, int64_t
   return 0;
 }
 
-// ------------------------------------------------------------------------------------------------
-// predict rows: Z[x,:] = L^-1 P^-1 k*(x) ; mu = beta + Z_x . w ; sig2 = 1 - |Z_x|^2
-// ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256)
-predict_rows_kernel(int N, const double* __restrict__ Z, int64_t ldz, int nx, const double* __restrict__ w,
-                    double beta, double varK, double* __restrict__ mu, double* __restrict__ sig,
-                    double* __restrict__ sig2, int* __restrict__ n_negative) {
-  __shared__ double sh[32];
-  const int x = blockIdx.x;
-  const double* zr = Z + (int64_t)x * ldz;
-  double d1 = 0, d2 = 0;
-  for (int i = threadIdx.x; i < N; i += blockDim.x) {
-    const double v = zr[i];
-    d1 += v * w[i];
-    d2 += v * v;
-  }
-  d1 = block_sum(d1, sh);
-  d2 = block_sum(d2, sh);
-  if (threadIdx.x == 0) {
-    const double s2 = 1.0 - d2;
-    mu[x] = beta + d1;
-    if (sig2) sig2[x] = s2;
-    if (s2 < 0 && n_negative) atomicAdd(n_negative, 1);
-    sig[x] = sqrt(fmax(s2, 0.0)) * sqrt(varK);
-  }
-}
-
 // Posterior with x-derivatives: per test point the d + 1 solved rows z0 = L^-1 P^-1 k*, z_j = L^-1 P^-1 dk*/dx_j give
 //   mu = beta + z0.w ; sig2 = 1 - |z0|^2 ; dmu/dx_j = z_j.w ; dsig/dx_j = -varK (z_j.z0) / sig   (0 where sig = 0)
-// (eval/GpEvalModel.py:319-354: calc_dmudx, calc_dsigdx).
+// (eval/GpEvalModel.py:319-354: calc_dmudx, calc_dsigdx).  With d = 0 (one row per point, dmu and dsig unused) it is
+// the plain posterior of gegp_predict.
 __global__ void __launch_bounds__(256)
 predict_grad_rows_kernel(int N, int d, const double* __restrict__ Z, int64_t ldz, const double* __restrict__ w,
                          double beta, double varK, double* __restrict__ mu, double* __restrict__ sig,
@@ -478,99 +452,45 @@ int launch_predict_grad_rows(const Ctx& ctx, int N, int d, const double* Z, int6
   return 0;
 }
 
-// Surrogate Hessian contractions for ONE test point (eval/GpEvalModel.py:175-180, 356-382; the second x-derivatives of
-// the cross covariance are kernel/KernelSqExp.py:66-88 for value entries and :432-468 for gradient entries).
-// CTA (i, k):  out[0][i,k] = sum_col d2k*[i,k,col] a[col]    (a = K^-1 (y - H beta)      -> d2mu/dx2)
-//              out[1][i,k] = sum_col d2k*[i,k,col] b[col]    (b = K^-1 k*                -> term1 of d2sig2/dx2)
-//              out[2][i,k] = z_i . z_k                        (forward-solved derivative rows -> term2)
-// with r = x_train - x* and the radial profile f1, f2, f3 (kernels.h; Gaussian kernel: f2 = k, f1 = f3 = -k):
-//   value entry a        : 4 th_i th_k r_i r_k f2 + 2 th_i delta_ik f1
-//   gradient entry (j, a): (4 th_i th_j (delta_ik r_j + delta_jk r_i) + 4 delta_ij th_i th_k r_k) f2
-//                           + 8 th_i th_j th_k r_i r_j r_k f3
-// (kernel/KernelMatern5f2.py:54-96, 272-331 and kernel/KernelRatQuad.py:54-97, 556-633 for the other two families)
-__global__ void __launch_bounds__(256)
-predict_hess_kernel(Geom gm, const double* __restrict__ theta, const double* __restrict__ xs,
-                    const double* __restrict__ a, const double* __restrict__ b, const double* __restrict__ Z,
-                    int64_t ldz, double* __restrict__ out) {
-  __shared__ double sh[32];
-  const int d = gm.d, n = gm.n, ng = gm.ng, N = gm.N;
-  const int i = blockIdx.y, k = blockIdx.x;
-  const double thi = theta[i], thk = theta[k];
-  double s0 = 0.0, s1 = 0.0;
-  for (int p = threadIdx.x; p < n; p += blockDim.x) {
-    const double* xp = gm.X + (int64_t)p * d;
-    double e = 0.0;
-    for (int q = 0; q < d; q++) {
-      const double r = xp[q] - xs[q];
-      e += theta[q] * (r * r);
-    }
-    const RadialProfile ph = radial_profile(gm.ktype, gm.khp, e);
-    const double ri = xp[i] - xs[i], rk = xp[k] - xs[k];
-    const double hv = 4.0 * thi * thk * ri * rk * ph.f2 + ((i == k) ? 2.0 * thi * ph.f1 : 0.0);
-    s0 += hv * a[p];
-    s1 += hv * b[p];
-    const int sp = gm.slot ? gm.slot[p] : p;
-    if (sp >= 0) {
-      for (int j = 0; j < d; j++) {
-        const double thj = theta[j], rj = xp[j] - xs[j];
-        double v = 0.0;
-        if (i == k) v += 4.0 * thi * thj * rj;
-        if (j == k) v += 4.0 * thi * thj * ri;
-        if (i == j) v += 4.0 * thi * thk * rk;
-        v = v * ph.f2 + 8.0 * thi * thj * thk * ri * rj * rk * ph.f3;
-        const int col = n + j * ng + sp;
-        s0 += v * a[col];
-        s1 += v * b[col];
-      }
-    }
-  }
-  s0 = block_sum(s0, sh);
-  s1 = block_sum(s1, sh);
-  const double* zi = Z + (int64_t)(1 + i) * ldz;
-  const double* zk = Z + (int64_t)(1 + k) * ldz;
-  double s2 = 0.0;
-  for (int c = threadIdx.x; c < N; c += blockDim.x) s2 += zi[c] * zk[c];
-  s2 = block_sum(s2, sh);
-  if (threadIdx.x == 0) {
-    out[i * d + k] = s0;
-    out[d * d + i * d + k] = s1;
-    out[2 * d * d + i * d + k] = s2;
-  }
-}
-
-int launch_predict_hess(const Ctx& ctx, const Geom& gm, const double* theta, const double* xs, const double* a,
-                        const double* b, const double* Z, int64_t ldz, double* out) {
-  predict_hess_kernel<<<dim3(gm.d, gm.d, 1), 256, 0, ctx.stream>>>(gm, theta, xs, a, b, Z, ldz, out);
-  GEGP_CHECK_LAUNCH();
-  return 0;
-}
-
-// Surrogate Hessians for a batch of test points: one CTA per point (blockIdx.x), the same three outputs per point as
-// predict_hess_kernel.  Summing that kernel's gradient entries over j gives, per training point p with value coefficient
-// c_p, gradient coefficients G_p[j] (zero where slot[p] < 0), s_p = sum_j th_j r_j G_p[j] and r = x_p - x*:
+// Surrogate Hessians (eval/GpEvalModel.py:175-180, 356-382; the second x-derivatives of the cross covariance are
+// kernel/KernelSqExp.py:66-88 for value entries and :432-468 for gradient entries, kernel/KernelMatern5f2.py:54-96,
+// 272-331 and kernel/KernelRatQuad.py:54-97, 556-633 for the other two families).  Per test point, with r = x_p - x* and
+// the radial profile f1, f2, f3 (kernels.h), the second derivatives of k* are
+//   value entry p        : 4 th_i th_k r_i r_k f2 + 2 th_i delta_ik f1
+//   gradient entry (j, p): (4 th_i th_j (delta_ik r_j + delta_jk r_i) + 4 delta_ij th_i th_k r_k) f2
+//                           + 8 th_i th_j th_k r_i r_j r_k f3.
+// Summing the gradient entries over j gives, per training point p with value coefficient c_p, gradient coefficients
+// G_p[j] (zero where slot[p] < 0) and s_p = sum_j th_j r_j G_p[j]:
 //   H[i,k] = th_i th_k M[i,k] + delta_ik th_i W,   W = sum_p (2 f1 c_p + 4 f2 s_p),
 //   M[i,k] = sum_p (r_i q_k + r_k q_i),           q_j = 2 (f2 c_p + 2 f3 s_p) r_j + 4 f2 G_p[j],
 // so each radial profile is computed once per (test point, training point) pair: O(n d^2) per point instead of O(n d^3).
 // Applied with c, G from a = K^-1 (y - H beta) (-> d2mu/dx2) and from b = P^-1 L^-T z0 = K^-1 k* (-> term1).
 // term2[i,k] = z_i . z_k reads the point's d solved derivative rows once, in column tiles through shared memory.
-// Thread t owns the upper-triangle pairs e = t, t + 256, ... (d(d+1)/2 >= 256) or, for small d, pair t % P of the
-// point / column subset t / P; the subsets are summed in a fixed order.  Every entry is computed once for i <= k and
-// mirrored, so each Hessian is exactly symmetric.
+// CTA (x, y) is point x, page y of its d(d+1)/2 upper-triangle pairs (2048 pairs a page).  Thread t owns the pairs
+// y 2048 + t, + 256, ... (d(d+1)/2 >= 256) or, for small d, pair t % P of the point / column subset t / P; the subsets
+// are summed in a fixed order.  Every entry is computed once for i <= k and mirrored, so each Hessian is exactly
+// symmetric.  Every page recomputes the training-point tiles and W, which only its diagonal pairs use.
 constexpr int HB_T = 256;     // threads per CTA
-constexpr int HB_TP = 64;     // training points per tile
+constexpr int HB_TP = 64;     // training points per tile where it fits (every d <= 145)
 constexpr int HB_CT = 64;     // columns per term2 tile
-constexpr int HB_MAXI = 8;    // upper-triangle pairs per thread: d(d + 1) / 2 <= 8 * 256, d <= 63
-constexpr int HB_MAXD = 63;
+constexpr int HB_MAXI = 8;    // upper-triangle pairs per thread and page
+constexpr int HB_PAGE = HB_T * HB_MAXI;
 
-__host__ __device__ inline size_t hess_batch_smem_doubles(int d) {
-  const size_t tile = (size_t)HB_TP * (3 * d + 1), gram = (size_t)d * (HB_CT + 1);
-  return 2 * (size_t)d + 3 * HB_T + (tile > gram ? tile : gram);
+static size_t hess_batch_smem_bytes(int d, int tp) {   // dynamic shared memory of a CTA, tile height tp
+  const size_t tile = (size_t)tp * (3 * (size_t)d + 1), gram = (size_t)d * (HB_CT + 1);
+  return (2 * (size_t)d + 3 * HB_T + (tile > gram ? tile : gram)) * sizeof(double);
+}
+
+int hess_batch_tile_height(int d) {
+  for (int tp = HB_TP; tp >= 1; tp /= 2)   // 32 doubles of static shared memory: block_sum's scratch
+    if (hess_batch_smem_bytes(d, tp) + 32 * sizeof(double) <= (size_t)GEGP_MAX_DYN_SMEM) return tp;
+  return 0;
 }
 
 __global__ void __launch_bounds__(HB_T)
 predict_hess_batch_kernel(Geom gm, const double* __restrict__ theta, const double* __restrict__ Xs,
                           const double* __restrict__ a, const double* __restrict__ bt, int64_t ldb,
-                          const double* __restrict__ pinv, const double* __restrict__ Z, int64_t ldz,
+                          const double* __restrict__ pinv, const double* __restrict__ Z, int64_t ldz, int tp,
                           double* __restrict__ out) {
   extern __shared__ double sm[];
   __shared__ double sh[32];
@@ -580,12 +500,12 @@ predict_hess_batch_kernel(Geom gm, const double* __restrict__ theta, const doubl
   double* xs = sm;                 // [d]
   double* th = xs + d;             // [d]
   double* red = th + d;            // [3][HB_T] subset partial sums
-  double* tile = red + 3 * HB_T;   // [HB_TP][3d + 1] (r | q_a | q_b) or [d][HB_CT + 1] (derivative rows)
+  double* tile = red + 3 * HB_T;   // [tp][3d + 1] (r | q_a | q_b) or [d][HB_CT + 1] (derivative rows)
   const int P = d * (d + 1) / 2;
   const int G = P >= HB_T ? 1 : HB_T / P;    // subsets of the point / column range
   const int g = G > 1 ? t / P : 0;
   const bool active = G == 1 || t < G * P;
-  const int e0 = G > 1 ? t % P : t;
+  const int e0 = G > 1 ? t % P : blockIdx.y * HB_PAGE + t;
   const int nit = G > 1 ? 1 : HB_MAXI;
   for (int j = t; j < d; j += HB_T) { xs[j] = Xs[(int64_t)x * d + j]; th[j] = theta[j]; }
   int ii[HB_MAXI], kk[HB_MAXI];
@@ -627,9 +547,9 @@ predict_hess_batch_kernel(Geom gm, const double* __restrict__ theta, const doubl
   // ---- d2mu/dx2 and term1: the closed-form contraction over the training points
   const int TLD = 3 * d + 1;
   double wa = 0.0, wb = 0.0;
-  for (int p0 = 0; p0 < n; p0 += HB_TP) {
+  for (int p0 = 0; p0 < n; p0 += tp) {
     __syncthreads();
-    if (t < HB_TP) {
+    if (t < tp) {
       double* rr = tile + t * TLD;
       double* qa = rr + d;
       double* qb = qa + d;
@@ -674,7 +594,7 @@ predict_hess_batch_kernel(Geom gm, const double* __restrict__ theta, const doubl
         if (ii[m] < 0) continue;
         const int i = ii[m], k = kk[m];
         double s0 = acc0[m], s1 = acc1[m];
-        for (int q = g; q < HB_TP; q += G) {
+        for (int q = g; q < tp; q += G) {
           const double* rr = tile + q * TLD;
           const double ri = rr[i], rk = rr[k];
           s0 += ri * rr[d + k] + rk * rr[d + i];
@@ -734,18 +654,12 @@ predict_hess_batch_kernel(Geom gm, const double* __restrict__ theta, const doubl
 int launch_predict_hess_batch(const Ctx& ctx, const Geom& gm, const double* theta, const double* Xs, int nx, const double* a,
                               const double* bt, int64_t ldb, const double* pinv, const double* Z, int64_t ldz, double* out) {
   if (nx <= 0) return 0;
-  if (gm.d > HB_MAXD) return -908;
-  const size_t smem = hess_batch_smem_doubles(gm.d) * sizeof(double);
+  const int tp = hess_batch_tile_height(gm.d);
+  if (tp == 0) return -908;
+  const size_t smem = hess_batch_smem_bytes(gm.d, tp);
   if (smem > 48 * 1024) GEGP_SET_SMEM(predict_hess_batch_kernel, GEGP_MAX_DYN_SMEM);
-  predict_hess_batch_kernel<<<nx, HB_T, smem, ctx.stream>>>(gm, theta, Xs, a, bt, ldb, pinv, Z, ldz, out);
-  GEGP_CHECK_LAUNCH();
-  return 0;
-}
-
-int launch_predict_rows(const Ctx& ctx, int N, const double* Z, int64_t ldz, int nx, const double* w, double beta,
-                        double varK, double* mu, double* sig, double* sig2, int* n_negative) {
-  if (nx <= 0) return 0;
-  predict_rows_kernel<<<nx, 256, 0, ctx.stream>>>(N, Z, ldz, nx, w, beta, varK, mu, sig, sig2, n_negative);
+  const int pages = (gm.d * (gm.d + 1) / 2 + HB_PAGE - 1) / HB_PAGE;
+  predict_hess_batch_kernel<<<dim3(nx, pages), HB_T, smem, ctx.stream>>>(gm, theta, Xs, a, bt, ldb, pinv, Z, ldz, tp, out);
   GEGP_CHECK_LAUNCH();
   return 0;
 }

@@ -1270,13 +1270,8 @@ class GaussianProcess:
         self.KernEta_chofac = self._pred if good else None
         self.invKernEta_fdiff = DeviceMatrix(self._pred.alpha) if good else None
 
-    def eval_model(self, x2model_in, calc_grad=False, calc_hess=False, squeeze_nx=False):
-        """(mu, sig, dmudx, dsigdx, d2mudx2, d2sigdx2) -- eval/GpEvalModel.py:59-198.  calc_grad adds d mu / d x and
-        d sig / d x [nx, dim] (:170-173, 319-354); calc_hess adds the Hessians [1, dim, dim] for ONE point per call,
-        like the reference (:175-180, 356-382)."""
-        assert self.KernEta_chofac is not None, "To evaluate the surr the Cholesky decomposition is required"
-        if calc_hess:
-            assert calc_grad, "To return the hessian calc_grad must also be set to True"
+    def _test_points(self, x2model_in, squeeze_nx=False):
+        """x2model_in as a [nx, dim] array, with the checks eval_model and its variants share (eval/GpEvalModel.py)."""
         x = np.asarray(x2model_in, dtype=float)
         if x.ndim == 1:
             x = x[None, :]
@@ -1286,6 +1281,16 @@ class GaussianProcess:
             assert x.shape[0] == 1, "If squeeze_nx is True, then x_acq must only have one point"
         if not (self.hp_vals == self._hp_vals_model_setup):
             raise Exception("Cannot change hp_vals between calling setup_eval_model() and eval_model()")
+        return x
+
+    def eval_model(self, x2model_in, calc_grad=False, calc_hess=False, squeeze_nx=False):
+        """(mu, sig, dmudx, dsigdx, d2mudx2, d2sigdx2) -- eval/GpEvalModel.py:59-198.  calc_grad adds d mu / d x and
+        d sig / d x [nx, dim] (:170-173, 319-354); calc_hess adds the Hessians [1, dim, dim] for ONE point per call,
+        like the reference (:175-180, 356-382)."""
+        assert self.KernEta_chofac is not None, "To evaluate the surr the Cholesky decomposition is required"
+        if calc_hess:
+            assert calc_grad, "To return the hessian calc_grad must also be set to True"
+        x = self._test_points(x2model_in, squeeze_nx)
         if self.b_use_data_scl:
             x = self.DataScl.x_init_2_scl(x)
         dmudx = dsigdx = d2mudx2 = d2sigdx2 = None
@@ -1322,13 +1327,7 @@ class GaussianProcess:
         that takes Newton or trust-region steps on the surrogate from many starts at once.  Same guards as eval_model;
         d2sigdx2 is NaN at a point where sig = 0 (eval/GpEvalModel.py:374-375)."""
         assert self.KernEta_chofac is not None, "To evaluate the surr the Cholesky decomposition is required"
-        x = np.asarray(x2model_in, dtype=float)
-        if x.ndim == 1:
-            x = x[None, :]
-        elif x.ndim != 2:
-            raise Exception(f"x2model_in should be a 2d array but it has shape {x.shape}")
-        if not (self.hp_vals == self._hp_vals_model_setup):
-            raise Exception("Cannot change hp_vals between calling setup_eval_model() and eval_model()")
+        x = self._test_points(x2model_in)
         if self.b_use_data_scl:
             x = self.DataScl.x_init_2_scl(x)
         varK = float(self.hp_vals.varK)
@@ -1351,15 +1350,7 @@ class GaussianProcess:
         if calc_hess:
             assert calc_grad, "To return the hessian calc_grad must also be set to True"
             raise Exception("Must add method to calculate d2sig2dx2")          # the reference's own message (:303)
-        x = np.asarray(x2model_in, dtype=float)
-        if x.ndim == 1:
-            x = x[None, :]
-        elif x.ndim != 2:
-            raise Exception(f"x2model_in should be a 2d array but it has shape {x.shape}")
-        if squeeze_nx:
-            assert x.shape[0] == 1, "If squeeze_nx is True, then x_acq must only have one point"
-        if not (self.hp_vals == self._hp_vals_model_setup):
-            raise Exception("Cannot change hp_vals between calling setup_eval_model() and eval_model()")
+        x = self._test_points(x2model_in, squeeze_nx)
         varK = float(self.hp_vals.varK)
         dsig2dx = None
         if calc_grad:

@@ -184,7 +184,7 @@ int gegp_predict_grad(int n, int n_g, int d, const double* X, const int32_t* gra
  *   hess3[0] = d2mu/dx2,  hess3[1] = (d2 kstar / dx2) . (K^-1 kstar)  (term1),
  *   hess3[2] = (d kstar / dx) K^-1 (d kstar / dx)^T  (term2), kstar = K(X, xs);
  * the caller forms d2sig2/dx2 = -2 varK (term1 + term2) and d2sig/dx2 = (d2sig2/dx2 - 2 dsig dsig^T) / (2 sig).
- * work >= (d + 2) * gegp_ld(N) * 8 bytes. */
+ * Each d x d slab is exactly symmetric.  work >= (d + 2) * gegp_ld(N) * 8 bytes. */
 int gegp_predict_hess(int n, int n_g, int d, const double* X, const int32_t* grad_slot, const double* theta, int kernel, double kernel_hp,
                       const double* A, int64_t lda, const double* dinv, const double* p, const double* alpha, int mode,
                       double beta, double varK, const double* xs, double* mu, double* sig, double* sig2_out,
@@ -197,9 +197,10 @@ int gegp_predict_hess(int n, int n_g, int d, const double* X, const int32_t* gra
  * one-point call (d2mu/dx2, term1, term2); n_negative_dev counts the negative sig2 entries.  Per chunk of points: one
  * cross-covariance launch, one forward solve of the (d + 1) rows of every point, one back substitution of all the points'
  * K^-1 k* at once and one contraction launch.  mu, sig, sig2, dmudx and dsigdx are those of gegp_predict_grad for the same
- * chunk; hess3 agrees with the one-point call to rounding (its sums run in another order) and every d x d slab is exactly
- * symmetric.  d <= 63 (else -3).  work >= gegp_dinv_doubles(N) * 8 bytes, plus ((d + 1) * gegp_ld(N) + 128) * 8 bytes per
- * point of a chunk; the chunk is as many points as fit (at least one, else -25).  nx = 0 writes nothing. */
+ * chunk; hess3 agrees with the one-point call to rounding (the one-point call solves for K^-1 k* with its own back
+ * substitution; the contraction is the same) and every d x d slab is exactly symmetric.  d <= 421, where the
+ * contraction's shared-memory tiles fit (else -3); gegp_predict_setup itself accepts d up to about 353.
+ * work >= gegp_dinv_doubles(N) * 8 bytes, plus ((d + 1) * gegp_ld(N) + 128) * 8 bytes per point of a chunk; the chunk is as many points as fit (at least one, else -25).  nx = 0 writes nothing. */
 int gegp_predict_hess_batch(int n, int n_g, int d, const double* X, const int32_t* grad_slot, const double* theta, int kernel,
                             double kernel_hp, const double* A, int64_t lda, const double* dinv, const double* p,
                             const double* alpha, int mode, double beta, double varK, const double* Xs, int nx, double* mu,

@@ -193,6 +193,27 @@ def test_agrees_with_the_one_point_path(size):
     assert int(out[6][0]) == int(grad[5][0])
 
 
+WIDE = [  # kernel, masked, noisy, mode, n, d: 2, 3 and 7 pages of upper-triangle pairs; tiles of 32 training points at d = 160
+    ("SqExp", True, True, "precon", 6, 64), ("RatQu", False, True, "base", 5, 100), ("Ma5f2", True, False, "precon", 4, 160)]
+
+
+@pytest.mark.parametrize("case", WIDE, ids=lambda c: f"{c[0]}-d{c[5]}")
+def test_wide_vs_oracle_and_one_point(case):
+    """d > 63: the batched and the one-point call against the oracle, and against each other to 1e-12.  Each test point
+    lies at s = 0.5 from one training point: in this many dimensions the rest of the data is out of reach."""
+    from gpgradpy_b200 import backend as bk
+    kname, masked, noisy, mode, n, d = case
+    p = _problem(n, d, kname, masked=masked, noisy=noisy, mode=mode, seed=27)
+    z = np.random.default_rng(28).normal(size=(n, d))
+    xs = p["x"] + z * np.sqrt(0.5 / np.sum(_theta(n, d) * z * z, axis=1))[:, None]
+    out = _batch(p, xs)
+    ones = [_np(*bk.predict_hess(p["st"], xs[i], VARK)) for i in range(n)]
+    one = [np.stack([o[k].reshape(np.shape(out[k][0])) for o in ones]) for k in range(6)]
+    _close(out, one)
+    _check_oracle(p, xs, _derived(out))
+    _check_oracle(p, xs, _derived(one + [None]))
+
+
 def test_gaussian_process_batch_is_the_stacked_one_point_calls():
     """GaussianProcess.eval_model_hess_batch(X)[k][i] == eval_model(X[i:i+1], calc_grad=True, calc_hess=True)[k][0] to
     1e-12, in a rescale mode (rescale_origin: inputs, outputs and derivatives go through data_scl_2_init)."""

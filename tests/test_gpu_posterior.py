@@ -355,3 +355,4 @@ def test_predict_hess_vs_oracle(case):
     assert e["mu"] < 1e-8 and e["dmu"] < 1e-8 and e["d2mu"] < 1e-8
     assert e["dsig"] < 1e-6 and e["d2sig"] < 1e-5
     assert np.array_equal(sig, np.sqrt(np.maximum(sig2, 0.0)) * np.sqrt(VARK)) and int(nneg[0]) == int(sig2[0] < 0)
+    assert np.array_equal(h3, h3.transpose(0, 2, 1))         # each slab exactly symmetric

@@ -59,7 +59,7 @@ def test_oracle_batch_of_no_points():
     assert [o.shape for o in out] == [(0,), (0,), (0, 2), (0, 2), (0, 2, 2), (0, 2, 2)]
 
 
-def test_argument_codes_without_touching_the_gpu():
+def test_argument_codes_and_dimension_bound_without_touching_the_gpu():
     from gpgradpy_b200 import _lib
     lib = _lib.load()
     f = lib.gegp_predict_hess_batch
@@ -73,7 +73,9 @@ def test_argument_codes_without_touching_the_gpu():
         return f(*a.values())
 
     assert call(n=0) == -1 and call(n_g=5) == -1 and call(d=0) == -1
-    assert call(d=64, lda=320) == -3                      # the contraction kernel holds d <= 63
+    # the contraction's shared-memory tiles fit up to d = 421; nx = 0 returns after the checks
+    assert call(d=422, lda=1696) == -3
+    assert call(d=64, lda=320, nx=0) == 0 and call(d=421, lda=1696, nx=0) == 0
     assert call(kernel=7) == -50 and call(kernel=_lib.KERNEL_RATQUAD, khp=0.0) == -50
     assert call(X=0) == -4
     assert call(n_g=2, slot=0) == -5
