@@ -28,6 +28,8 @@ EXPORTS = (
     "gegp_abi_version", "gegp_set_option", "gegp_workspace_bytes", "gegp_ld", "gegp_build_cov", "gegp_cross_cov", "gegp_potrf",
     "gegp_trsm_rows", "gegp_dinv_doubles", "gegp_potri", "gegp_dgemm", "gegp_lml_eval", "gegp_predict_setup", "gegp_predict", "gegp_profile_begin", "gegp_profile_end",
     "gegp_predict_grad", "gegp_predict_hess", "gegp_predict_hess_batch", "gegp_lml_layout", "gegp_symv", "gegp_row_abs_sum", "gegp_row_sq_sum", "gegp_weighted_grad", "gegp_lanczos_step", "gegp_lincomb", "gegp_quad_grad_work_bytes", "gegp_quad_grad", "gegp_dmma_peak", "gegp_lml_direct_terms",
+    "gegp_symv_batch", "gegp_lanczos_step_batch", "gegp_lincomb_batch", "gegp_quad_grad_batch_work_bytes",
+    "gegp_quad_grad_batch", "gegp_build_cov_batch",
 )
 
 
@@ -105,6 +107,18 @@ def load():
     lib.gegp_quad_grad_work_bytes.argtypes = [i, i, i]
     lib.gegp_quad_grad.restype = i
     lib.gegp_quad_grad.argtypes = [i, i, i, dp, ip, dp, i, dbl, dp, i, dbl, i, dp, dp, vp, sz, vp]
+    lib.gegp_symv_batch.restype = i
+    lib.gegp_symv_batch.argtypes = [i, i, dp, i64, i64, dp, i64, dp, i64, ip, vp]
+    lib.gegp_lanczos_step_batch.restype = i
+    lib.gegp_lanczos_step_batch.argtypes = [i, i, i, dp, i64, i64, dp, i64, dp, dp, i64, ip, vp]
+    lib.gegp_lincomb_batch.restype = i
+    lib.gegp_lincomb_batch.argtypes = [i, i, i, ip, dp, i64, i64, dp, i64, dp, i64, ip, vp]
+    lib.gegp_quad_grad_batch_work_bytes.restype = sz
+    lib.gegp_quad_grad_batch_work_bytes.argtypes = [i, i, i, i]
+    lib.gegp_quad_grad_batch.restype = i
+    lib.gegp_quad_grad_batch.argtypes = [i, dp, dp, i, dp, i, i, i, dp, ip, dp, i64, i, dbl, i, dp, vp, sz, vp]
+    lib.gegp_build_cov_batch.restype = i
+    lib.gegp_build_cov_batch.argtypes = [i, dp, dp, i, dp, i, i, i, dp, ip, dp, i, dbl, dp, i64, i64, dp, i64, i, vp]
     lib.gegp_lml_direct_terms.restype = i
     lib.gegp_lml_direct_terms.argtypes = [i, i, i, dp, ip, dp, i, dbl, i, dbl, i, dp, vp, sz, dp, dp, vp]
     lib.gegp_dmma_peak.restype = i

@@ -513,71 +513,128 @@ def extreme_eig(M: torch.Tensor, N: int, *, k: int = 40, tol: float = 1e-12, max
     stops as soon as the residual estimate |beta_j s_j| <= tol |lambda| (or an invariant subspace is hit); after k steps
     it restarts from the Ritz vector.  `v0` (device vector) warm-starts the iteration -- e.g. the eigenvector of the
     previous optimiser iterate; it is mixed with the fixed pseudo-random start vector so that no eigen-direction is
-    ever excluded.  Returns (lambda, v [N] device tensor with |v| = 1, relative residual estimate, matvecs)."""
+    ever excluded.  Returns (lambda, v [N] device tensor with |v| = 1, relative residual estimate, matvecs).
+    This is the one-candidate case of extreme_eig_batch."""
+    lam, v, resid, matvecs = extreme_eig_batch(M[None], N, k=k, tol=tol, max_cycles=max_cycles, v0=[v0], chunk=chunk)
+    return lam[0], v[0], resid[0], matvecs[0]
+
+
+def _tridiag_ritz(a, b, j):
+    """Largest Ritz pair of the j-step Lanczos tridiagonal (a, b) -> (basis size m, lambda, s, relative residual)."""
     from scipy.linalg import eigh_tridiagonal
+    scale = max(float(np.max(np.abs(a[:j]))), 1e-300)
+    m = j
+    for q in range(j):            # breakdown: an invariant subspace was found after q + 1 steps
+        if not (b[q] > 1e-14 * scale):
+            m = q + 1
+            break
+    evals, evecs = eigh_tridiagonal(a[:m], b[:m - 1]) if m > 1 else (a[:1], np.ones((1, 1)))
+    lam, s_vec = float(evals[-1]), evecs[:, -1]
+    return m, lam, s_vec, abs(float(b[m - 1]) * float(s_vec[-1])) / max(abs(lam), 1e-300)
+
+
+def extreme_eig_batch(M: torch.Tensor, N: int, *, k: int = 40, tol: float = 1e-12, max_cycles: int = 12, v0=None,
+                      chunk: int = 8, rows=None):
+    """extreme_eig for B symmetric matrices at once.  M: [B, >= N, ld] device view with unit column stride (e.g. the
+    candidates' buffers in a gegp_lml_eval workspace); v0: None or a list of B warm-start vectors (entries may be None).
+
+    Every candidate still iterating is at the same Lanczos step within a cycle, so each step is one gegp_symv_batch and
+    one gegp_lanczos_step_batch over those candidates; after each `chunk` steps the alphas and betas of all candidates
+    come to the host in one copy, and each candidate takes its own converge / restart / breakdown decision exactly as
+    extreme_eig does alone.  Converged candidates leave the launches through the active list.  A candidate's result is
+    bit-identical to extreme_eig on its matrix alone.  rows: the candidates to iterate (default all); the others are
+    skipped and get None.  -> (lambdas, vectors [N] device tensors, residuals, matvecs), lists of B."""
     lib = L.load()
+    B = M.shape[0]
+    assert M.stride(-1) == 1 and B >= 1
     k = int(max(2, min(k, N, 200)))
     ld = ld_of(N)
     dev = device()
-    V = torch.zeros((k + 1, ld), dtype=F64, device=dev)
-    w = torch.zeros(ld, dtype=F64, device=dev)
-    r = torch.zeros(ld, dtype=F64, device=dev)
-    ab = torch.zeros((2, k), dtype=F64, device=dev)
-    coef = torch.zeros(k, dtype=F64, device=dev)
-    one = torch.ones(1, dtype=F64, device=dev)
+    st = _stream()
+    ldm, sM = M.stride(-2), (M.stride(0) if B > 1 else 0)
+    V = torch.zeros((B, k + 1, ld), dtype=F64, device=dev)
+    w = torch.zeros((B, ld), dtype=F64, device=dev)
+    r = torch.zeros((B, ld), dtype=F64, device=dev)
+    ab = torch.zeros((B, 2, k), dtype=F64, device=dev)     # alpha_z, beta_z: one device-to-host copy per chunk
+    coef = torch.zeros((B, k), dtype=F64, device=dev)
+    ks = torch.ones(B, dtype=torch.int32, device=dev)
     rnd = to_dev(np.random.default_rng(12345).standard_normal(N))   # fixed: deterministic results
-    if v0 is None:
-        V[0, :N] = rnd
-    else:
-        V[0, :N] = v0[:N] + (1e-3 / np.sqrt(N)) * rnd
-    rc = lib.gegp_lincomb(N, 1, _p(V), ld, _p(one), _p(r), _stream())      # normalise
-    _check(rc, "gegp_lincomb")
-    V[0].copy_(r)
-    lam, resid, matvecs = float("nan"), float("inf"), 0
+    V[:, 0, :N] = rnd
+    for c, v in enumerate(v0 if v0 is not None else []):
+        if v is not None:
+            V[c, 0, :N] = v[:N] + (1e-3 / np.sqrt(N)) * rnd
+    sV = (k + 1) * ld
+
+    def lincomb(rows, kmax):
+        act = None if len(rows) == B else torch.as_tensor(np.asarray(rows, dtype=np.int32)).to(dev)
+        rc = lib.gegp_lincomb_batch(len(rows), N, kmax, _p(ks), _p(V), ld, sV, _p(coef), k, _p(r), ld, _p(act), st)
+        _check(rc, "gegp_lincomb_batch")
+        idx = torch.as_tensor(rows, dtype=torch.long, device=dev)
+        V[idx, 0] = r[idx]
+
+    alive = list(range(B)) if rows is None else sorted(set(int(c) for c in rows))
+    todo = set(alive)
+    lam, resid, matvecs = [float("nan")] * B, [float("inf")] * B, [0] * B
+    if not alive:
+        return [None] * B, [None] * B, [None] * B, [None] * B
+    coef[:, 0] = 1.0
+    lincomb(alive, 1)                                                       # normalise the start vectors
     for _cycle in range(max_cycles):
-        j, done, m = 0, False, k
-        while j < k and not done:
+        if not alive:
+            break
+        j, active = 0, list(alive)
+        while j < k and active:
+            act = None if len(active) == B else torch.as_tensor(np.asarray(active, dtype=np.int32)).to(dev)
             jn = min(k, j + chunk)
             for jj in range(j, jn):
-                rc = lib.gegp_symv(N, _p(M), M.stride(0), _p(V[jj]), _p(w), _stream())
-                _check(rc, "gegp_symv")
-                rc = lib.gegp_lanczos_step(N, jj, _p(V), ld, _p(w), _p(ab[0]), _p(ab[1]), _stream())
-                _check(rc, "gegp_lanczos_step")
-            matvecs += jn - j
-            j = jn
+                rc = lib.gegp_symv_batch(len(active), N, _p(M), ldm, sM, _p(V[0, jj]), sV, _p(w), ld, _p(act), st)
+                _check(rc, "gegp_symv_batch")
+                rc = lib.gegp_lanczos_step_batch(len(active), N, jj, _p(V), ld, sV, _p(w), ld, _p(ab[0, 0]), _p(ab[0, 1]),
+                                                 2 * k, _p(act), st)
+                _check(rc, "gegp_lanczos_step_batch")
             h = ab.cpu().numpy()
-            a, b = h[0], h[1]
-            scale = max(float(np.max(np.abs(a[:j]))), 1e-300)
-            m = j
-            for q in range(j):            # breakdown: an invariant subspace was found after q + 1 steps
-                if not (b[q] > 1e-14 * scale):
-                    m = q + 1
-                    break
-            evals, evecs = eigh_tridiagonal(a[:m], b[:m - 1]) if m > 1 else (a[:1], np.ones((1, 1)))
-            lam, s_vec = float(evals[-1]), evecs[:, -1]
-            resid = abs(float(b[m - 1]) * float(s_vec[-1])) / max(abs(lam), 1e-300)
-            done = resid <= tol or m < j
-        coef[:m] = to_dev(np.ascontiguousarray(s_vec))
-        rc = lib.gegp_lincomb(N, m, _p(V), ld, _p(coef), _p(r), _stream())
-        _check(rc, "gegp_lincomb")
-        V[0].copy_(r)
-        if done:
-            break
-    return lam, r[:N].clone(), resid, matvecs
+            finished, coef_h, ks_h, kmax = [], np.zeros((B, k)), np.ones(B, dtype=np.int32), 1
+            for c in active:
+                matvecs[c] += jn - j
+                m, lam[c], s_vec, resid[c] = _tridiag_ritz(h[c, 0], h[c, 1], jn)
+                done = resid[c] <= tol or m < jn
+                if done or jn == k:            # restart (or finish) from the Ritz vector
+                    finished.append(c)
+                    coef_h[c, :m], ks_h[c], kmax = s_vec, m, max(kmax, m)
+                    if done:
+                        alive.remove(c)
+            j = jn
+            if finished:
+                coef.copy_(torch.from_numpy(coef_h))
+                ks.copy_(torch.from_numpy(ks_h))
+                lincomb(finished, kmax)
+                active = [c for c in active if c not in finished]
+    return ([lam[c] if c in todo else None for c in range(B)], [r[c, :N].clone() if c in todo else None for c in range(B)],
+            [resid[c] if c in todo else None for c in range(B)], [matvecs[c] if c in todo else None for c in range(B)])
 
 
 def cond2(Kfull: torch.Tensor, Kinv: torch.Tensor, N: int, *, tol: float = 1e-12, warm=None):
     """kappa_2 = lambda_max(K) * lambda_max(K^-1) with both extreme eigenvectors.  `warm`: a previous result of this
     function for a nearby matrix of the same order (its eigenvectors warm-start the two iterations).
     -> dict(cond, lam_max, lam_min, v_max, v_min, resid_max, resid_min, cycles = matvecs of the two iterations)."""
-    w1 = w2 = None
-    if warm is not None and warm.get("v_max") is not None and warm["v_max"].numel() == N:
-        w1, w2 = warm["v_max"], warm["v_min"]
-    lmax, vmax, r1, c1 = extreme_eig(Kfull, N, tol=tol, v0=w1)
-    imax, vmin, r2, c2 = extreme_eig(Kinv, N, tol=tol, v0=w2)
-    lmin = 1.0 / imax
-    return dict(cond=lmax * imax, lam_max=lmax, lam_min=lmin, v_max=vmax, v_min=vmin, resid_max=r1, resid_min=r2,
-                cycles=(c1, c2))
+    return cond2_batch(Kfull[None], Kinv[None], N, tol=tol, warm=[warm])[0]
+
+
+def cond2_batch(Kfull: torch.Tensor, Kinv: torch.Tensor, N: int, *, tol: float = 1e-12, warm=None, rows=None):
+    """cond2 for B candidates: Kfull, Kinv [B, >= N, ld] device views (e.g. the U and Kinv buffers of a gegp_lml_eval
+    workspace, lml_views_batch); warm: None or a list of B earlier results (entries may be None); rows: the candidates
+    to evaluate (default all; the others get None).  -> list of B dicts, each bit-identical to cond2 on that candidate
+    alone."""
+    B = Kfull.shape[0]
+    warm = warm if warm is not None else [None] * B
+    ok = [wm is not None and wm.get("v_max") is not None and wm["v_max"].numel() == N for wm in warm]
+    lmax, vmax, r1, c1 = extreme_eig_batch(Kfull, N, tol=tol, v0=[wm["v_max"] if o else None for wm, o in zip(warm, ok)],
+                                           rows=rows)
+    imax, vmin, r2, c2 = extreme_eig_batch(Kinv, N, tol=tol, v0=[wm["v_min"] if o else None for wm, o in zip(warm, ok)],
+                                           rows=rows)
+    return [None if lmax[c] is None else
+            dict(cond=lmax[c] * imax[c], lam_max=lmax[c], lam_min=1.0 / imax[c], v_max=vmax[c], v_min=vmin[c],
+                 resid_max=r1[c], resid_min=r2[c], cycles=(c1[c], c2[c])) for c in range(B)]
 
 
 def quad_grad(X, theta, v, *, n_g=None, slot=None, eta=0.0, noisy=False, varK=1.0, kernel=None):
@@ -623,17 +680,98 @@ def lml_direct_terms(X, theta, *, n_g=None, slot=None, mode=L.MODE_PRECON, eta=0
 def lml_views(n: int, n_g: int, d: int):
     """Views of candidate 0's arrays inside the shared workspace, valid right after a B = 1 lml_eval(want_grad=True)
     (eager or graph replay) on this device: dict(A [N+2, ld] factor, U [N, ld], Kinv [N, ld], ld)."""
+    v = lml_views_batch(n, n_g, d, 1)
+    return dict(A=v["A"][0], U=v["U"][0], Kinv=v["Kinv"][0], p=v["p"][0], pinv=v["pinv"][0], ld=v["ld"])
+
+
+def lml_views_batch(n: int, n_g: int, d: int, B: int):
+    """Strided views of the arrays of candidates 0 .. B-1 inside the shared workspace, valid right after an
+    lml_eval(want_grad=True) of B rows that fitted the workspace in one chunk (lml_chunk_rows): dict(A [B, N+2, ld],
+    U [B, N, ld], Kinv [B, N, ld], p [B, N], pinv [B, N], ld, stride = doubles between candidates)."""
     lib = L.load()
     o = (C.c_int64 * 8)()
-    rc = lib.gegp_lml_layout(n, n_g, d, 1, 1, o)
+    rc = lib.gegp_lml_layout(n, n_g, d, 1, B, o)
     _check(rc, "gegp_lml_layout")
     header, ld, per, offA, offP, _offD, offU, offK = (int(x) for x in o)
     ws = _ws_cache.get(torch.cuda.current_device())
-    assert ws is not None and ws.numel() >= header + 8 * per, "no likelihood evaluation has run on this device yet"
-    dbl = ws[header:header + 8 * per].view(F64)
+    assert ws is not None and ws.numel() >= header + 8 * per * B, "no likelihood evaluation of this size has run on this device"
+    dbl = ws[header:header + 8 * per * B].view(F64)
     N = n + n_g * d
-    return dict(A=dbl[offA:offA + (N + 2) * ld].view(N + 2, ld), U=dbl[offU:offU + N * ld].view(N, ld),
-                Kinv=dbl[offK:offK + N * ld].view(N, ld), p=dbl[offP:offP + N], pinv=dbl[offP + ld:offP + ld + N], ld=ld)
+
+    def view(off, rows, cols=None):   # as_strided takes the offset from the start of the storage, not of `dbl`
+        if cols is None:
+            return dbl.as_strided((B, rows), (per, 1), dbl.storage_offset() + off)
+        return dbl.as_strided((B, rows, cols), (per, ld, 1), dbl.storage_offset() + off)
+    return dict(A=view(offA, N + 2, ld), U=view(offU, N, ld), Kinv=view(offK, N, ld), p=view(offP, N),
+                pinv=view(offP + ld, N), ld=ld, stride=per)
+
+
+def lml_chunk_rows(n: int, n_g: int, d: int, B: int, *, want_grad=True, max_ws_bytes=None) -> int:
+    """How many of B candidate rows to hand to one lml_eval call whose workspace arrays are read afterwards (gegp_lml_eval
+    chunks the rows itself and overwrites earlier chunks' arrays with later ones).  At most max_ws_bytes of workspace
+    (default: what lml_eval would use); the workspace is grown so that an lml_eval of that many rows runs in one chunk."""
+    lib = L.load()
+    op = L.OP_LML_GRAD if want_grad else L.OP_LML
+    ws = _lml_workspace(lib, op, n, n_g, d, B, max_ws_bytes)
+    o = (C.c_int64 * 8)()
+    _check(lib.gegp_lml_layout(n, n_g, d, int(bool(want_grad)), B, o), "gegp_lml_layout")
+    header, per = int(o[0]), 8 * int(o[2])
+    avail = ws.numel() if max_ws_bytes is None else min(ws.numel(), int(max_ws_bytes))
+    c = int(max(1, min(B, (avail - header - 4 * B - 256) // per)))
+    workspace(int(lib.gegp_workspace_bytes(op, n, n_g, d, c)) + 4 * c + 256)   # lml_eval of c rows: one chunk
+    return c
+
+
+def build_cov_batch(X, theta_rows, *, n_g=None, slot=None, noise=None, varK_rows=None, mode=L.MODE_BASE, eta=0.0,
+                    out=None, kernel=None, kernel_hp_rows=None):
+    """gegp_build_cov_batch: one covariance matrix per theta row into out [B, >= N, ld] (strided device view, e.g. the
+    U buffers of lml_views_batch).  noise: one device vector for every row, divided by varK_rows[z] on the device."""
+    lib = L.load()
+    X, th = to_dev(X), to_dev(theta_rows)
+    n, d = X.shape
+    th = th.reshape(-1, d).contiguous()
+    B = th.shape[0]
+    n_g = n if n_g is None else n_g
+    N = n + n_g * d
+    vk = to_dev(varK_rows).reshape(-1).contiguous() if varK_rows is not None else None
+    kid, khp = _kern(kernel)
+    khp_dev = None
+    if kid == L.KERNEL_RATQUAD:
+        khp_dev = to_dev(kernel_hp_rows).reshape(-1) if kernel_hp_rows is not None else torch.full((B,), khp, dtype=F64,
+                                                                                                   device=device())
+    ld = ld_of(N)
+    p = torch.empty((B, 2 * ld), dtype=F64, device=device()) if mode == L.MODE_PRECON else None
+    rc = lib.gegp_build_cov_batch(B, _p(th), _p(vk), kid, _p(khp_dev), n, n_g, d, _p(X), _p(slot), _p(noise), int(mode),
+                                  float(eta), _p(out), out.stride(1), out.stride(0) if B > 1 else 0, _p(p), 2 * ld, 0,
+                                  _stream())
+    _check(rc, "gegp_build_cov_batch")
+    return out
+
+
+def quad_grad_batch(X, theta_rows, V: torch.Tensor, *, n_g=None, slot=None, eta=0.0, noisy=False, varK_rows=None,
+                    kernel=None, kernel_hp_rows=None):
+    """gegp_quad_grad_batch: v_z^T (dKcov/dhp) v_z for the rows of V [B, >= N] (unit column stride), each with its own
+    theta row (base mode) -> device table [B, 9+d] laid out as GEGP_OUT_*; row z is bit-identical to quad_grad."""
+    lib = L.load()
+    X, th = to_dev(X), to_dev(theta_rows)
+    n, d = X.shape
+    th = th.reshape(-1, d).contiguous()
+    B = th.shape[0]
+    n_g = n if n_g is None else n_g
+    assert V.shape[0] == B and V.stride(-1) == 1
+    out = torch.zeros((B, L.out_len(d)), dtype=F64, device=device())
+    vk = to_dev(varK_rows).reshape(-1).contiguous() if noisy else None
+    kid, khp = _kern(kernel)
+    khp_dev = None
+    if kid == L.KERNEL_RATQUAD:
+        khp_dev = to_dev(kernel_hp_rows).reshape(-1) if kernel_hp_rows is not None else torch.full((B,), khp, dtype=F64,
+                                                                                                   device=device())
+    nbytes = int(lib.gegp_quad_grad_batch_work_bytes(B, n, n_g, d))
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=device())
+    rc = lib.gegp_quad_grad_batch(B, _p(th), _p(vk), kid, _p(khp_dev), n, n_g, d, _p(X), _p(slot), _p(V), V.stride(0),
+                                  L.MODE_BASE, float(eta), int(bool(noisy)), _p(out), _p(ws), nbytes, _stream())
+    _check(rc, "gegp_quad_grad_batch")
+    return out
 
 
 def cond_fro_of_matrix(K: torch.Tensor, N: int) -> float:

@@ -269,6 +269,36 @@ int gegp_build_cov(int n, int n_g, int d, const double* X, const int32_t* grad_s
   return launch_build_cov(ctx, gm, theta, 0, ns, p_out ? p_out + N : nullptr, 0, mode, eta, K_out, ldk, 0, uplo ? 1 : 0);
 }
 
+int gegp_build_cov_batch(int B, const double* theta_batch, const double* varK_batch, int kernel,
+                         const double* kernel_hp_batch, int n, int n_g, int d, const double* X, const int32_t* grad_slot,
+                         const double* noise, int mode, double eta, double* K_out, int64_t ldk, int64_t strideK,
+                         double* p_out, int64_t strideP, int uplo, void* stream) {
+  if (B <= 0 || B > 65535) return -1;
+  if (!theta_batch) return -2;
+  if (kernel < GEGP_KERNEL_SQEXP || kernel > GEGP_KERNEL_RATQUAD) return -50;
+  if (kernel == GEGP_KERNEL_RATQUAD && !kernel_hp_batch) return -50;
+  if (bad_geom(n, n_g, d)) return -6;
+  if (!X) return -9;
+  if (n_g != n && !grad_slot) return -10;
+  if (mode < GEGP_MODE_BASE || mode > GEGP_MODE_PRECON_COV) return -12;
+  if (!K_out) return -14;
+  const int N = n + n_g * d;
+  if (ldk < N) return -15;
+  if (strideK < 0) return -16;
+  if (mode == GEGP_MODE_PRECON && !p_out) return -17;
+  if (p_out && strideP < 2 * (int64_t)N) return -18;
+  Ctx ctx{(cudaStream_t)stream, B};
+  const Geom gm = make_geom(n, n_g, d, X, grad_slot, kernel, 0.0, kernel_hp_batch);
+  NoiseSpec ns{noise, 0, varK_batch, 1.0, (noise && varK_batch) ? 1 : 0};
+  int rc = 0;
+  if (p_out) {
+    rc = launch_prep_p(ctx, gm, theta_batch, d, ns, mode, p_out, p_out + N, strideP);
+    if (rc) return rc;
+  }
+  return launch_build_cov(ctx, gm, theta_batch, d, ns, p_out ? p_out + N : nullptr, strideP, mode, eta, K_out, ldk, strideK,
+                          uplo ? 1 : 0);
+}
+
 int gegp_cross_cov(int n, int n_g, int d, const double* X, const int32_t* grad_slot, const double* Xs, int nx,
                    const double* theta, int kernel, double kernel_hp, const double* pinv, double* Kx, int64_t ld, void* stream) {
   if (bad_geom(n, n_g, d)) return -1;
@@ -446,7 +476,22 @@ int gegp_symv(int N, const double* M, int64_t ld, const double* x, double* y, vo
   if (!x || (reinterpret_cast<uintptr_t>(x) & 15)) return -4;
   if (!y) return -5;
   Ctx ctx{(cudaStream_t)stream, 1};
-  return symv_full(ctx, N, M, ld, x, y);
+  return symv_full(ctx, N, M, ld, 0, x, 0, y, 0, nullptr);
+}
+
+int gegp_symv_batch(int B, int N, const double* M, int64_t ld, int64_t strideM, const double* x, int64_t strideX,
+                    double* y, int64_t strideY, const int32_t* active, void* stream) {
+  if (B <= 0 || B > 65535) return -1;
+  if (N <= 0) return -2;
+  if (!M || (reinterpret_cast<uintptr_t>(M) & 15)) return -3;
+  if (ld < N || (ld & 1)) return -4;
+  if (strideM < 0 || (strideM & 1)) return -5;
+  if (!x || (reinterpret_cast<uintptr_t>(x) & 15)) return -6;
+  if (strideX < 0 || (strideX & 1)) return -7;
+  if (!y) return -8;
+  if (strideY < 0) return -9;
+  Ctx ctx{(cudaStream_t)stream, B};
+  return symv_full(ctx, N, M, ld, strideM, x, strideX, y, strideY, active);
 }
 
 int gegp_row_abs_sum(int N, const double* M, int64_t ld, double* out, void* stream) {
@@ -476,7 +521,24 @@ int gegp_lanczos_step(int N, int j, double* V, int64_t ldv, double* w, double* a
   if (!alpha) return -6;
   if (!beta) return -7;
   Ctx ctx{(cudaStream_t)stream, 1};
-  return lanczos_step(ctx, N, j, V, ldv, w, alpha, beta);
+  return lanczos_step(ctx, N, j, V, ldv, 0, w, 0, alpha, beta, 0, nullptr);
+}
+
+int gegp_lanczos_step_batch(int B, int N, int j, double* V, int64_t ldv, int64_t strideV, double* w, int64_t strideW,
+                            double* alpha, double* beta, int64_t strideAB, const int32_t* active, void* stream) {
+  if (B <= 0) return -1;
+  if (N <= 0) return -2;
+  if (j < 0 || j >= 255) return -3;
+  if (!V) return -4;
+  if (ldv < N) return -5;
+  if (strideV < 0) return -6;
+  if (!w) return -7;
+  if (strideW < 0) return -8;
+  if (!alpha) return -9;
+  if (!beta) return -10;
+  if (strideAB < 0) return -11;
+  Ctx ctx{(cudaStream_t)stream, B};
+  return lanczos_step(ctx, N, j, V, ldv, strideV, w, strideW, alpha, beta, strideAB, active);
 }
 
 int gegp_lincomb(int N, int k, const double* V, int64_t ldv, const double* coef, double* out, void* stream) {
@@ -487,14 +549,54 @@ int gegp_lincomb(int N, int k, const double* V, int64_t ldv, const double* coef,
   if (!coef) return -5;
   if (!out) return -6;
   Ctx ctx{(cudaStream_t)stream, 1};
-  return lincomb_rows(ctx, N, k, V, ldv, coef, out);
+  return lincomb_rows(ctx, N, k, nullptr, V, ldv, 0, coef, 0, out, 0, nullptr);
 }
 
-size_t gegp_quad_grad_work_bytes(int n, int n_g, int d) {
-  if (bad_geom(n, n_g, d)) return 0;
-  const int N = n + n_g * d;
-  return ((size_t)round_up(N, 2) + (size_t)round_up((int64_t)lml_grad_partial_doubles(n, d), 2)) * sizeof(double);
+int gegp_lincomb_batch(int B, int N, int k, const int32_t* ks, const double* V, int64_t ldv, int64_t strideV,
+                       const double* coef, int64_t strideCoef, double* out, int64_t strideOut, const int32_t* active,
+                       void* stream) {
+  if (B <= 0) return -1;
+  if (N <= 0) return -2;
+  if (k < 1 || k > 256) return -3;
+  if (!V) return -5;
+  if (ldv < N) return -6;
+  if (strideV < 0) return -7;
+  if (!coef) return -8;
+  if (strideCoef < 0) return -9;
+  if (!out) return -10;
+  if (strideOut < 0) return -11;
+  Ctx ctx{(cudaStream_t)stream, B};
+  return lincomb_rows(ctx, N, k, ks, V, ldv, strideV, coef, strideCoef, out, strideOut, active);
 }
+
+size_t gegp_quad_grad_work_bytes(int n, int n_g, int d) { return gegp_quad_grad_batch_work_bytes(1, n, n_g, d); }
+
+size_t gegp_quad_grad_batch_work_bytes(int B, int n, int n_g, int d) {
+  if (bad_geom(n, n_g, d) || B <= 0) return 0;
+  const int N = n + n_g * d;
+  return ((size_t)round_up(N, 2) + (size_t)B * (size_t)round_up((int64_t)lml_grad_partial_doubles(n, d), 2)) *
+         sizeof(double);
+}
+
+}  // extern "C"
+
+namespace {
+// v_z^T (dKcov/dhp) v_z for ctx.batch vectors at once: rank-one weights (quad 1) of the LML-gradient contraction,
+// p^-1 = 1 (base mode) shared by every candidate, one partial table per candidate behind it in `work`.
+int quad_grad_rows(const Ctx& ctx, const Geom& gm, const double* theta, int64_t strideTheta, const double* v,
+                   int64_t strideV, double eta, int noisy, const double* varK, double* out, void* work) {
+  double* ones = reinterpret_cast<double*>(work);
+  double* partial = ones + round_up(gm.N, 2);
+  NoiseSpec ns{nullptr, 0, nullptr, 1.0, 0};
+  int rc = launch_prep_p(Ctx{ctx.stream, 1}, gm, theta, 0, ns, GEGP_MODE_BASE, nullptr, ones, 0);
+  if (rc) return rc;
+  return launch_lml_grad(ctx, gm, theta, strideTheta, nullptr, 0, 0, v, strideV, ones, 0, GEGP_MODE_BASE, eta, noisy,
+                         varK, 0.0, partial, round_up((int64_t)lml_grad_partial_doubles(gm.n, gm.d), 2), out,
+                         GEGP_OUT_LEN(gm.d), 1);
+}
+}  // namespace
+
+extern "C" {
 
 int gegp_quad_grad(int n, int n_g, int d, const double* X, const int32_t* grad_slot, const double* theta, int kernel, double kernel_hp,
                    const double* v, int mode, double eta, int noisy, const double* varK_dev, double* out, void* work,
@@ -510,16 +612,32 @@ int gegp_quad_grad(int n, int n_g, int d, const double* X, const int32_t* grad_s
   if (!out) return -12;
   if (!work || (reinterpret_cast<uintptr_t>(work) & 15)) return -13;
   if (work_bytes < gegp_quad_grad_work_bytes(n, n_g, d)) return -14;
-  const int N = n + n_g * d;
   Ctx ctx{(cudaStream_t)stream, 1};
-  const Geom gm = make_geom(n, n_g, d, X, grad_slot, kernel, kernel_hp);
-  double* ones = reinterpret_cast<double*>(work);           // p^-1 = 1 in base mode
-  double* partial = ones + round_up(N, 2);
-  NoiseSpec ns{nullptr, 0, nullptr, 1.0, 0};
-  int rc = launch_prep_p(ctx, gm, theta, 0, ns, GEGP_MODE_BASE, nullptr, ones, 0);
-  if (rc) return rc;
-  return launch_lml_grad(ctx, gm, theta, 0, nullptr, 0, 0, v, 0, ones, 0, mode, eta, noisy, varK_dev, 0.0, partial, 0, out,
-                         0, 1);
+  return quad_grad_rows(ctx, make_geom(n, n_g, d, X, grad_slot, kernel, kernel_hp), theta, 0, v, 0, eta, noisy, varK_dev,
+                        out, work);
+}
+
+int gegp_quad_grad_batch(int B, const double* theta_batch, const double* varK_batch, int kernel,
+                         const double* kernel_hp_batch, int n, int n_g, int d, const double* X, const int32_t* grad_slot,
+                         const double* V, int64_t ldv, int mode, double eta, int noisy, double* out, void* work,
+                         size_t work_bytes, void* stream) {
+  if (B <= 0 || B > 65535) return -1;
+  if (!theta_batch) return -2;
+  if (noisy && !varK_batch) return -3;
+  if (kernel < GEGP_KERNEL_SQEXP || kernel > GEGP_KERNEL_RATQUAD) return -50;
+  if (kernel == GEGP_KERNEL_RATQUAD && !kernel_hp_batch) return -50;
+  if (bad_geom(n, n_g, d)) return -6;
+  if (!X) return -9;
+  if (n_g != n && !grad_slot) return -10;
+  if (!V) return -11;
+  if (ldv < n + n_g * d) return -12;
+  if (mode != GEGP_MODE_BASE) return -13;
+  if (!out) return -16;
+  if (!work || (reinterpret_cast<uintptr_t>(work) & 15)) return -17;
+  if (work_bytes < gegp_quad_grad_batch_work_bytes(B, n, n_g, d)) return -18;
+  Ctx ctx{(cudaStream_t)stream, B};
+  const Geom gm = make_geom(n, n_g, d, X, grad_slot, kernel, 0.0, kernel_hp_batch);
+  return quad_grad_rows(ctx, gm, theta_batch, d, V, ldv, eta, noisy, varK_batch, out, work);
 }
 
 int gegp_weighted_grad(int n, int n_g, int d, const double* X, const int32_t* grad_slot, const double* theta, int kernel, double kernel_hp,

@@ -114,14 +114,21 @@ int trmv_upper(const Ctx& ctx, const double* U, int64_t ldu, int64_t strideU, co
 
 
 // --- extreme eigenpairs (Lanczos building blocks, csrc/eig.cu) ---
+// Each takes ctx.batch candidates at once: candidate z's arrays sit `stride` doubles after candidate 0's, and the
+// optional int32 list `active` names the candidate of each of the ctx.batch launch rows (nullptr: rows 0 .. batch-1).
+// The arithmetic for one candidate does not depend on the batch.
 // y = M x for a dense row-major N x ld matrix.
-int symv_full(const Ctx& ctx, int N, const double* M, int64_t ld, const double* x, double* y);
+int symv_full(const Ctx& ctx, int N, const double* M, int64_t ld, int64_t strideM, const double* x, int64_t strideX,
+              double* y, int64_t strideY, const int* active);
 // out[row] = sum_c |M[row, c]| (Gershgorin row sums for the variable nugget) or sum_c M[row, c]^2 (Frobenius norm).
 int row_abs_sum(const Ctx& ctx, int N, const double* M, int64_t ld, double* out, bool squares = false);
 // One Lanczos step with full re-orthogonalisation: V rows 0..j orthonormal, w = M v_j on entry; writes alpha[j],
 // beta[j] (device) and V row j+1 (j < 255).
-int lanczos_step(const Ctx& ctx, int N, int j, double* V, int64_t ldv, double* w, double* alpha, double* beta);
-// out = normalised sum_i coef[i] V_i (k <= 256, coef on the device).
-int lincomb_rows(const Ctx& ctx, int N, int k, const double* V, int64_t ldv, const double* coef, double* out);
+int lanczos_step(const Ctx& ctx, int N, int j, double* V, int64_t ldv, int64_t strideV, double* w, int64_t strideW,
+                 double* alpha, double* beta, int64_t strideAB, const int* active);
+// out = normalised sum_i coef[i] V_i (k <= 256, coef on the device); ks (optional, device): each candidate's own k,
+// clamped to 1 .. k.
+int lincomb_rows(const Ctx& ctx, int N, int k, const int* ks, const double* V, int64_t ldv, int64_t strideV,
+                 const double* coef, int64_t strideCoef, double* out, int64_t strideOut, const int* active);
 
 }  // namespace gegp

@@ -726,19 +726,29 @@ class GaussianProcess:
     def _cond_grad_from_vectors(self, hp_vals, res, varK):
         """dkappa/dhp = (v_max^T dKcov v_max - kappa v_min^T dKcov v_min) / max(lambda_min, 1e-16)
         (optz/GpHparaCon.py:178-193), the quadratic forms evaluated with dKcov/dhp generated on the fly."""
+        return self._cond_grads([hp_vals], [res], [varK])[0]
+
+    def _cond_grads(self, hp_list, res_list, varK_list):
+        """_cond_grad_from_vectors for many rows: the 2 quadratic forms of every row in one gegp_quad_grad_batch call."""
         if self.wellcond_mtd == "precon":
-            return None          # the reference has no condition-number gradient in precon mode (:171-173)
-        if res.get("v_max") is None:
-            return np.zeros(self.hp_info_optz_lkd.n_hp)
-        hi, d = self.hp_info_optz_lkd, self.dim
-        theta = np.asarray(hp_vals.theta, dtype=float)
-        noisy = self.b_has_noisy_data
-        kw = dict(n_g=self.n_grad, slot=self._slot_dev, eta=getattr(self, "_eta_used", self._etaK), noisy=noisy, varK=varK,
-                  kernel=self._kern(hp_vals))
-        qa = bk.quad_grad(self._X_dev, theta, res["v_max"], **kw).cpu().numpy()
-        qi = bk.quad_grad(self._X_dev, theta, res["v_min"], **kw).cpu().numpy()
-        q = (qa - res["cond"] * qi) / max(res["lam_min"], 1e-16)     # lam_min of Kcov (varK included)
-        return self._hp_row_to_grad(q)
+            return [None] * len(hp_list)   # the reference has no condition-number gradient in precon mode (:171-173)
+        out = [np.zeros(self.hp_info_optz_lkd.n_hp) for _ in hp_list]
+        live = [i for i, r in enumerate(res_list) if r.get("v_max") is not None]
+        if not live:
+            return out
+        import torch
+        th = np.vstack([np.asarray(hp_list[i].theta, dtype=float) for i in live])
+        V = torch.stack([res_list[i]["v_max"] for i in live] + [res_list[i]["v_min"] for i in live])
+        vk = np.array([float(varK_list[i]) for i in live])
+        khp = np.array([self._kern(hp_list[i])[1] for i in live])
+        q = bk.quad_grad_batch(self._X_dev, np.vstack([th, th]), V, n_g=self.n_grad, slot=self._slot_dev,
+                               eta=getattr(self, "_eta_used", self._etaK), noisy=self.b_has_noisy_data,
+                               varK_rows=np.hstack([vk, vk]), kernel=self._kern(), kernel_hp_rows=np.hstack([khp, khp])
+                               ).cpu().numpy()
+        for k, i in enumerate(live):
+            r = res_list[i]
+            out[i] = self._hp_row_to_grad((q[k] - r["cond"] * q[len(live) + k]) / max(r["lam_min"], 1e-16))
+        return out
 
     def _hp_row_to_grad(self, q):
         """GEGP_OUT_* row of per-hyper-parameter sums -> vector in the optimiser's hyper-parameter order."""
@@ -757,34 +767,63 @@ class GaussianProcess:
                 g[hi.idx_var_fgrad] = q[L.OUT_DVARG]
         return g
 
-    def _cond_from_workspace(self, hp_vals, calc_grad):
-        """Condition number (+ gradient) of the matrix whose factor L, L^-T and explicit inverse the likelihood
-        evaluation that has just run left in the workspace: the matrix itself is rebuilt into the (no longer needed)
-        L^-T buffer for the lambda_max products, lambda_min comes from products with the inverse."""
-        theta, noise, varK = self._cond_matrix_args(hp_vals)
-        v = bk.lml_views(self.n_eval, self.n_grad, self.dim)
-        mode, N = self._mode, self.n_data
+    def _rebuild_in_workspace(self, hp_list, calc_grad):
+        """Views of the len(hp_list) candidates whose factor, L^-T and explicit inverse the likelihood evaluation that
+        has just run left in the workspace, with each candidate's matrix rebuilt into its (no longer needed) L^-T buffer
+        for the lambda_max products (lambda_min comes from products with the inverse).  Every row shares the noise
+        vector of hp_list[0]."""
+        B, N, mode = len(hp_list), self.n_data, self._mode
+        v = bk.lml_views_batch(self.n_eval, self.n_grad, self.dim, B)
         if self.wellcond_mtd == "precon" and calc_grad:
             # reference quirk (optz/CalcLkd.py:341-343): with calc_grad the number returned in precon mode is kappa of
             # the UN-preconditioned Kcov = P Kt P, whose inverse is P^-1 Kt^-1 P^-1
             mode = L.MODE_PRECON_COV
-            v["Kinv"][:, :N].mul_(v["pinv"][:, None]).mul_(v["pinv"][None, :])
-        bk.build_cov(self._X_dev, theta, n_g=self.n_grad, slot=self._slot_dev, noise=noise, mode=mode,
-                     eta=getattr(self, "_eta_used", self._etaK), varK=varK, out=v["U"], kernel=self._kern(hp_vals))
+            v["Kinv"][:, :, :N].mul_(v["pinv"][:, :, None]).mul_(v["pinv"][:, None, :])
+        noise = varK = None
+        if self.b_has_noisy_data:      # the device divides the noise by each row's varK (kernel/Kernel.py:218)
+            nv = self.calc_noise_vec(hp_list[0])
+            noise = bk.to_dev(nv) if np.any(nv) else None
+            varK = np.array([float(h.varK) for h in hp_list])
+        bk.build_cov_batch(self._X_dev, np.vstack([np.asarray(h.theta, dtype=float) for h in hp_list]), n_g=self.n_grad,
+                           slot=self._slot_dev, noise=noise, varK_rows=varK, mode=mode,
+                           eta=getattr(self, "_eta_used", self._etaK), out=v["U"], kernel=self._kern(),
+                           kernel_hp_rows=np.array([self._kern(h)[1] for h in hp_list]))
+        return v
+
+    def _cond2_from_workspace(self, hp_list, calc_grad, warm, rows=None):
+        """kappa_2 (+ gradient) of every candidate of the evaluation that has just run (_rebuild_in_workspace), the
+        Lanczos iterations of all candidates batched (backend.cond2_batch); warm: one earlier result or None per row;
+        rows: the candidates to evaluate (default all; the others get None throughout).
+        -> (list of kappa, list of gradient or None, list of cond2 results)."""
+        v = self._rebuild_in_workspace(hp_list, calc_grad)
+        res = bk.cond2_batch(v["U"], v["Kinv"], self.n_data, warm=warm, rows=rows)
+        idx = [i for i, r in enumerate(res) if r is not None]
+        vk = [float(h.varK) if self.b_has_noisy_data else 1.0 for h in hp_list]
+        grads = [None] * len(hp_list)
+        if calc_grad:
+            for i, g in zip(idx, self._cond_grads([hp_list[i] for i in idx], [res[i] for i in idx], [vk[i] for i in idx])):
+                grads[i] = g
+        return [None if r is None else float(r["cond"]) for r in res], grads, res
+
+    def _cond_from_workspace(self, hp_vals, calc_grad):
+        """Condition number (+ gradient) of the matrix the likelihood evaluation that has just run factored."""
+        if self.cond_norm not in (2, "fro"):
+            raise Exception(f'cond_norm must be either 2 or "fro" but it is {self.cond_norm}')
         if self.cond_norm == "fro":   # optz/GpHparaCon.py:237-261
+            v = self._rebuild_in_workspace([hp_vals], calc_grad)
+            theta, _, varK = self._cond_matrix_args(hp_vals)
             want_w = calc_grad and self.wellcond_mtd != "precon"
-            cond, W = bk.cond_fro(v["U"], v["Kinv"], N, want_w)
+            cond, W = bk.cond_fro(v["U"][0], v["Kinv"][0], self.n_data, want_w)
             if not want_w:
                 return cond, None
             q = bk.weighted_grad(self._X_dev, theta, W, n_g=self.n_grad, slot=self._slot_dev,
                                  eta=getattr(self, "_eta_used", self._etaK), noisy=self.b_has_noisy_data,
                                  varK=varK, kernel=self._kern(hp_vals)).cpu().numpy()
             return cond, self._hp_row_to_grad(q)
-        if self.cond_norm != 2:
-            raise Exception(f'cond_norm must be either 2 or "fro" but it is {self.cond_norm}')
-        res = bk.cond2(v["U"], v["Kinv"], N, warm=getattr(self, "_last_cond", None) if self.cond_warm_start else None)
-        self._last_cond = res
-        return float(res["cond"]), (self._cond_grad_from_vectors(hp_vals, res, varK) if calc_grad else None)
+        warm = getattr(self, "_last_cond", None) if self.cond_warm_start else None
+        cond, grad, res = self._cond2_from_workspace([hp_vals], calc_grad, [warm])
+        self._last_cond = res[0]
+        return cond[0], grad[0]
 
     def _cond_on_failure(self, hp_vals, calc_grad=False):
         """Failed Cholesky: the reference substitutes -cond (and -cond_grad) for the objective (optz/OptzLkd.py:75-77).
@@ -799,15 +838,27 @@ class GaussianProcess:
         except Exception:
             return np.inf, (np.zeros(self.hp_info_optz_lkd.n_hp) if calc_grad else None)
 
-    def calc_lkd_batch(self, hp_vec_rows, calc_grad=False):
-        """LML (and d/dtheta) of many noise-free candidate rows at once, sharded over the process group.
+    def calc_lkd_batch(self, hp_vec_rows, calc_grad=False, calc_cond=False):
+        """LML (and d/dtheta) of many candidate rows at once, sharded over the process group.
 
         hp_vec_rows: [B, n_hp] in optimiser coordinates (log10 where bvec_log_optz).  Returns a NumPy table
         [B, 9+d] laid out as GEGP_OUT_* -- identical on every rank.  This is the batched form of the loops at
-        optz/GpHparaX0.py:39-45 and optz/OptzLkd.py:249-270."""
+        optz/GpHparaX0.py:39-45 and optz/OptzLkd.py:249-270.
+
+        calc_cond=True appends the 2-norm condition number kappa of the factored matrix as column 9+d and, with calc_grad
+        outside precon mode, dkappa/dhp in the optimiser's hyper-parameter order (n_hp columns more): row i holds what
+        calc_lkd_all(row i, calc_cond=True, calc_grad=calc_grad) returns as cond / cond_grad (a failed Cholesky takes
+        kappa from the shifted refactorisation of _cond_on_failure).  The likelihood columns then come from the
+        gradient-path evaluation calc_lkd_all runs for kappa; where kappa > cond_max_abs outside precon mode,
+        calc_lkd_all reports no likelihood and OUT_LML is NaN.  The Lanczos iterations of all rows run batched and are
+        not warm-started, so every row is bit-identical to calc_lkd_all with cond_warm_start = False.  Needs
+        cond_norm = 2 and a constant nugget."""
         rows = np.atleast_2d(np.asarray(hp_vec_rows, dtype=float))
         hi = self.hp_info_optz_lkd
         assert not (hi.has_var_fval or hi.has_var_fgrad), "rows with their own noise variance are evaluated one by one"
+        if calc_cond and (self.cond_norm != 2 or not self.cond_eta_is_const):
+            raise Exception("calc_lkd_batch(calc_cond=True) needs cond_norm = 2 and a constant nugget, but cond_norm = "
+                            f"{self.cond_norm} and cond_eta_is_const = {self.cond_eta_is_const}")
         th = rows[:, hi.idx_theta].copy()
         if self.optz_log_hp_theta:
             th = 10 ** th
@@ -826,13 +877,81 @@ class GaussianProcess:
         d = self.dim
         c_k = d if self.kernel_has_hp else None
         c_v = (d + (1 if self.kernel_has_hp else 0)) if self.b_has_noisy_data else None
+        width = L.out_len(d)
 
-        def eval_shard(c):
-            return self._eval_rows(c[:, :d].contiguous(), want_grad=calc_grad,
-                                   khp_rows=c[:, c_k].cpu().numpy() if c_k is not None else None,
-                                   varK_rows=c[:, c_v].cpu().numpy() if c_v is not None else None, noise_vec=noise)
-        table = parallel.sharded_eval(eval_shard, cand, self.dist_group, width=L.out_len(self.dim))
+        if not calc_cond:
+            def eval_shard(c):
+                return self._eval_rows(c[:, :d].contiguous(), want_grad=calc_grad,
+                                       khp_rows=c[:, c_k].cpu().numpy() if c_k is not None else None,
+                                       varK_rows=c[:, c_v].cpu().numpy() if c_v is not None else None, noise_vec=noise)
+        else:
+            with_grad = calc_grad and self.wellcond_mtd != "precon"
+            width += 1 + (hi.n_hp if with_grad else 0)
+
+            def eval_shard(c):
+                import torch
+                h = c.cpu().numpy()
+                hp_list = [self.make_hp_class(theta=h[i, :d].copy(), kernel=h[i, c_k] if c_k is not None else None,
+                                              varK=h[i, c_v] if c_v is not None else None) for i in range(h.shape[0])]
+                out, cond, cgrad = self._lkd_cond_rows(hp_list, calc_grad, noise)[:3]
+                tab = np.hstack([out, cond[:, None]] + ([cgrad] if with_grad else []))
+                return torch.as_tensor(tab).to(c.device)
+        table = parallel.sharded_eval(eval_shard, cand, self.dist_group, width=width)
         return table.cpu().numpy()
+
+    lml_ws_max_bytes = None   # cap on the likelihood workspace of batched evaluations that also need kappa (None: 60% free)
+
+    def _lkd_cond_rows(self, hp_list, calc_grad, noise=None, warm=None):
+        """Likelihood rows (gradient path, GEGP_OUT_*) and kappa_2 (+ dkappa/dhp outside precon mode) of many
+        hyper-parameter rows that share the nugget and the noise vector `noise`.  gegp_lml_eval reuses its workspace
+        chunk by chunk, so the rows go to the device in chunks that fit it, and kappa of a chunk is computed before the
+        next chunk overwrites its factors.  warm: None or one earlier cond2 result per row.
+        -> (out [B, 9+d], kappa [B], dkappa [B, n_hp] or None, the warm state each row leaves behind (what
+        calc_lkd_all leaves in _last_cond), b_chofac_good [B] as calc_lkd_all returns it)."""
+        B, d = len(hp_list), self.dim
+        n_hp = self.hp_info_optz_lkd.n_hp
+        with_grad = calc_grad and self.wellcond_mtd != "precon"
+        out = np.zeros((B, L.out_len(d)))
+        cond = np.zeros(B)
+        cgrad = np.zeros((B, n_hp)) if with_grad else None
+        warm = list(warm) if warm is not None else [None] * B
+        res_all = list(warm)
+        good_all = np.zeros(B, dtype=bool)
+        self._eta_used = self._etaK
+        last_cond = getattr(self, "_last_cond", None)
+        chunk = self._cond_chunk_rows(B)
+        for c0 in range(0, B, chunk):
+            part = hp_list[c0:c0 + chunk]
+            th = np.vstack([np.asarray(h.theta, dtype=float) for h in part])
+            khp = np.array([self._kern(h)[1] for h in part]) if self.kernel_has_hp else None
+            vk = np.array([float(h.varK) for h in part]) if self.b_has_noisy_data else None
+            o = self._eval_rows(th, want_grad=True, khp_rows=khp, varK_rows=vk, noise_vec=noise).cpu().numpy()
+            out[c0:c0 + len(part)] = o
+            good = [i for i in range(len(part)) if o[i, L.OUT_INFO] == 0]
+            if good:
+                c, g, res = self._cond2_from_workspace(part, calc_grad, warm[c0:c0 + len(part)], rows=good)
+                for i in good:
+                    cond[c0 + i], res_all[c0 + i] = c[i], res[i]
+                    if with_grad:
+                        cgrad[c0 + i] = g[i]
+            for i in range(len(part)):
+                if o[i, L.OUT_INFO] != 0:      # failed Cholesky: shifted refactorisation, row by row
+                    self._last_cond = warm[c0 + i]
+                    c, g = self._cond_on_failure(part[i], calc_grad)
+                    cond[c0 + i], res_all[c0 + i] = c, self._last_cond
+                    if with_grad:
+                        cgrad[c0 + i] = g
+                elif self.wellcond_mtd != "precon" and cond[c0 + i] > self.cond_max_abs:
+                    out[c0 + i, L.OUT_LML] = np.nan       # kernel/Kernel.py:282-283: no likelihood
+                else:
+                    good_all[c0 + i] = True
+        self._last_cond = last_cond
+        return out, cond, cgrad, res_all, good_all
+
+    def _cond_chunk_rows(self, B):
+        """Rows per likelihood call of _lkd_cond_rows: as many as the workspace keeps at once (lml_ws_max_bytes)."""
+        self._ensure_device()
+        return bk.lml_chunk_rows(self.n_eval, self.n_grad, self.dim, B, want_grad=True, max_ws_bytes=self.lml_ws_max_bytes)
 
     # ------------------------------------------------------------------ optimiser callbacks (optz/OptzLkd.py:16-113)
     def calc_store_likelihood(self, hp_vec, always_calc_cond=False, calc_grad=True):
@@ -1059,14 +1178,23 @@ class GaussianProcess:
                                         varK=None if self.b_has_noisy_data else 1)[4]
 
     def _can_batch_fit(self):
-        """The batched objective covers the noise-free, unconstrained (precon) fit with a constant nugget."""
-        return (not self.b_has_noisy_data) and (not self.b_use_cond_cstr) and self.cond_eta_is_const \
+        """The batched objective covers the noise-free fit with a constant nugget: unconstrained (precon), or with the
+        kappa_2 <= cond_max constraint of the base / rescale / dflt modes (adjoint-form gradient)."""
+        cstr_ok = (not self.b_use_cond_cstr) or (self.cond_norm == 2 and self.lkd_use_adj_mtd)
+        return (not self.b_has_noisy_data) and cstr_ok and self.cond_eta_is_const \
             and (not self.lkd_varK_pnlt_use) and self.optz_log_hp_theta and (not self.kernel_has_hp)
 
     def _optz_multistart_lockstep(self, hp_x0_all, optz_bound, opt):
         """Batch point B (optz/OptzLkd.py:249-270): every start row is its own SLSQP instance; their objective requests
         are evaluated together (multistart.minimize_lockstep), the start rows sharded over the ranks of dist_group.
-        Same trajectories and the same selected optimum as the sequential loop (batched == single, bit for bit)."""
+        Same trajectories and the same selected optimum as the sequential loop (batched == single, bit for bit).
+
+        With the condition-number constraint every request also returns kappa_2 and its gradient (_lkd_cond_rows, the
+        Lanczos iterations of all requests batched), following calc_store_likelihood exactly, and the per-start
+        bookkeeping of the sequential loop is reproduced.  Warm start: each start row begins from the GP's warm state
+        on entry and then carries its own, so start i follows the trajectory it would follow as the only start row of a
+        sequential fit begun in the same state (the sequential loop chains the warm vectors across start rows, so with
+        cond_warm_start the two agree to the Lanczos tolerance; without it, bit for bit)."""
         import torch
         from . import multistart
         hi = self.hp_info_optz_lkd
@@ -1074,6 +1202,8 @@ class GaussianProcess:
         n_optz = hp_x0_all.shape[0]
         lo, hi_row = parallel.shard_bounds(n_optz, rank, size)
         d = self.dim
+        cstr = self.b_use_cond_cstr
+        warm_state = {i: getattr(self, "_last_cond", None) for i in range(lo, hi_row)}
 
         def batch_val_and_grad(Xlog):
             th = 10 ** Xlog[:, hi.idx_theta]
@@ -1092,29 +1222,79 @@ class GaussianProcess:
                     vals[r] = self._cond_on_failure(hp_vals, False)[0]
             return vals, grads
 
-        local = np.full((max(hi_row - lo, 0), hi.n_hp + 3), np.nan)
+        def batch_cond(Xlog, ids):
+            """calc_store_likelihood(x, calc_grad=True) for every request, negated for minimisation."""
+            hp_list = [self.hp_vec2dataclass(hi, x) for x in Xlog]
+            warm = [warm_state[i] for i in ids] if self.cond_warm_start else None
+            out, cond, cgrad, res, good = self._lkd_cond_rows(hp_list, True, None, warm)
+            if self.cond_warm_start:
+                warm_state.update(zip(ids, res))
+            b = hi.bvec_log_optz
+            vals, grads, cgs = np.empty(len(ids)), np.zeros((len(ids), hi.n_hp)), np.zeros((len(ids), hi.n_hp))
+            for r, hp_vec in enumerate(Xlog):
+                if good[r]:
+                    val = out[r, L.OUT_LML]
+                    grad = np.zeros(hi.n_hp)
+                    grad[hi.idx_theta] = out[r, L.OUT_GRAD:L.OUT_GRAD + d]
+                    grad[b] *= 10 ** hp_vec[b] * np.log(10)
+                    cg = cgrad[r].copy()
+                    cg[b] *= 10 ** hp_vec[b] * np.log(10)
+                else:   # failed Cholesky or kappa > cond_max_abs: -kappa is the objective (optz/OptzLkd.py:75-77)
+                    val, grad, cg = -cond[r], -cgrad[r], cgrad[r]
+                vals[r], grads[r], cgs[r] = -val, -grad, cg
+            return vals, grads, cond.copy(), cgs
+
+        W = hi.n_hp + (6 if cstr else 3)
+        local = np.full((max(hi_row - lo, 0), W), np.nan)
         self._lockstep_stats = None
         if hi_row > lo:
             cur_dev = torch.cuda.current_device() if torch.cuda.is_available() else None
             init = (lambda: torch.cuda.set_device(cur_dev)) if cur_dev is not None else None
-            res, ev = multistart.minimize_lockstep(batch_val_and_grad, hp_x0_all[lo:hi_row], optz_bound, opt,
-                                                   thread_init=init)
+            if cstr:
+                res, ev = multistart.minimize_lockstep(batch_cond, hp_x0_all[lo:hi_row], optz_bound, opt,
+                                                       thread_init=init, with_ids=True, cond_ub=self.condnum_nlc.ub)
+            else:
+                res, ev = multistart.minimize_lockstep(batch_val_and_grad, hp_x0_all[lo:hi_row], optz_bound, opt,
+                                                       thread_init=init)
             self._lockstep_stats = dict(n_batches=ev.n_batches, n_evals=ev.n_evals, batch_sizes=ev.batch_sizes)
             for i, r in enumerate(res):
-                local[i, :hi.n_hp], local[i, hi.n_hp:] = r.x, (r.fun, float(r.success), r.nit)
+                local[i, :hi.n_hp], local[i, hi.n_hp:hi.n_hp + 3] = r.x, (r.fun, float(r.success), r.nit)
+                if cstr:   # kappa at the solution; LML and kappa at x0 (-objective is the LML, or -kappa on failure)
+                    local[i, hi.n_hp + 3:] = (ev.at_solution[i][2], -ev.at_x0[i][0], ev.at_x0[i][2])
         if size > 1:
             # a rank without start rows (more ranks than rows) contributes an empty block but enters the collective
             t = torch.as_tensor(local)
             t = t.to(bk.device()) if torch.cuda.is_available() else t
-            table = parallel.gather_rows(t, n_optz, self.dist_group, width=hi.n_hp + 3).cpu().numpy()
+            table = parallel.gather_rows(t, n_optz, self.dist_group, width=W).cpu().numpy()
         else:
             table = local
-        self._multistart_table = table          # per start row: solution, objective, success, iterations
+        self._multistart_table = table   # per start row: solution, objective, success, iterations (+ kappa columns)
         sol, obj, ok, nit = table[:, :hi.n_hp], table[:, hi.n_hp], table[:, hi.n_hp + 1], table[:, hi.n_hp + 2]
-        best = sol[np.nanargmin(obj), :]
+        if not cstr:
+            best = sol[np.nanargmin(obj), :]
+            info = {"hp_optz_success": float(np.mean(ok)), "hp_optz_iter_mean": float(np.mean(nit)),
+                    "hp_optz_iter_max": float(np.max(nit)), "hp_optz_con_good": 1.0, "optz_n_cho_fail": 0,
+                    "optz_n_cond2big": 0, "optz_max_init_cond": np.nan}
+            return best, self._final_cond(best), info
+        cond_sol, lkd_x0, cond_x0 = table[:, hi.n_hp + 3], table[:, hi.n_hp + 4], table[:, hi.n_hp + 5]
+        n_cho_fail = n_cond2big = 0
+        max_init_cond = np.nan
+        for i in range(n_optz):          # the bookkeeping of the sequential loop, in its order
+            max_init_cond = np.nanmax((max_init_cond, cond_x0[i]))
+            if np.isnan(lkd_x0[i]):
+                n_cho_fail += 1
+            if cond_x0[i] > self.cond_max:
+                n_cond2big += 1
+        con_good = cond_sol < 1.01 * self.cond_max
+        if np.any(con_good):
+            obj_ok, sol_ok = obj[con_good], sol[con_good, :]
+        else:
+            print("*** No solutions satisfy the constraints for the GP hyperparameter optimization ***")
+            obj_ok, sol_ok = obj, sol
+        best = sol_ok[np.nanargmin(obj_ok), :]
         info = {"hp_optz_success": float(np.mean(ok)), "hp_optz_iter_mean": float(np.mean(nit)),
-                "hp_optz_iter_max": float(np.max(nit)), "hp_optz_con_good": 1.0, "optz_n_cho_fail": 0,
-                "optz_n_cond2big": 0, "optz_max_init_cond": np.nan}
+                "hp_optz_iter_max": float(np.max(nit)), "hp_optz_con_good": float(np.mean(con_good)),
+                "optz_n_cho_fail": n_cho_fail, "optz_n_cond2big": n_cond2big, "optz_max_init_cond": max_init_cond}
         return best, self._final_cond(best), info
 
     def rescaling_data_w_theta_sol(self, X_scl_v1, xvec_scale_v1, hp_theta, tol_min_dist_x=1e-15):

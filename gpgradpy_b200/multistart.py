@@ -14,7 +14,7 @@ from __future__ import annotations
 import threading
 
 import numpy as np
-from scipy.optimize import minimize
+from scipy.optimize import NonlinearConstraint, minimize
 
 
 class LockstepEvaluator:
@@ -66,43 +66,55 @@ class LockstepEvaluator:
                 self._flush_locked()
 
 
-def minimize_lockstep(batch_val_and_grad, x0_rows, bounds, options, constraints=(), thread_init=None):
+def minimize_lockstep(batch_val_and_grad, x0_rows, bounds, options, constraints=(), thread_init=None, *,
+                      with_ids=False, cond_ub=None):
     """SLSQP from every row of x0_rows, objective/gradient requests batched across the rows.
 
-    batch_val_and_grad(X [b, n_hp]) -> (vals [b], grads [b, n_hp]) of the function to MINIMISE.
+    batch_val_and_grad(X [b, n_hp]) -> (vals [b], grads [b, n_hp]) of the function to MINIMISE; with_ids: it is called
+    as batch_val_and_grad(X, ids) with the start row of every request (for per-start state such as warm starts).
     thread_init: called first in every worker thread (the CUDA device is per-thread state: a worker that ends up
     running the batched device call must select the caller's device).
+    cond_ub: the condition-number-constrained fit of optz/OptzLkd.py:225-270.  batch_val_and_grad then also returns
+    (conds [b], cond_grads [b, n_hp]); every start gets the SLSQP constraint cond <= cond_ub, whose callbacks read the
+    start's cache that the same request filled.  As in the sequential loop, every start is evaluated once at its x0
+    before its SLSQP runs (with a cleared cache afterwards) and once more at its solution; those two results per start
+    are kept in ev.at_x0 and ev.at_solution as (val, grad, cond, cond_grad).
     Returns (list of scipy OptimizeResult in row order, LockstepEvaluator with its statistics)."""
     x0_rows = np.atleast_2d(np.asarray(x0_rows, dtype=float))
     n = x0_rows.shape[0]
 
     def batch_fn(req):
         X = np.vstack([x for _, x in req])
-        vals, grads = batch_val_and_grad(X)
-        return {i: (float(vals[k]), np.array(grads[k], dtype=float)) for k, (i, _) in enumerate(req)}
+        outs = batch_val_and_grad(X, [i for i, _ in req]) if with_ids else batch_val_and_grad(X)
+        return {i: tuple(float(o[k]) if np.ndim(o[k]) == 0 else np.array(o[k], dtype=float) for o in outs)
+                for k, (i, _) in enumerate(req)}
 
     ev = LockstepEvaluator(batch_fn, n)
+    ev.at_x0, ev.at_solution = [None] * n, [None] * n
     results = [None] * n
     errors = [None] * n
 
     def worker(i):
-        last = {"x": None, "val": None, "grad": None}
+        last = {"x": None, "r": None}
 
-        def fun(x):
+        def get(x):
             if last["x"] is None or not np.array_equal(x, last["x"]):
-                v, g = ev.evaluate(i, x)
-                last.update(x=np.array(x, copy=True), val=v, grad=g)
-            return last["val"]
-
-        def jac(x):
-            fun(x)
-            return last["grad"]
+                r = ev.evaluate(i, x)
+                last.update(x=np.array(x, copy=True), r=r)
+            return last["r"]
 
         try:
             if thread_init is not None:
                 thread_init()
-            results[i] = minimize(fun, x0_rows[i], method="SLSQP", jac=jac, bounds=bounds, constraints=constraints,
-                                  options=options)
+            cons = constraints
+            if cond_ub is not None:
+                ev.at_x0[i] = get(x0_rows[i])
+                last["x"] = None
+                cons = NonlinearConstraint(lambda x: get(x)[2], -np.inf, cond_ub, jac=lambda x: get(x)[3])
+            results[i] = minimize(lambda x: get(x)[0], x0_rows[i], method="SLSQP", jac=lambda x: get(x)[1],
+                                  bounds=bounds, constraints=cons, options=options)
+            if cond_ub is not None:
+                ev.at_solution[i] = get(results[i].x)
         except BaseException as exc:   # noqa: BLE001
             errors[i] = exc
         finally:

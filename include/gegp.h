@@ -247,6 +247,40 @@ int gegp_quad_grad(int n, int n_g, int d, const double* X, const int32_t* grad_s
                    const double* v, int mode, double eta, int noisy, const double* varK_dev, double* out,
                    void* work, size_t work_bytes, void* stream);
 
+/* Batched forms of the condition-number building blocks for B candidates of one problem geometry (the B matrices that
+ * B likelihood evaluations leave in the gegp_lml_eval workspace, gegp_lml_layout): candidate z's arrays sit
+ * z * stride doubles after candidate 0's.  `active` (int32[B] on the device, or NULL for 0 .. B-1) names the candidate
+ * of each of the B launch rows, so candidates that have converged drop out without copying.  A candidate's results do
+ * not depend on B, on the other candidates or on `active`: each is bit-identical to the single-candidate call.
+ *   gegp_symv_batch:          y_z = M_z x_z (M 16-byte aligned, ld and strideM even, x 16-byte aligned, strideX even);
+ *                             B <= 65535.
+ *   gegp_lanczos_step_batch:  gegp_lanczos_step on every candidate at the same step j; alpha_z, beta_z are strideAB apart.
+ *   gegp_lincomb_batch:       gegp_lincomb per candidate; ks (int32[.] on the device, indexed by candidate, or NULL)
+ *                             gives candidate z its own basis size ks[z] (clamped to 1 .. k), k <= 256.
+ *   gegp_quad_grad_batch:     gegp_quad_grad for B vectors V + z * ldv, each with its own theta row (theta_batch[B, d]),
+ *                             varK (varK_batch[B], when noisy) and kernel hyper-parameter (kernel_hp_batch[B], required
+ *                             for the rational-quadratic kernel); out[B, GEGP_OUT_LEN(d)] (zeroed by the caller).
+ *                             work >= gegp_quad_grad_batch_work_bytes(B, n, n_g, d).
+ *   gegp_build_cov_batch:     gegp_build_cov for B theta rows into K_out + z * strideK.  varK_batch[B] or NULL (1); with
+ *                             both noise and varK_batch the noise is divided by varK_z (kernel/Kernel.py:218).  p_out
+ *                             (p then 1/p, strideP >= 2N apart) is required for GEGP_MODE_PRECON, else may be NULL. */
+int gegp_symv_batch(int B, int N, const double* M, int64_t ld, int64_t strideM, const double* x, int64_t strideX,
+                    double* y, int64_t strideY, const int32_t* active, void* stream);
+int gegp_lanczos_step_batch(int B, int N, int j, double* V, int64_t ldv, int64_t strideV, double* w, int64_t strideW,
+                            double* alpha, double* beta, int64_t strideAB, const int32_t* active, void* stream);
+int gegp_lincomb_batch(int B, int N, int k, const int32_t* ks, const double* V, int64_t ldv, int64_t strideV,
+                       const double* coef, int64_t strideCoef, double* out, int64_t strideOut, const int32_t* active,
+                       void* stream);
+size_t gegp_quad_grad_batch_work_bytes(int B, int n, int n_g, int d);
+int gegp_quad_grad_batch(int B, const double* theta_batch, const double* varK_batch, int kernel,
+                         const double* kernel_hp_batch, int n, int n_g, int d, const double* X, const int32_t* grad_slot,
+                         const double* V, int64_t ldv, int mode, double eta, int noisy, double* out, void* work,
+                         size_t work_bytes, void* stream);
+int gegp_build_cov_batch(int B, const double* theta_batch, const double* varK_batch, int kernel,
+                         const double* kernel_hp_batch, int n, int n_g, int d, const double* X, const int32_t* grad_slot,
+                         const double* noise, int mode, double eta, double* K_out, int64_t ldk, int64_t strideK,
+                         double* p_out, int64_t strideP, int uplo, void* stream);
+
 /* Direct (non-adjoint) likelihood form, lkd_use_adj_mtd = False (optz/CalcLkd.py:64-85, 104-116, 135-147, 349-367;
  * eval/GpMeanFun.py:110-120; noisy data: optz/CalcLkd.py:206-207, 238-241, 253-265).  The reference forms, for every
  * hyper-parameter hp_k with D_k = dKcov/dhp_k:  a^T D_k a,  h^T D_k a  and  tr(K^-1 D_k)  (a = K^-1 (y - H beta),
