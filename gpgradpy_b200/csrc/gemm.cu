@@ -5,7 +5,7 @@
 // kernel.  CTA tile BM x BN x 16, multi-stage cp.async pipeline into padded shared memory whose row
 // strides (20 / BN+4 doubles) make every DMMA fragment load bank-conflict free, warp tile WM x WN built
 // from m8n8k4 fp64 MMAs.  Triangular operands are exploited by clipping the k range per output tile.
-#include "linalg.h"
+#include "gemm_tile.cuh"
 #include <cstdlib>
 
 namespace gegp {
@@ -33,17 +33,8 @@ gemm_f64_kernel(const GemmArgs g) {
   double* sA = smem;
   double* sB = smem + STAGES * Cfg::A_STAGE;
 
-  // k range clipped above by the column tile (KHI_N0): the work of a tile grows with its column.  CTAs are dispatched
-  // in linear blockIdx order, so the tiles are re-mapped to longest-processing-time-first: all tiles of the last
-  // (longest) column, then the one before, ...  (list-scheduling simulation of the 32 x 32-tile product of the inverse on
-  // 592 CTA slots: makespan 1.73x the ideal in row-major order, 1.10x in this order; ncu showed the SMs idle a third of
-  // the kernel before.)
   int bx = blockIdx.x, by = blockIdx.y;
-  if (g.khi_mode == KHI_N0) {
-    const int lin = blockIdx.y * gridDim.x + blockIdx.x;
-    bx = (int)gridDim.x - 1 - lin / (int)gridDim.y;
-    by = lin % (int)gridDim.y;
-  }
+  if (g.khi_mode == KHI_N0) longest_first(bx, by);
   const int m0 = by * BM, n0 = bx * BN;
   if (g.cmode != C_FULL && n0 >= m0 + BM) return;  // tile entirely above the diagonal
 
@@ -53,14 +44,8 @@ gemm_f64_kernel(const GemmArgs g) {
   double* __restrict__ C = g.C + zo * g.sCo + zi * g.sCi;
   double* __restrict__ Ct = g.Ct ? g.Ct + zo * g.sCto + zi * g.sCti : nullptr;
 
-  int kb = 0, ke = g.K;
-  if (g.klo_mode == KLO_M0) kb = m0;
-  else if (g.klo_mode == KLO_N0) kb = n0;
-  else if (g.klo_mode == KLO_MAXMN) kb = max(m0, n0);
-  if (g.khi_mode == KHI_M0) ke = min(ke, m0 + BM);
-  else if (g.khi_mode == KHI_N0) ke = min(ke, g.khi_off + n0 + BN);
-  kb = (kb / BK) * BK;
-  const int ktiles = ke > kb ? (ke - kb + BK - 1) / BK : 0;
+  const KRange kr = tile_k_range<BN, BK>(g, m0, n0);
+  const int kb = kr.kb, ke = kr.ke, ktiles = kr.tiles;
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int wm0 = (warp / Cfg::WARPS_N) * WM, wn0 = (warp % Cfg::WARPS_N) * WN;
@@ -178,40 +163,14 @@ gemm_f64_kernel(const GemmArgs g) {
   }
   cp_async_wait<0>();
 
-  // epilogue
   const bool vec_ok = ((g.ldc & 1) == 0) && ((reinterpret_cast<uintptr_t>(C) & 15) == 0);
 #pragma unroll
   for (int i = 0; i < Cfg::MI; i++) {
     const int row = m0 + wm0 + i * 8 + lr;
     if (row >= g.M) continue;
 #pragma unroll
-    for (int j = 0; j < Cfg::NI; j++) {
-      const int col = n0 + wn0 + j * 8 + 2 * lk;
-      if (col >= g.N) continue;
-      double* cp = C + (int64_t)row * g.ldc + col;
-      double v0 = g.alpha * acc[i][j][0], v1 = g.alpha * acc[i][j][1];
-      const bool has1 = (col + 1 < g.N);
-      bool st0 = true, st1 = has1;
-      if (g.cmode != C_FULL) { st0 = (col <= row); st1 = has1 && (col + 1 <= row); }
-      if (g.beta != 0.0) {
-        if (st0) v0 += g.beta * cp[0];
-        if (st1) v1 += g.beta * cp[1];
-      }
-      if (st0 && st1 && vec_ok) {
-        *reinterpret_cast<double2*>(cp) = make_double2(v0, v1);
-      } else {
-        if (st0) cp[0] = v0;
-        if (st1) cp[1] = v1;
-      }
-      if (g.cmode == C_LOWER_MIRROR) {
-        if (st0 && col < row) C[(int64_t)col * g.ldc + row] = v0;
-        if (st1 && col + 1 < row) C[(int64_t)(col + 1) * g.ldc + row] = v1;
-      }
-      if (Ct) {
-        if (st0) Ct[(int64_t)col * g.ldct + row] = v0;
-        if (st1) Ct[(int64_t)(col + 1) * g.ldct + row] = v1;
-      }
-    }
+    for (int j = 0; j < Cfg::NI; j++)
+      store_pair(g, C, Ct, vec_ok, row, n0 + wn0 + j * 8 + 2 * lk, acc[i][j][0], acc[i][j][1]);
   }
 }
 
@@ -228,16 +187,10 @@ double gemm_useful_flops(const GemmArgs& g) {
 template <int BM, int BN, int WM, int WN, int STAGES, bool B_KCONT>
 static int launch_cfg(const Ctx& ctx, const GemmArgs& g) {
   using Cfg = GemmCfg<BM, BN, WM, WN, STAGES, B_KCONT>;
-  auto kern = gemm_f64_kernel<BM, BN, WM, WN, STAGES, B_KCONT>;
-  GEGP_SET_SMEM(kern, Cfg::SMEM);
-  dim3 grid((g.N + BN - 1) / BN, (g.M + BM - 1) / BM, g.outer * g.inner);
-  prof_gemm_begin(ctx.stream);
-  timeline_begin(ctx.stream, BM == 32 ? "gemm32" : (BM == 64 ? (STAGES == 2 ? "gemm64s2" : "gemm64s4") : "gemm128"), g.M, g.N, g.K, timeline_on() ? gemm_useful_flops(g) * 1e-6 : 0.0);
-  kern<<<grid, Cfg::THREADS, Cfg::SMEM, ctx.stream>>>(g);
-  timeline_end(ctx.stream);
-  if (prof().on) prof_gemm_end(ctx.stream, gemm_useful_flops(g));
-  GEGP_CHECK_LAUNCH();
-  return 0;
+  const dim3 grid((g.N + BN - 1) / BN, (g.M + BM - 1) / BM, g.outer * g.inner);
+  const char* label = BM == 32 ? "gemm32" : (BM == 64 ? (STAGES == 2 ? "gemm64s2" : "gemm64s4") : "gemm128");
+  return launch_gemm<gemm_f64_kernel<BM, BN, WM, WN, STAGES, B_KCONT>>(ctx, g, grid, Cfg::THREADS, Cfg::SMEM, label, g.M,
+                                                                       g.N, g.K, g);
 }
 
 
@@ -316,44 +269,16 @@ gemm_k128_kernel(const GemmArgs g) {
     const int row = m0 + r0 + i * 8 + lr;
     if (row >= g.M) continue;
 #pragma unroll
-    for (int j = 0; j < NI; j++) {
-      const int col = c0 + j * 8 + 2 * lk;
-      if (col >= g.N) continue;
-      double* cp = C + (int64_t)row * g.ldc + col;
-      double v0 = g.alpha * acc[i][j][0], v1 = g.alpha * acc[i][j][1];
-      const bool has1 = (col + 1 < g.N);
-      bool st0 = true, st1 = has1;
-      if (g.cmode != C_FULL) { st0 = (col <= row); st1 = has1 && (col + 1 <= row); }
-      if (g.beta != 0.0) {
-        if (st0) v0 += g.beta * cp[0];
-        if (st1) v1 += g.beta * cp[1];
-      }
-      if (st0 && st1 && vec_ok) {
-        *reinterpret_cast<double2*>(cp) = make_double2(v0, v1);
-      } else {
-        if (st0) cp[0] = v0;
-        if (st1) cp[1] = v1;
-      }
-      if (g.cmode == C_LOWER_MIRROR) {
-        if (st0 && col < row) C[(int64_t)col * g.ldc + row] = v0;
-        if (st1 && col + 1 < row) C[(int64_t)(col + 1) * g.ldc + row] = v1;
-      }
-    }
+    for (int j = 0; j < NI; j++)
+      store_pair(g, C, nullptr, vec_ok, row, c0 + j * 8 + 2 * lk, acc[i][j][0], acc[i][j][1]);
   }
 }
 
 template <int BM>
 static int launch_k128(const Ctx& ctx, const GemmArgs& g) {
   const size_t smem = (size_t)(BM + 128) * K128_LD * sizeof(double);
-  GEGP_SET_SMEM(gemm_k128_kernel<BM>, smem);
-  dim3 grid((g.M + BM - 1) / BM, 1, g.outer);
-  prof_gemm_begin(ctx.stream);
-  timeline_begin(ctx.stream, "gemm_k128", g.M, g.N, BM, timeline_on() ? gemm_useful_flops(g) * 1e-6 : 0.0);
-  gemm_k128_kernel<BM><<<grid, 256, smem, ctx.stream>>>(g);
-  timeline_end(ctx.stream);
-  if (prof().on) prof_gemm_end(ctx.stream, gemm_useful_flops(g));
-  GEGP_CHECK_LAUNCH();
-  return 0;
+  return launch_gemm<gemm_k128_kernel<BM>>(ctx, g, dim3((g.M + BM - 1) / BM, 1, g.outer), 256, smem, "gemm_k128", g.M,
+                                           g.N, BM, g);
 }
 
 // rows per CTA: the smallest of 16 / 32 / 64 that still gives every CTA an SM of its own (one wave), else 64
@@ -383,11 +308,21 @@ GemmArgs gemm_args(const double* A, int64_t lda, const double* B, int64_t ldb, d
   g.M = M; g.N = N; g.K = K; g.alpha = alpha; g.beta = beta; g.b_kcont = b_kcont;
   g.klo_mode = KLO_ZERO; g.khi_mode = KHI_K; g.cmode = C_FULL; g.khi_off = 0;
   g.inner = 1; g.outer = 1;
-  g.row_owner = false;
   g.inner_steps = false; g.iAr = g.iAc = g.iBr = g.iBc = 0;
   g.Ct = nullptr; g.ldct = 0; g.sCto = g.sCti = 0;
   g.sAo = g.sBo = g.sCo = g.sAi = g.sBi = g.sCi = 0;
   return g;
+}
+
+// output tiles of one M x N problem in tile x tile tiles; a lower-triangular output skips those strictly above the diagonal
+static long tiles(int M, int N, int tile, int cmode) {
+  const long rt = (M + tile - 1) / tile, ct = (N + tile - 1) / tile;
+  long t = rt * ct;
+  if (cmode != C_FULL) {
+    const long sq = rt < ct ? rt : ct;
+    t -= sq * (sq - 1) / 2 + (ct > rt ? (ct - rt) * rt : 0);
+  }
+  return t;
 }
 
 int gemm_f64(const Ctx& ctx, GemmArgs g) {
@@ -400,24 +335,12 @@ int gemm_f64(const Ctx& ctx, GemmArgs g) {
   // Large tile when one problem still fills the machine with it, small tile otherwise.  The choice depends on the
   // shape of ONE problem only, never on the batch count: a candidate evaluated alone, in a batch, or on another rank
   // of a sharded batch goes through the same kernels and gives bit-identical results.
-  const long rt = (g.M + 127) / 128, ct = (g.N + 127) / 128;
-  long tiles_big = rt * ct;
-  if (g.cmode != C_FULL) {   // tiles strictly above the diagonal are skipped
-    const long sq = rt < ct ? rt : ct;
-    tiles_big -= sq * (sq - 1) / 2 + (ct > rt ? (ct - rt) * rt : 0);
-  }
-  tiles_big *= g.inner;
+  const long tiles_big = tiles(g.M, g.N, 128, g.cmode) * g.inner;
   // Measured on B200 (d=10, n=500 and d=20, n=1000 evaluations): with fewer than ~400 tiles of 128 x 128 per problem
   // the TMA kernel loses more to wave quantisation than it gains over the 64 x 64 cp.async kernel; between 400 and 1000
   // the two are equal, above the TMA kernel wins (measured with 128 x 64 tiles on 296 CTA slots; re-checked at both sizes
   // with the 128 x 128 tiles / 148 slots the kernel has now: 150 ... 400 give the same evaluation times).
   const bool big = tiles_big >= tma_min_tiles() && g.M >= 128 && g.N >= 128;
-  if (g.row_owner) {
-    // in-place right multiply: one column tile must cover all of N so that a CTA only overwrites rows it alone reads
-    if (g.N > 128 || g.A != g.C || g.b_kcont) return -904;
-    return launch_cfg<128, 128, 64, 32, 4, false>(ctx, g);
-  }
-  static const int exp_cfg = getenv("GEGP_GEMM_CFG") ? atoi(getenv("GEGP_GEMM_CFG")) : 0;  // tuning experiments
   // K = LEAF panel updates (tall, at most 128 wide): the single-wave kernel; BM (rows per CTA) only changes which CTA
   // owns a row, not the arithmetic of an element.
   // Only while one wave of whole-SM CTAs covers the panel (M <= 148 * 64): beyond that the problem is throughput-bound and
@@ -425,9 +348,9 @@ int gemm_f64(const Ctx& ctx, GemmArgs g) {
   // It accumulates every element in the same k order as the generic kernels (bit-identical results, tested), which is why
   // this choice -- like the 32 x 32 one below -- may look at the batch count.
   if (g.b_kcont && g.K == K128 && g.N <= 128 && g.klo_mode == KLO_ZERO && g.khi_mode == KHI_K && !g.Ct && g.inner == 1 &&
-      (long)g.M * g.outer <= 148L * 64 && exp_cfg != 7)
+      (long)g.M * g.outer <= 148L * 64)
     return gemm_k128(ctx, g);
-  if (g.b_kcont && big && exp_cfg != 9) {
+  if (g.b_kcont && big) {
     const int rc = gemm_tma_nt(ctx, g);
     if (rc <= 0) return rc;
   }
@@ -437,22 +360,15 @@ int gemm_f64(const Ctx& ctx, GemmArgs g) {
     // path: 128 x 128 x K, lower) is bound by the latency of ONE CTA walking K; 32 x 32 tiles put it on 4x as many
     // SMs.  Same k order per output element, so the result does not depend on the tile size (tested bit for bit),
     // which is why this choice -- unlike the TMA one -- may look at the batch count.
-    long t64 = ((g.M + 63) / 64) * (long)((g.N + 63) / 64);
-    if (g.cmode != C_FULL) {
-      const long r64 = (g.M + 63) / 64, c64 = (g.N + 63) / 64, sq = r64 < c64 ? r64 : c64;
-      t64 -= sq * (sq - 1) / 2 + (c64 > r64 ? (c64 - r64) * r64 : 0);
-    }
-    if (t64 * g.inner * g.outer <= small_tile_max()) return launch_cfg<32, 32, 16, 16, 4, true>(ctx, g);
+    const long ctas = tiles(g.M, g.N, 64, g.cmode) * g.inner * g.outer;   // of 64 x 64 tiles
+    if (ctas <= small_tile_max()) return launch_cfg<32, 32, 16, 16, 4, true>(ctx, g);
     // skinny and deep (one block column updated by a long panel: the just-in-time pieces of the factorisation that the
     // critical path reaches first): less than one 64 x 64 tile per SM, each walking a long K -- 32 x 32 tiles again
-    if (g.N <= 128 && g.K >= 512 && t64 * g.inner * g.outer <= 148 && exp_cfg != 5)
-      return launch_cfg<32, 32, 16, 16, 4, true>(ctx, g);
+    if (g.N <= 128 && g.K >= 512 && ctas <= 148) return launch_cfg<32, 32, 16, 16, 4, true>(ctx, g);
     // 64 x 64 tiles: with enough CTAs to give every SM several, a 2-stage ring (41 KB, 4 CTAs = 16 warps per SM)
     // beats the 4-stage one (82 KB, 2 CTAs per SM) by 10-15 % (measured: 2048^3 32.5 vs 28.2 TFLOP/s, the batched
     // N=1200 scan +12 %); with few CTAs the deeper prefetch of the 4-stage ring wins.  Same arithmetic either way.
-    const long ctas = t64 * g.inner * g.outer;
-    const bool many = exp_cfg == 2 ? true : (exp_cfg == 4 ? false : ctas >= 4 * 148);
-    if (many) return launch_cfg<64, 64, 32, 32, 2, true>(ctx, g);
+    if (ctas >= 4 * 148) return launch_cfg<64, 64, 32, 32, 2, true>(ctx, g);
     return launch_cfg<64, 64, 32, 32, 4, true>(ctx, g);
   } else {
     if (big) return launch_cfg<128, 128, 64, 32, 4, false>(ctx, g);

@@ -13,9 +13,8 @@
 // index, so each DMMA step s may pick any 4 of the 16 k values as long as A and B pick the same ones: lanes with
 // (lane & 3) < 2 read chunk s, the others chunk s + 4, which makes the 16 lanes of a half-warp touch all eight
 // chunk positions of the line exactly once.
-#include "linalg.h"
+#include "gemm_tile.cuh"
 #include <cuda.h>
-#include <cstdlib>
 #include <cstring>
 #include <mutex>
 #include <unordered_map>
@@ -28,25 +27,22 @@ constexpr int TBK = 16;
 constexpr int TWM = 64, TWN = 32;                  // warp tile
 constexpr int TMI = TWM / 8, TNI = TWN / 8;
 
-// CTA tile TBM x TBN (multiples of the 64 x 32 warp tile), TSTAGES-deep ring, MINB CTAs per SM.
-// SOLO: the CTA asks for ALL the shared memory a block may have (227 KB), so that no other CTA -- of this grid, of
-// another kernel of this library or of a foreign kernel on another stream -- can share its SM.
-template <int TBM_, int TBN_, int TSTAGES_, int MINB_, bool SOLO_, bool LATE_ = false>
+// CTA tile TBM x TBN (multiples of the 64 x 32 warp tile), TSTAGES-deep ring, one CTA per SM: the CTA asks for ALL the
+// shared memory a block may have (227 KB, SOLO), so that no other CTA -- of this grid, of another kernel of this library
+// or of a foreign kernel on another stream -- can share its SM.
 struct TmaCfg {
-  static constexpr bool LATE = LATE_;   // experiment: release a ring stage one k-tile late (see CfgSharedLate)
-  static constexpr int TBM = TBM_, TBN = TBN_, TSTAGES = TSTAGES_, MINB = MINB_;
+  static constexpr int TBM = 128, TBN = 128, TSTAGES = 6;
   static constexpr int CONSUMERS = (TBM / TWM) * (TBN / TWN);
   static constexpr int THREADS = (CONSUMERS + 1) * 32;    // + 1 producer warp
   static constexpr uint32_t A_BYTES = TBM * TBK * sizeof(double);
   static constexpr uint32_t B_BYTES = TBN * TBK * sizeof(double);
   static constexpr uint32_t STAGE_BYTES = A_BYTES + B_BYTES;
   static constexpr size_t USED = (size_t)TSTAGES * STAGE_BYTES + 2 * TSTAGES * sizeof(uint64_t) + 1024;  // + alignment slack
-  static constexpr size_t SMEM = SOLO_ ? (size_t)GEGP_MAX_DYN_SMEM : USED;
+  static constexpr size_t SMEM = GEGP_MAX_DYN_SMEM;
   static_assert(USED <= (size_t)GEGP_MAX_DYN_SMEM, "ring does not fit");
 };
-// WHY SOLO.  With the 128 x 64 tile / two CTAs per SM this kernel was first built with (CfgShared below; 35.2 TFLOP/s at
-// 8192^3), an evaluation was NOT reproducible whenever CTAs of this kernel shared SMs with CTAs of other kernels: beside
-// foreign cuBLAS DGEMMs on another stream 18 of 30 factorisations at N = 21000 came out wrong (a few tiles of a product,
+// WHY SOLO.  With the 128 x 64 tile / two CTAs per SM this kernel was first built with (35.2 TFLOP/s at 8192^3), an
+// evaluation was NOT reproducible whenever CTAs of this kernel shared SMs with CTAs of other kernels: beside foreign cuBLAS DGEMMs on another stream 18 of 30 factorisations at N = 21000 came out wrong (a few tiles of a product,
 // up to NaN), and with this library's own inverse running beside the factorisation 3 to 5 of 24 evaluations at
 // N = 41000 / 51000 deviated by up to 1e-7 (tools/repro_probe.py; profiles/r02/repro_tma_shared_sm.log).  The cp.async
 // kernels never deviated under the same load, nor did this kernel once it had the SM to itself; tensor maps in global
@@ -54,14 +50,7 @@ struct TmaCfg {
 // help (each tried).  The mechanism was not found -- every dependency of the ring is on an mbarrier and the protocol is
 // the textbook one -- so the kernel simply no longer shares an SM: 128 x 128 tile, 8 math warps + 1 producer warp,
 // 6 stages, the whole 227 KB.  Same k order per element as before (bit-identical results), same speed at N = 5500 and
-// 21000.  GEGP_TMA_SHARED_SM=1 brings the old configuration back (for reproducing the problem only).
-using CfgSolo = TmaCfg<128, 128, 6, 1, true>;
-using CfgShared = TmaCfg<128, 64, 4, 2, false>;
-// Experiment prepared for the prime suspect (DESIGN 7.0), not yet run: the shared configuration with every stage released
-// one k-tile LATE -- after the wait for the next stage, i.e. in program order behind every DMMA (and therefore every
-// completed shared-memory load) of the stage it releases -- instead of between the stage's last loads and the DMMAs that
-// consume them, where ptxas schedules the release otherwise.  GEGP_TMA_SHARED_SM=2 selects it.
-using CfgSharedLate = TmaCfg<128, 64, 4, 2, false, true>;
+// 21000.  The two-CTA configuration is in the history of this file (git show 815988e:gpgradpy_b200/csrc/gemm_tma.cu).
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
@@ -94,30 +83,15 @@ __device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* map
       : "memory");
 }
 
-struct TmaGemmArgs {
-  double* C;
-  int64_t ldc, sCo, sCi;
-  int M, N, K;
-  double alpha, beta;
-  int klo_mode, khi_mode, cmode, khi_off;
-  int inner;
-  int iAr, iAc, iBr, iBc;  // inner-batch row / column steps of the operands (tensor-map coordinates)
-  double* Ct;              // optional transposed second destination
-  int64_t ldct, sCto, sCti;
-};
-
-template <class Cfg>
-__global__ void __launch_bounds__(Cfg::THREADS, Cfg::MINB)
+__global__ void __launch_bounds__(TmaCfg::THREADS, 1)
 gemm_tma_nt_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-                   const TmaGemmArgs g) {
-  constexpr int TBM = Cfg::TBM, TBN = Cfg::TBN, TSTAGES = Cfg::TSTAGES, TCONSUMERS = Cfg::CONSUMERS;
-  constexpr uint32_t TILE_BYTES = Cfg::A_BYTES, STAGE_BYTES = Cfg::STAGE_BYTES;
+                   const __grid_constant__ GemmArgs g) {
+  constexpr int TBM = TmaCfg::TBM, TBN = TmaCfg::TBN, TSTAGES = TmaCfg::TSTAGES, TCONSUMERS = TmaCfg::CONSUMERS;
+  constexpr uint32_t TILE_BYTES = TmaCfg::A_BYTES, STAGE_BYTES = TmaCfg::STAGE_BYTES;
   extern __shared__ uint8_t smem_raw[];
   int bx = blockIdx.x, by = blockIdx.y;
-  if (g.khi_mode == KHI_N0) {   // longest tiles (last columns) first over the whole grid: see gemm.cu
-    const int lin = blockIdx.y * gridDim.x + blockIdx.x;
-    bx = (int)gridDim.x - 1 - lin / (int)gridDim.y;
-    by = lin % (int)gridDim.y;
+  if (g.khi_mode == KHI_N0) {
+    longest_first(bx, by);
   } else {
     // Grouped raster: CTAs are dispatched in linear block order, so walk the tiles in bands of RASTER_ROWS row tiles,
     // down the rows of a band first.  The ~296 CTAs in flight then cover RASTER_ROWS A panels x ~37 B panels instead
@@ -142,14 +116,8 @@ gemm_tma_nt_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
 
   const int zo = blockIdx.z / g.inner, zi = blockIdx.z - zo * g.inner;
 
-  int kb = 0, ke = g.K;
-  if (g.klo_mode == KLO_M0) kb = m0;
-  else if (g.klo_mode == KLO_N0) kb = n0;
-  else if (g.klo_mode == KLO_MAXMN) kb = max(m0, n0);
-  if (g.khi_mode == KHI_M0) ke = min(ke, m0 + TBM);
-  else if (g.khi_mode == KHI_N0) ke = min(ke, g.khi_off + n0 + TBN);
-  kb = (kb / TBK) * TBK;
-  const int ktiles = ke > kb ? (ke - kb + TBK - 1) / TBK : 0;
+  const KRange kr = tile_k_range<TBN, TBK>(g, m0, n0);
+  const int kb = kr.kb, ktiles = kr.tiles;
   const bool k_down = g.klo_mode != KLO_ZERO && g.khi_mode == KHI_K;
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -202,12 +170,6 @@ gemm_tma_nt_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
   for (int kt = 0; kt < ktiles; kt++) {
     const int s = kt % TSTAGES;
     mbar_wait(bar_full + 8 * s, (kt / TSTAGES) & 1);
-    if constexpr (Cfg::LATE) {
-      if (kt > 0) {
-        __syncwarp();
-        if (lane == 0) mbar_arrive(bar_empty + 8 * ((kt - 1) % TSTAGES));
-      }
-    }
     const uint8_t* st = tiles + s * STAGE_BYTES;
 #pragma unroll
     for (int q = 0; q < 4; q++) {
@@ -223,10 +185,8 @@ gemm_tma_nt_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
 #pragma unroll
         for (int j = 0; j < TNI; j++) dmma884(acc[i][j][0], acc[i][j][1], af[i], bf[j]);
     }
-    if constexpr (!Cfg::LATE) {
-      __syncwarp();
-      if (lane == 0) mbar_arrive(bar_empty + 8 * s);
-    }
+    __syncwarp();
+    if (lane == 0) mbar_arrive(bar_empty + 8 * s);
   }
 
   // ===== epilogue =====
@@ -238,33 +198,8 @@ gemm_tma_nt_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
     const int row = m0 + wm0 + i * 8 + lr;
     if (row >= g.M) continue;
 #pragma unroll
-    for (int j = 0; j < TNI; j++) {
-      const int col = n0 + wn0 + j * 8 + 2 * lk;
-      if (col >= g.N) continue;
-      double* cp = C + (int64_t)row * g.ldc + col;
-      double v0 = g.alpha * acc[i][j][0], v1 = g.alpha * acc[i][j][1];
-      const bool has1 = (col + 1 < g.N);
-      bool st0 = true, st1 = has1;
-      if (g.cmode != C_FULL) { st0 = (col <= row); st1 = has1 && (col + 1 <= row); }
-      if (g.beta != 0.0) {
-        if (st0) v0 += g.beta * cp[0];
-        if (st1) v1 += g.beta * cp[1];
-      }
-      if (st0 && st1 && vec_ok) {
-        *reinterpret_cast<double2*>(cp) = make_double2(v0, v1);
-      } else {
-        if (st0) cp[0] = v0;
-        if (st1) cp[1] = v1;
-      }
-      if (g.cmode == C_LOWER_MIRROR) {
-        if (st0 && col < row) C[(int64_t)col * g.ldc + row] = v0;
-        if (st1 && col + 1 < row) C[(int64_t)(col + 1) * g.ldc + row] = v1;
-      }
-      if (Ct) {
-        if (st0) Ct[(int64_t)col * g.ldct + row] = v0;
-        if (st1) Ct[(int64_t)(col + 1) * g.ldct + row] = v1;
-      }
-    }
+    for (int j = 0; j < TNI; j++)
+      store_pair(g, C, Ct, vec_ok, row, n0 + wn0 + j * 8 + 2 * lk, acc[i][j][0], acc[i][j][1]);
   }
 }
 
@@ -328,32 +263,10 @@ bool get_map(const double* ptr, uint64_t d0, uint64_t d1, uint64_t d2, uint64_t 
 
 }  // namespace
 
-template <class Cfg>
-static int launch_tma(const Ctx& ctx, const GemmArgs& g, uint64_t a_d0, uint64_t a_d1, uint64_t b_d0, uint64_t b_d1) {
-  CUtensorMap tmA, tmB;
-  if (!get_map(g.A, a_d0, a_d1, g.outer, g.lda, g.sAo, Cfg::TBM, &tmA)) return 1;
-  if (!get_map(g.B, b_d0, b_d1, g.outer, g.ldb, g.sBo, Cfg::TBN, &tmB)) return 1;
-  TmaGemmArgs t{};
-  t.C = g.C; t.ldc = g.ldc; t.sCo = g.sCo; t.sCi = g.sCi;
-  t.M = g.M; t.N = g.N; t.K = g.K; t.alpha = g.alpha; t.beta = g.beta;
-  t.klo_mode = g.klo_mode; t.khi_mode = g.khi_mode; t.cmode = g.cmode; t.khi_off = g.khi_off;
-  t.inner = g.inner; t.iAr = g.iAr; t.iAc = g.iAc; t.iBr = g.iBr; t.iBc = g.iBc;
-  t.Ct = g.Ct; t.ldct = g.ldct; t.sCto = g.sCto; t.sCti = g.sCti;
-  GEGP_SET_SMEM(gemm_tma_nt_kernel<Cfg>, Cfg::SMEM);
-  dim3 grid((g.N + Cfg::TBN - 1) / Cfg::TBN, (g.M + Cfg::TBM - 1) / Cfg::TBM, g.outer * g.inner);
-  prof_gemm_begin(ctx.stream);
-  timeline_begin(ctx.stream, "gemm_tma", g.M, g.N, g.K, timeline_on() ? gemm_useful_flops(g) * 1e-6 : 0.0);
-  gemm_tma_nt_kernel<Cfg><<<grid, Cfg::THREADS, Cfg::SMEM, ctx.stream>>>(tmA, tmB, t);
-  timeline_end(ctx.stream);
-  if (prof().on) prof_gemm_end(ctx.stream, gemm_useful_flops(g));
-  GEGP_CHECK_LAUNCH();
-  return 0;
-}
-
 // Returns 0 on launch, 1 when this GEMM is outside what the TMA kernel covers (caller falls back to the
 // cp.async engine), negative on a launch error.
 int gemm_tma_nt(const Ctx& ctx, const GemmArgs& g) {
-  if (!g.b_kcont || g.row_owner) return 1;
+  if (!g.b_kcont) return 1;
   if (g.M < 1 || g.N < 1) return 1;
   if (g.inner > 1 && !g.inner_steps) return 1;
   if ((g.sAo & 1) || (g.sBo & 1)) return 1;
@@ -361,10 +274,12 @@ int gemm_tma_nt(const Ctx& ctx, const GemmArgs& g) {
   const uint64_t a_d0 = (uint64_t)(inner - 1) * g.iAc + g.K, a_d1 = (uint64_t)(inner - 1) * g.iAr + g.M;
   const uint64_t b_d0 = (uint64_t)(inner - 1) * g.iBc + g.K, b_d1 = (uint64_t)(inner - 1) * g.iBr + g.N;
   if (g.K < 1 || a_d0 > (uint64_t)g.lda || b_d0 > (uint64_t)g.ldb) return 1;
-  static const int shared_sm = getenv("GEGP_TMA_SHARED_SM") ? atoi(getenv("GEGP_TMA_SHARED_SM")) : 0;
-  if (shared_sm == 2) return launch_tma<CfgSharedLate>(ctx, g, a_d0, a_d1, b_d0, b_d1);
-  if (shared_sm) return launch_tma<CfgShared>(ctx, g, a_d0, a_d1, b_d0, b_d1);
-  return launch_tma<CfgSolo>(ctx, g, a_d0, a_d1, b_d0, b_d1);
+  CUtensorMap tmA, tmB;
+  if (!get_map(g.A, a_d0, a_d1, g.outer, g.lda, g.sAo, TmaCfg::TBM, &tmA)) return 1;
+  if (!get_map(g.B, b_d0, b_d1, g.outer, g.ldb, g.sBo, TmaCfg::TBN, &tmB)) return 1;
+  const dim3 grid((g.N + TmaCfg::TBN - 1) / TmaCfg::TBN, (g.M + TmaCfg::TBM - 1) / TmaCfg::TBM, g.outer * g.inner);
+  return launch_gemm<gemm_tma_nt_kernel>(ctx, g, grid, TmaCfg::THREADS, TmaCfg::SMEM, "gemm_tma", g.M, g.N, g.K, tmA, tmB,
+                                         g);
 }
 
 }  // namespace gegp

@@ -6,7 +6,7 @@
 namespace gegp {
 
 enum KLo { KLO_ZERO = 0, KLO_M0 = 1, KLO_N0 = 2, KLO_MAXMN = 3 };
-enum KHi { KHI_K = 0, KHI_M0 = 1, KHI_N0 = 2 };
+enum KHi { KHI_K = 0, KHI_N0 = 2 };
 enum CMode { C_FULL = 0, C_LOWER = 1, C_LOWER_MIRROR = 2 };
 
 struct GemmArgs {
@@ -30,11 +30,16 @@ struct GemmArgs {
   // optional second, transposed destination: Ct[col * ldct + row] = value for every stored C(row, col)
   double* Ct;
   int64_t ldct, sCto, sCti;
-  bool row_owner;  // C aliases A (in-place right multiply): every CTA must own complete rows (one column tile)
 };
 
 GemmArgs gemm_args(const double* A, int64_t lda, const double* B, int64_t ldb, double* C, int64_t ldc,
                    int M, int N, int K, double alpha, double beta, bool b_kcont);
+// g over the ctx.batch problems of a call, whose A, B and C lie sA, sB and sC doubles after those of the previous one
+inline GemmArgs batched(const Ctx& ctx, GemmArgs g, int64_t sA, int64_t sB, int64_t sC) {
+  g.outer = ctx.batch; g.inner = 1;
+  g.sAo = sA; g.sBo = sB; g.sCo = sC;
+  return g;
+}
 
 // C = alpha*A*op(B) + beta*C on fp64 tensor cores (DMMA). Returns 0 or a negative launch error.
 int gemm_f64(const Ctx& ctx, GemmArgs g);

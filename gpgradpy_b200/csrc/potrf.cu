@@ -25,12 +25,6 @@ static inline int split_point(int k) {
   return k1;
 }
 
-static GemmArgs batched(const Ctx& ctx, GemmArgs g, int64_t sA, int64_t sB, int64_t sC) {
-  g.outer = ctx.batch; g.inner = 1;
-  g.sAo = sA; g.sBo = sB; g.sCo = sC;
-  return g;
-}
-
 static const double* dinv_block(const double* Dinv, int col0) { return Dinv + (int64_t)(col0 / LEAF) * LEAF * LEAF; }
 
 int trsm_right_rec(const Ctx& ctx, const double* L, int64_t ldl, int64_t strideL, const double* Dinv, int64_t strideD,
@@ -99,6 +93,49 @@ int trsm_right_lower_rec(const Ctx& ctx, const double* L, int64_t ldl, const dou
   return trsm_right_lower_rec(ctx, L, ldl, Dinv, Lt, col0, B, ldb, r, k1, T);
 }
 
+// ---- the products of the explicit inverse ----
+// U = L^-T (upper) and, while U is built, W = U^T = L^-1 in the lower triangle of T (the Kinv buffer); each builder
+// returns the GEMM over the ctx.batch problems of the call (U, L and T of one problem sU, sL and sT doubles apart).
+// A pair is a = [r, r+m), b = [r+m, r+m+n) on the diagonal:  U_ab = -(U_aa L_ba^T) U_bb.
+
+// first product of a pair: T_ab = U_aa L_ba^T, staged in the upper triangle of T at the coordinates of U_ab.  U_aa is upper
+// triangular (k >= i): k clipped below by the row tile.
+static GemmArgs pair_first(const Ctx& ctx, const double* L, int64_t ldl, int64_t sL, const double* U, int64_t ldu,
+                           int64_t sU, double* T, int64_t ldt, int64_t sT, int r, int m, int n) {
+  GemmArgs g = gemm_args(U + (int64_t)r * ldu + r, ldu, L + (int64_t)(r + m) * ldl + r, ldl, T + (int64_t)r * ldt + r + m,
+                         ldt, m, n, m, 1.0, 0.0, true);
+  g.klo_mode = KLO_M0;
+  return batched(ctx, g, sU, sL, sT);
+}
+// second product: U_ab = -T_ab W_bb^T, W_bb = L_bb^-1 (lower: element (j, k) nonzero for k <= j, read from the lower
+// triangle of T; k clipped above by the column tile), only the columns [c_from, n) of U_ab: the rows [c_from, n) of
+// W_bb, whose k range starts c_from columns earlier.  store_w: U_ab^T is stored a second time, as W_ba in T.
+static GemmArgs pair_second(const Ctx& ctx, double* U, int64_t ldu, int64_t sU, double* T, int64_t ldt, int64_t sT, int r,
+                            int m, int n, int c_from, bool store_w) {
+  GemmArgs g = gemm_args(T + (int64_t)r * ldt + r + m, ldt, T + (int64_t)(r + m + c_from) * ldt + r + m, ldt,
+                         U + (int64_t)r * ldu + r + m + c_from, ldu, m, n - c_from, n, -1.0, 0.0, true);
+  g.khi_mode = KHI_N0;
+  g.khi_off = c_from;
+  if (store_w) { g.Ct = T + (int64_t)(r + m + c_from) * ldt + r; g.ldct = ldt; g.sCto = sT; }
+  return batched(ctx, g, sT, sT, sU);
+}
+// K^-1 = U U^T on the n x n diagonal block that starts at U and Kinv: U upper, so the sum runs over k >= max(i, j); the
+// lower tiles are computed and mirrored to the upper half.
+static GemmArgs kinv_from_u(const Ctx& ctx, const double* U, int64_t ldu, int64_t sU, double* Kinv, int64_t ldk,
+                            int64_t sK, int n) {
+  GemmArgs g = gemm_args(U, ldu, U, ldu, Kinv, ldk, n, n, n, 1.0, 0.0, true);
+  g.klo_mode = KLO_MAXMN;
+  g.cmode = C_LOWER_MIRROR;
+  return batched(ctx, g, sU, sU, sK);
+}
+// Kinv_aa += U_a,x U_a,x^T for a = [0, m) and the columns x = [c0, c1) of U (lower tiles, mirrored)
+static GemmArgs kinv_add_cols(const Ctx& ctx, const double* U, int64_t ldu, int64_t sU, double* Kinv, int64_t ldk,
+                              int64_t sK, int m, int c0, int c1) {
+  GemmArgs g = gemm_args(U + c0, ldu, U + c0, ldu, Kinv, ldk, m, m, c1 - c0, 1.0, 1.0, true);
+  g.cmode = C_LOWER_MIRROR;
+  return batched(ctx, g, sU, sU, sK);
+}
+
 // U = L^-T by levels: diagonal LEAF blocks first, then for block size bs = LEAF, 2*LEAF, ... every pair
 // (a = [s, s+bs), b = [s+bs, s+2bs)):  U_ab = -(U_aa * L_ba^T) * U_bb.  The product in parentheses is staged in the
 // upper triangle of T (the Kinv buffer, same coordinates as U_ab).  The LOWER triangle of T meanwhile collects
@@ -119,31 +156,18 @@ static int inverse_transposed(const Ctx& ctx, const double* L, int64_t ldl, int6
         s = npairs_full * 2 * bs; bsz = N - s - bs; inner = 1;
         if (bsz <= 0) continue;
       }
-      const int64_t pstepL = (int64_t)2 * bs * (ldl + 1), pstepU = (int64_t)2 * bs * (ldu + 1),
-                    pstepT = (int64_t)2 * bs * (ldt + 1);
-      const double* Uaa = U + (int64_t)s * ldu + s;
-      const double* Lba = L + (int64_t)(s + bs) * ldl + s;
-      double* Tab = T + (int64_t)s * ldt + s + bs;
-      // T_ab (bs x bsz) = U_aa (bs x bs, upper: k >= i) * L_ba^T  -> k clipped below by m0
-      GemmArgs g1 = gemm_args(Uaa, ldu, Lba, ldl, Tab, ldt, bs, bsz, bs, 1.0, 0.0, true);
-      g1.klo_mode = KLO_M0;
-      g1.outer = ctx.batch; g1.inner = inner;
-      g1.sAo = strideU; g1.sBo = strideL; g1.sCo = strideT; g1.sAi = pstepU; g1.sBi = pstepL; g1.sCi = pstepT;
-      g1.inner_steps = true; g1.iAr = g1.iAc = g1.iBr = g1.iBc = 2 * bs;
-      rc = gemm_f64(ctx, g1);
+      // the inner batch: pair i + 1 lies 2 bs rows and columns further down the diagonal of every operand
+      auto pairs = [&](GemmArgs g) {
+        const int64_t step = 2 * bs;
+        g.inner = inner;
+        g.sAi = step * (g.lda + 1); g.sBi = step * (g.ldb + 1); g.sCi = step * (g.ldc + 1);
+        if (g.Ct) g.sCti = step * (g.ldct + 1);
+        g.inner_steps = true; g.iAr = g.iAc = g.iBr = g.iBc = 2 * bs;
+        return g;
+      };
+      rc = gemm_f64(ctx, pairs(pair_first(ctx, L, ldl, strideL, U, ldu, strideU, T, ldt, strideT, s, bs, bsz)));
       if (rc) return rc;
-      // U_ab = -T_ab (bs x bsz) * W_bb^T,  W_bb = L_bb^-1 (bsz x bsz lower: element (j, k) nonzero for k <= j, read
-      // from the lower triangle of T; k clipped above by n0 + BN); the transposed copy W_ba = U_ab^T goes there too.
-      const double* Wbb = T + (int64_t)(s + bs) * ldt + s + bs;
-      double* Uab = U + (int64_t)s * ldu + s + bs;
-      double* Wba = T + (int64_t)(s + bs) * ldt + s;
-      GemmArgs g2 = gemm_args(Tab, ldt, Wbb, ldt, Uab, ldu, bs, bsz, bsz, -1.0, 0.0, true);
-      g2.khi_mode = KHI_N0;
-      g2.Ct = Wba; g2.ldct = ldt; g2.sCto = strideT; g2.sCti = pstepT;
-      g2.outer = ctx.batch; g2.inner = inner;
-      g2.sAo = strideT; g2.sBo = strideT; g2.sCo = strideU; g2.sAi = pstepT; g2.sBi = pstepT; g2.sCi = pstepU;
-      g2.inner_steps = true; g2.iAr = g2.iAc = g2.iBr = g2.iBc = 2 * bs;
-      rc = gemm_f64(ctx, g2);
+      rc = gemm_f64(ctx, pairs(pair_second(ctx, U, ldu, strideU, T, ldt, strideT, s, bs, bsz, 0, true)));
       if (rc) return rc;
     }
   }
@@ -378,35 +402,17 @@ int inv_pair_first(LookAhead* la, const InvHook* h, const Ctx& chain, int row0, 
   int rc = inv_sync(la, chain.stream);
   if (rc) return rc;
   const Ctx ic{la->inv, chain.batch};
-  const double* Uaa = h->U + (int64_t)row0 * (h->ldu + 1);
-  const double* Lba = h->A0 + (int64_t)(row0 + k1) * h->lda + row0;
-  double* Tab = h->T + (int64_t)row0 * h->ldt + row0 + k1;
-  GemmArgs g1 = gemm_args(Uaa, h->ldu, Lba, h->lda, Tab, h->ldt, k1, kc, k1, 1.0, 0.0, true);
-  g1.klo_mode = KLO_M0;
-  g1.outer = ic.batch; g1.inner = 1;
-  g1.sAo = h->sU; g1.sBo = h->sA; g1.sCo = h->sT;
-  return gemm_f64(ic, g1);
+  return gemm_f64(ic, pair_first(ic, h->A0, h->lda, h->sA, h->U, h->ldu, h->sU, h->T, h->ldt, h->sT, row0, k1, kc));
 }
 // second product: U_ab = -T_ab W_bb^T (W_bb = L_bb^-1 from the lower triangle of T), with the transposed copy W_ba.
-// `c_from` > 0 (root only): the first c_from columns of U_ab have been produced early (inv_root_early_pair), only the
-// columns [c_from, kc) are computed -- the rows [c_from, kc) of W_bb, whose k range starts c_from columns earlier.
+// `c_from` > 0 (root only): the first c_from columns of U_ab have been produced early (inv_root_early_pair).
 // The root's W_ba is never read (the root is nobody's right child), so no transposed copy is stored then.
 int inv_pair_second(LookAhead* la, const InvHook* h, const Ctx& chain, int row0, int k1, int kc, int c_from = 0,
                     bool store_w = true) {
   int rc = inv_sync(la, chain.stream);
   if (rc) return rc;
   const Ctx ic{la->inv, chain.batch};
-  const double* Tab = h->T + (int64_t)row0 * h->ldt + row0 + k1;
-  const double* Wbb = h->T + (int64_t)(row0 + k1 + c_from) * h->ldt + row0 + k1;
-  double* Uab = h->U + (int64_t)row0 * h->ldu + row0 + k1 + c_from;
-  double* Wba = h->T + (int64_t)(row0 + k1 + c_from) * h->ldt + row0;
-  GemmArgs g2 = gemm_args(Tab, h->ldt, Wbb, h->ldt, Uab, h->ldu, k1, kc - c_from, kc, -1.0, 0.0, true);
-  g2.khi_mode = KHI_N0;
-  g2.khi_off = c_from;
-  if (store_w) { g2.Ct = Wba; g2.ldct = h->ldt; g2.sCto = h->sT; g2.sCti = 0; }
-  g2.outer = ic.batch; g2.inner = 1;
-  g2.sAo = h->sT; g2.sBo = h->sT; g2.sCo = h->sU;
-  return gemm_f64(ic, g2);
+  return gemm_f64(ic, pair_second(ic, h->U, h->ldu, h->sU, h->T, h->ldt, h->sT, row0, k1, kc, c_from, store_w));
 }
 
 // ---- early pieces of K^-1 (root node only; a = the root's left child, b = its right child with children ba, bb) ----
@@ -418,12 +424,7 @@ int inv_root_early_aa(LookAhead* la, const InvHook* h, const Ctx& chain, int k1)
   if (cudaEventRecord(la->ev_early, la->inv) != cudaSuccess) return -1130;
   if (cudaStreamWaitEvent(la->early, la->ev_early, 0) != cudaSuccess) return -1130;
   const Ctx ec{la->early, chain.batch};
-  GemmArgs g = gemm_args(h->U, h->ldu, h->U, h->ldu, h->T, h->ldt, k1, k1, k1, 1.0, 0.0, true);
-  g.klo_mode = KLO_MAXMN;
-  g.cmode = C_LOWER_MIRROR;
-  g.outer = ec.batch; g.inner = 1;
-  g.sAo = h->sU; g.sBo = h->sU; g.sCo = h->sT;
-  const int rc = gemm_f64(ec, g);
+  const int rc = gemm_f64(ec, kinv_from_u(ec, h->U, h->ldu, h->sU, h->T, h->ldt, h->sT, k1));
   if (!rc) la->early_k1 = k1;
   return rc;
 }
@@ -433,20 +434,9 @@ int inv_root_early_pair(LookAhead* la, const InvHook* h, const Ctx& chain, int k
   if (cudaEventRecord(la->ev_early, la->inv) != cudaSuccess) return -1131;
   if (cudaStreamWaitEvent(la->early, la->ev_early, 0) != cudaSuccess) return -1131;
   const Ctx ec{la->early, chain.batch};
-  const double* Tab = h->T + k1;
-  const double* Wbb = h->T + (int64_t)k1 * (h->ldt + 1);
-  double* Uab = h->U + k1;
-  GemmArgs g2 = gemm_args(Tab, h->ldt, Wbb, h->ldt, Uab, h->ldu, k1, kba, kba, -1.0, 0.0, true);
-  g2.khi_mode = KHI_N0;
-  g2.outer = ec.batch; g2.inner = 1;
-  g2.sAo = h->sT; g2.sBo = h->sT; g2.sCo = h->sU;
-  int rc = gemm_f64(ec, g2);
+  int rc = gemm_f64(ec, pair_second(ec, h->U, h->ldu, h->sU, h->T, h->ldt, h->sT, 0, k1, kba, 0, false));
   if (rc) return rc;
-  GemmArgs g = gemm_args(Uab, h->ldu, Uab, h->ldu, h->T, h->ldt, k1, k1, kba, 1.0, 1.0, true);
-  g.cmode = C_LOWER_MIRROR;
-  g.outer = ec.batch; g.inner = 1;
-  g.sAo = h->sU; g.sBo = h->sU; g.sCo = h->sT;
-  rc = gemm_f64(ec, g);
+  rc = gemm_f64(ec, kinv_add_cols(ec, h->U, h->ldu, h->sU, h->T, h->ldt, h->sT, k1, k1, k1 + kba));
   if (!rc) la->early_ba = kba;
   return rc;
 }
@@ -460,33 +450,22 @@ int finish_inverse_split(LookAhead* la, const InvHook* h, int batch, int N) {
   if (cudaStreamWaitEvent(la->col, la->ev_fin[0], 0) != cudaSuccess) return -1132;
   if (cudaStreamWaitEvent(la->late, la->ev_fin[0], 0) != cudaSuccess) return -1132;
   const double* Ubb = h->U + (int64_t)k1 * (h->ldu + 1);
-  const double* Uab = h->U + k1;
   int rc;
   {  // the largest first: Kinv_ab (k1 x kc) = U_ab U_bb^T, U_bb upper: k >= column
     const Ctx c{la->col, batch};
-    GemmArgs g = gemm_args(Uab, h->ldu, Ubb, h->ldu, h->T + k1, h->ldt, k1, kc, kc, 1.0, 0.0, true);
+    GemmArgs g = gemm_args(h->U + k1, h->ldu, Ubb, h->ldu, h->T + k1, h->ldt, k1, kc, kc, 1.0, 0.0, true);
     g.klo_mode = KLO_N0;
-    g.Ct = h->T + (int64_t)k1 * h->ldt; g.ldct = h->ldt; g.sCto = h->sT; g.sCti = 0;
-    g.outer = batch; g.inner = 1;
-    g.sAo = h->sU; g.sBo = h->sU; g.sCo = h->sT;
-    if ((rc = gemm_f64(c, g))) return rc;
+    g.Ct = h->T + (int64_t)k1 * h->ldt; g.ldct = h->ldt; g.sCto = h->sT;
+    if ((rc = gemm_f64(c, batched(c, g, h->sU, h->sU, h->sT)))) return rc;
   }
   {  // Kinv_aa += U_a,x U_a,x^T
     const Ctx c{la->late, batch};
-    GemmArgs g = gemm_args(Uab + off, h->ldu, Uab + off, h->ldu, h->T, h->ldt, k1, k1, kc - off, 1.0, 1.0, true);
-    g.cmode = C_LOWER_MIRROR;
-    g.outer = batch; g.inner = 1;
-    g.sAo = h->sU; g.sBo = h->sU; g.sCo = h->sT;
-    if ((rc = gemm_f64(c, g))) return rc;
+    if ((rc = gemm_f64(c, kinv_add_cols(c, h->U, h->ldu, h->sU, h->T, h->ldt, h->sT, k1, k1 + off, N)))) return rc;
   }
   {  // Kinv_bb = U_bb U_bb^T
     const Ctx c{la->hi, batch};
-    GemmArgs g = gemm_args(Ubb, h->ldu, Ubb, h->ldu, h->T + (int64_t)k1 * (h->ldt + 1), h->ldt, kc, kc, kc, 1.0, 0.0, true);
-    g.klo_mode = KLO_MAXMN;
-    g.cmode = C_LOWER_MIRROR;
-    g.outer = batch; g.inner = 1;
-    g.sAo = h->sU; g.sBo = h->sU; g.sCo = h->sT;
-    if ((rc = gemm_f64(c, g))) return rc;
+    if ((rc = gemm_f64(c, kinv_from_u(c, Ubb, h->ldu, h->sU, h->T + (int64_t)k1 * (h->ldt + 1), h->ldt, h->sT, kc))))
+      return rc;
   }
   if (cudaEventRecord(la->ev_fin[1], la->col) != cudaSuccess || cudaEventRecord(la->ev_fin[2], la->late) != cudaSuccess ||
       cudaStreamWaitEvent(la->hi, la->ev_fin[1], 0) != cudaSuccess ||
@@ -689,10 +668,7 @@ int chol_trap_inverse(const Ctx& ctx, double* A, int64_t lda, int64_t strideA, i
                       int64_t strideD, double* U, int64_t ldu, int64_t strideU, double* Kinv, int64_t ldk,
                       int64_t strideK) {
   const InvHook hook{U, ldu, strideU, Kinv, ldk, strideK, A, lda, strideA, Dinv, strideD, inv_unit_max()};
-  // (env GEGP_INV_MAX_N: largest N with the inverse interleaved; a debugging aid -- the deviations once seen with the two
-  // side by side at N >= 41000 came from the TMA GEMM sharing SMs with other kernels, see gemm_tma.cu)
-  static const int interleave_max_n = getenv("GEGP_INV_MAX_N") ? atoi(getenv("GEGP_INV_MAX_N")) : (1 << 30);
-  const bool interleave = inv_unit_max() >= LEAF && k <= interleave_max_n;
+  const bool interleave = inv_unit_max() >= LEAF;
   int done = 0;
   int rc = chol_trap_impl(ctx, A, lda, strideA, m, k, 0, info, Dinv, strideD, interleave ? &hook : nullptr, &done);
   if (rc) return rc;
@@ -702,13 +678,7 @@ int chol_trap_inverse(const Ctx& ctx, double* A, int64_t lda, int64_t strideA, i
     if (rc) return rc;
     return chol_inverse(ctx, A, lda, strideA, Dinv, strideD, U, ldu, strideU, Kinv, ldk, strideK, k);
   }
-  // Kinv = U * U^T, U upper: sum over k >= max(i, j); lower tiles computed, mirrored to the upper half.
-  GemmArgs g = gemm_args(U, ldu, U, ldu, Kinv, ldk, k, k, k, 1.0, 0.0, true);
-  g.klo_mode = KLO_MAXMN;
-  g.cmode = C_LOWER_MIRROR;
-  g.outer = ctx.batch; g.inner = 1;
-  g.sAo = strideU; g.sBo = strideU; g.sCo = strideK;
-  return gemm_f64(ctx, g);
+  return gemm_f64(ctx, kinv_from_u(ctx, U, ldu, strideU, Kinv, ldk, strideK, k));
 }
 
 int chol_inverse(const Ctx& ctx, const double* L, int64_t ldl, int64_t strideL, const double* Dinv, int64_t strideD,
@@ -719,13 +689,7 @@ int chol_inverse(const Ctx& ctx, const double* L, int64_t ldl, int64_t strideL, 
   // every GEMM below clips its k range at tile granularity and tiles nest inside the LEAF blocks.
   int rc = inverse_transposed(ctx, L, ldl, strideL, Dinv, strideD, U, ldu, strideU, Kinv, ldk, strideK, N);
   if (rc) return rc;
-  // Kinv = U * U^T, U upper: sum over k >= max(i, j); lower tiles computed, mirrored to the upper half.
-  GemmArgs g = gemm_args(U, ldu, U, ldu, Kinv, ldk, N, N, N, 1.0, 0.0, true);
-  g.klo_mode = KLO_MAXMN;
-  g.cmode = C_LOWER_MIRROR;
-  g.outer = ctx.batch; g.inner = 1;
-  g.sAo = strideU; g.sBo = strideU; g.sCo = strideK;
-  return gemm_f64(ctx, g);
+  return gemm_f64(ctx, kinv_from_u(ctx, U, ldu, strideU, Kinv, ldk, strideK, N));
 }
 
 }  // namespace gegp

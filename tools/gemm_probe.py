@@ -13,4 +13,4 @@ for (M, Nn, K, tb) in [(2048, 2048, 2048, True), (1536, 1536, 768, True), (2560,
     Bm = torch.randn((Nn, K) if tb else (K, Nn), dtype=torch.float64, device="cuda")
     Cm = torch.zeros((M, Nn), dtype=torch.float64, device="cuda")
     ms = ev(lambda: bk.dgemm(A, Bm, Cm, transb=tb))
-    print(f"cfg={os.environ.get('GEGP_GEMM_CFG','0')} dgemm M={M} N={Nn} K={K} transb={tb}: {ms:.3f} ms  {2*M*Nn*K/ms*1e-9:.2f} TFLOP/s", flush=True)
+    print(f"dgemm M={M} N={Nn} K={K} transb={tb}: {ms:.3f} ms  {2*M*Nn*K/ms*1e-9:.2f} TFLOP/s", flush=True)
