@@ -109,6 +109,7 @@ int launch_scale_vec(const Ctx& ctx, int N, const double* a, int64_t strideA, co
 // Per-CTA partial sums are written to `partial` and reduced in a fixed order by the finalize kernel.
 // ------------------------------------------------------------------------------------------------
 constexpr int GB = 128;
+constexpr int LML_GRAD_MAX_GRID_Y = 65535;
 
 // quad 0: LML gradient weights; 1: W = alpha alpha^T (Kinv not read); 2: W = the matrix passed as Kinv.
 // WIDE (d >= 8): four independent Kinv loads in flight per thread; otherwise the plain loop -- measured: the wide form
@@ -122,7 +123,7 @@ lml_grad_kernel(Geom gm, const double* __restrict__ theta_all, int64_t strideThe
                 int64_t ldk, int64_t strideK, const double* __restrict__ alpha_all, int64_t strideAlpha,
                 const double* __restrict__ pinv_all, int64_t strideP, const double* __restrict__ out_all,
                 int64_t strideOut, int noisy, double pnlt_grad, double* __restrict__ partial_all,
-                int64_t stridePartial) {
+                int64_t stridePartial, int a0) {
   extern __shared__ double sm[];
   const int d = gm.d, n = gm.n, ng = gm.ng, N = gm.N;
   double* vs = sm;              // [d][GB]  v_j = pinv[col_j] * u_j
@@ -131,7 +132,7 @@ lml_grad_kernel(Geom gm, const double* __restrict__ theta_all, int64_t strideThe
   double* th = xa + d;             // [d]
 
   const int tid = threadIdx.x, z = blockIdx.z;
-  const int a = blockIdx.y, b = blockIdx.x * GB + tid;
+  const int a = a0 + blockIdx.y, b = blockIdx.x * GB + tid;
   const double* theta = theta_all + z * strideTheta;
   const double* Kinv = Kinv_all + z * strideK;
   const double* alpha = alpha_all + z * strideAlpha;
@@ -364,27 +365,32 @@ int launch_lml_grad(const Ctx& ctx, const Geom& gm, const double* theta, int64_t
       else GEGP_SET_SMEM((lml_grad_kernel<2, true, false>), GEGP_MAX_DYN_SMEM);
     }
   }
-  dim3 grid((gm.n + GB - 1) / GB, gm.n, ctx.batch);
+  // point a is a0 + blockIdx.y: the launch is issued in slices of at most 65535 points a (the gridDim.y limit), each
+  // CTA computing and storing exactly what it would in one launch
+  const int nbt = (gm.n + GB - 1) / GB;
   timeline_begin(ctx.stream, "lmlgrad", gm.N, d, quad);
+  for (int a0 = 0; a0 < gm.n; a0 += LML_GRAD_MAX_GRID_Y) {
+    const dim3 grid(nbt, (gm.n - a0 < LML_GRAD_MAX_GRID_Y) ? gm.n - a0 : LML_GRAD_MAX_GRID_Y, ctx.batch);
 #define GEGP_LAUNCH_LML_GRAD(Q, W, G)                                                                                    \
-  lml_grad_kernel<Q, W, G><<<grid, GB, smem, ctx.stream>>>(gm, theta, strideTheta, Kinv, ldk, strideK, alpha_t,          \
-                                                           strideAlpha, pinv, strideP, out, strideOut, noisy, pnlt_grad, \
-                                                           partial, stridePartial)
+    lml_grad_kernel<Q, W, G><<<grid, GB, smem, ctx.stream>>>(gm, theta, strideTheta, Kinv, ldk, strideK, alpha_t,        \
+                                                             strideAlpha, pinv, strideP, out, strideOut, noisy, pnlt_grad, \
+                                                             partial, stridePartial, a0)
 #define GEGP_LAUNCH_LML_GRAD_W(Q, G) do { if (wide) GEGP_LAUNCH_LML_GRAD(Q, true, G); else GEGP_LAUNCH_LML_GRAD(Q, false, G); } while (0)
-  if (gauss) {
-    if (quad == 0) GEGP_LAUNCH_LML_GRAD_W(0, true);
-    else if (quad == 1) GEGP_LAUNCH_LML_GRAD_W(1, true);
-    else GEGP_LAUNCH_LML_GRAD_W(2, true);
-  } else {
-    if (quad == 0) GEGP_LAUNCH_LML_GRAD_W(0, false);
-    else if (quad == 1) GEGP_LAUNCH_LML_GRAD_W(1, false);
-    else GEGP_LAUNCH_LML_GRAD_W(2, false);
-  }
+    if (gauss) {
+      if (quad == 0) GEGP_LAUNCH_LML_GRAD_W(0, true);
+      else if (quad == 1) GEGP_LAUNCH_LML_GRAD_W(1, true);
+      else GEGP_LAUNCH_LML_GRAD_W(2, true);
+    } else {
+      if (quad == 0) GEGP_LAUNCH_LML_GRAD_W(0, false);
+      else if (quad == 1) GEGP_LAUNCH_LML_GRAD_W(1, false);
+      else GEGP_LAUNCH_LML_GRAD_W(2, false);
+    }
 #undef GEGP_LAUNCH_LML_GRAD_W
 #undef GEGP_LAUNCH_LML_GRAD
+    GEGP_CHECK_LAUNCH();
+  }
   timeline_end(ctx.stream);
-  GEGP_CHECK_LAUNCH();
-  const int64_t nparts = (int64_t)grid.x * grid.y;
+  const int64_t nparts = (int64_t)nbt * gm.n;
   const int np = 2 * d + 3;
   lml_grad_colsum_kernel<<<dim3(np, ctx.batch), 256, 0, ctx.stream>>>(np, nparts, partial, stridePartial);
   GEGP_CHECK_LAUNCH();
